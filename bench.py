@@ -5,6 +5,7 @@
   python bench.py --impl reference ...                     # the reference's own CPU path on the box's host cores
   torchrun --nproc-per-node N ... bench.py --gpus N ...    # one rank per GPU, utterances sharded, no collective
   python bench.py --config 3|4|5 ...                       # sample-rate sweep | FlowSE 32x10 s NFE 15 | training step
+  python bench.py ... --dump-outputs DIR                   # + what the last timed step computed (rank 0), DIR/<name>.npy
 
 Config 2 (default, the headline): a step = one BSRNN_SE forward (STFT -> BandSplit -> 6x[time BLSTM, band BLSTM] ->
 MaskDecoder -> mask+iSTFT) over one batch of synthetic noisy utterances with random-init BSRNN_baseline.yaml weights
@@ -32,6 +33,27 @@ FS = 48000
 NUM_CHANNEL, NUM_LAYER = 196, 6                      # conf/models/BSRNN_baseline.yaml:36-38
 METRIC, UNIT = "BSRNN audio-sec/sec enhanced at 48 kHz", "audio-s/s"
 RATES = (8000, 16000, 22050, 24000, 32000, 44100, 48000)          # SURVEY.md §8d cfg3
+DUMP_BYTES = 60_000_000                              # --dump-outputs: data of all arrays together (64 MB with the headers)
+
+
+def dump_outputs(out_dir, arrays):
+    """--dump-outputs: {name: tensor} -> out_dir/<name>.npy, so that two builds can be compared output for output.
+    Complex tensors get a trailing (re, im) axis; float64 stays float64, everything else is written as float32.  When
+    the arrays together hold more than DUMP_BYTES, each keeps the same fraction of its elements, flattened to 1-D: the
+    sorted distinct flat indices drawn by numpy's default_rng(0).  They depend on the array's size and on the total
+    size of all the arrays, so runs with the same arguments write the same elements.  Files of the same names are
+    overwritten; other files already in out_dir are left as they are."""
+    import numpy as np
+    arrays = {k: torch.view_as_real(t.detach()) if t.is_complex() else t.detach() for k, t in arrays.items()}
+    arrays = {k: t if t.dtype == torch.float64 else t.float() for k, t in arrays.items()}
+    total = sum(t.numel() * t.element_size() for t in arrays.values())
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        if total > DUMP_BYTES:
+            keep = max(1, t.numel() * DUMP_BYTES // total)
+            idx = np.unique(np.random.default_rng(0).integers(0, t.numel(), size=keep))
+            t = t.reshape(-1)[torch.from_numpy(idx).to(t.device)]
+        np.save(os.path.join(out_dir, name + ".npy"), t.cpu().numpy())
 
 
 def lstm_flops(tokens, N=NUM_CHANNEL, layers=NUM_LAYER):
@@ -332,11 +354,12 @@ def run_config2(ctx, args):
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     for _ in range(args.steps):
-        model(x_dev, lens, FS)
+        wav, spec = model(x_dev, lens, FS)
     e1.record()
     ctx.barrier()
     t_b = time.monotonic()
     ms = e0.elapsed_time(e1)
+    outputs = {"wav": wav, "spec": spec}                     # fresh tensors: later calls do not overwrite them
     ms_e2e, h2d, d2h = timed_e2e(ctx, model, host_p, lens, args.steps)
     t_c = time.monotonic()
 
@@ -455,6 +478,8 @@ def run_config2(ctx, args):
             line["fp32_mode"] = {"value": Bs * args.seconds * 2 / (ms32 / 1e3), "unit": UNIT, "ms_per_step": ms32 / 2,
                                  "batch": Bs, "dtype": "f32", "note": "precision='fp32': CUDA-core f32 kernels for every op "
                                  "(parity ~1e-6 vs the reference); bounded batch"}
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, outputs)
     _emit(line)
 
 
@@ -498,13 +523,16 @@ def run_config3(ctx, args):
     sampler.start()
     t_a = time.monotonic()
     per_batch = []
+    outputs = {}
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     for _ in range(args.steps):
-        for fs, x, lens in dev_batches:
+        for i, (fs, x, lens) in enumerate(dev_batches):
             a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-            a.record(); model(x, lens, fs); b.record()
+            a.record(); wav, spec = model(x, lens, fs); b.record()
             per_batch.append((fs, float(lens.sum()) / fs, a, b))
+            kind = ("full", "ragged")[i % 2]
+            outputs[f"wav_{fs}_{kind}"], outputs[f"spec_{fs}_{kind}"] = wav, spec
     e1.record()
     ctx.barrier()
     t_b = time.monotonic()
@@ -558,6 +586,8 @@ def run_config3(ctx, args):
                                  "on the recurrence's per-step dependency chain, not on the tensor pipe",
                          "peak_source": "MEASURED_PEAKS.json (bf16_tflops_sustained)"},
             "impl_notes": {"precision": args.precision, "launch": "host launches" if args.no_graph else "CUDA graph per batch signature"}}
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, outputs)
     _emit(line)
 
 
@@ -597,7 +627,7 @@ def run_config4(ctx, args):
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     for _ in range(args.steps):
-        m.enhance(y, FS, lens, N=args.nfe)
+        enhanced = m.enhance(y, FS, lens, N=args.nfe)
     e1.record()
     ctx.barrier()
     t_b = time.monotonic()
@@ -630,6 +660,8 @@ def run_config4(ctx, args):
                          "algorithmic_flops_per_step": flops, "peak_source": ctx.peak_source},
             "impl_notes": {"utterances_per_gpu": B, "nfe": args.nfe,
                            "launch": "host launches" if args.no_graph else "one network evaluation per CUDA-graph replay"}}
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"enhanced": enhanced})
     _emit(line)
 
 
@@ -662,11 +694,13 @@ def run_config5(ctx, args):
     e0, e1 = ev(), ev()
     e0.record()
     for _ in range(args.steps):
-        loss, _ = tr.step(noisy, clean, lens, fs_t)
+        loss, sisnr = tr.step(noisy, clean, lens, fs_t)
     e1.record()
     ctx.barrier()
     t_b = time.monotonic()
     ms = e0.elapsed_time(e1)
+    n_par = tr.flat.numel                                    # the passes below update the weights again: copy them now
+    outputs = {"loss": loss, "sisnr": sisnr, "params": tr.flat.flat[:n_par].clone(), "grads": tr.flat.grad[:n_par].clone()}
     # split of one step (separate EAGER pass: host launches, so the forward / backward shares are upper bounds of what
     # the graph replay spends there)
     a0, a1, a2, a3, a4 = ev(), ev(), ev(), ev(), ev()
@@ -712,6 +746,8 @@ def run_config5(ctx, args):
                                     "tensor-core step kernel per time step, split-K weight-gradient GEMMs",
                            "launch": "host launches" if args.no_graph else "CUDA graph replay of forward + loss + backward; "
                                      "allreduce and the fused clip+AdamW tail eager"}}
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, outputs)
     _emit(line)
 
 
@@ -755,9 +791,16 @@ def main():
     ap.add_argument("--no-fp32", action="store_true")
     ap.add_argument("--no-graph", action="store_true", help="launch every kernel from the host instead of replaying the "
                     "per-step kernel sequence from a captured CUDA graph")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last timed step computed "
+                    "as DIR/<name>.npy (float32 / float64, at most 64 MB in all: a fixed seeded sample of larger outputs); "
+                    "other files in DIR are kept, so give each run its own DIR")
     args = ap.parse_args()
     if args.steps is None:
         args.steps = {2: 3, 3: 2, 4: 1, 5: 5}[args.config]
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of --impl b200")
     ctx = Ctx(args)
     if args.impl == "reference":
         reference_arm(ctx, args)

@@ -51,6 +51,26 @@ def test_state_dict_layout_is_the_references():
     assert fm.dnn.t_cond[0].W.requires_grad is False
 
 
+def test_param_counts_are_the_published_ones():
+    """Our modules carry the parameter counts the reference publishes, conf/models/BSRNN_baseline.yaml:30-32:
+    'Parameters: 36.01795196533203 M' @48k, '32.0456657409668 M' @16k (unit 2**20, GroupNorm affine parameters not
+    counted), and the BSRNN_flowse.yaml model's 103 245 488 parameters."""
+    import types
+    from oracle import ref_loader
+    from urgent2026_challenge_track1_b200 import BSRNN_SE
+    from urgent2026_challenge_track1_b200.config import Config
+    from urgent2026_challenge_track1_b200.flow_model import FlowSEModel
+    b = BSRNN_SE(num_channel=196, num_layer=6).bsrnn.bsrnn
+    gn = {n for n, mod in b.named_modules() if isinstance(mod, torch.nn.GroupNorm)}
+    beyond_27 = lambda name: name.split(".")[0] in ("band_split", "mask_decoder") and int(name.split(".")[2]) >= 27
+    counted = [(n, p.numel()) for n, p in b.named_parameters() if n.rsplit(".", 1)[0] not in gn]
+    assert sum(c for _, c in counted) / 2 ** 20 == pytest.approx(36.01795196533203, abs=1e-9)
+    # @16 kHz only K'=27 bands of band_split / mask_decoder are touched
+    assert sum(c for n, c in counted if not beyond_27(n)) / 2 ** 20 == pytest.approx(32.0456657409668, abs=1e-9)
+    cfg = ref_loader.flowse_config(types.SimpleNamespace(Config=Config))
+    assert sum(p.numel() for p in FlowSEModel(cfg).parameters()) == 103_245_488
+
+
 def test_flowse_eval_swaps_ema_weights():
     from urgent2026_challenge_track1_b200.config import Config
     from urgent2026_challenge_track1_b200.flow_model import FlowSEModel
