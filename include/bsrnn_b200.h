@@ -144,6 +144,10 @@ int bsrnn_blstm_recurrence_f32(const float* gates_x, const float* w_hh, float* y
  *     8: epilogue 1 (f32 residual + statistics) with the tile's residual row segments moved by one bulk (TMA) copy
  *        per row into a shared-memory row buffer, updated there and stored back by one bulk store per row; rows must be
  *        16-byte aligned (ldo % 4 == 0, BN % 4 == 0, out 16-byte aligned)
+ *     Epilogues 0 and 4 store every column of every N tile (they do not clip at n_valid), so a call is rejected unless
+ *     n_tiles*BN <= ldo (epilogue 0) or n_tiles*BN <= 8*out_kcores (epilogue 4).  The row epilogues 1, 3, 7 and 8 (and
+ *     bsrnn_gemm_tc_scaled) need 0 < n_valid <= ldo.  Epilogue 2 writes k-cores < out_kcores only, with columns
+ *     n_valid .. 8*out_kcores - 1 stored as zeros when bias != NULL (the bias-free launches rely on zero weight rows there).
  * bsrnn_blstm_recurrence_tc: persistent cluster kernel, H = 392 only (csrc/lstm_tc.cu).  Sequences are grouped in
  *     tiles of 128 (seq = j*128 + r, valid iff seq < R); all operands are (step, seq_tile)-major:
  *       gates_x [step][seq_tile][dir][q][26][128][8] fp16 — epilogue 4 of bsrnn_gemm_tc over A tiles built with the

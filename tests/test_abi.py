@@ -63,6 +63,42 @@ def test_no_cpu_fallback(lib_path):
         m(torch.zeros(1, 4000), torch.tensor([4000]), 16000)
 
 
+# bsrnn_gemm_tc_ex calls whose epilogue would store outside what include/bsrnn_b200.h promises: (epilogue, n_tiles, BN, ldo,
+# n_valid, out_kcores, expected error).  Epilogues 0 and 4 store every column of every N tile.
+_OUT_OF_CONTRACT = {
+    "f16_rows_last_tile_past_ldo": (0, 2, 64, 120, 120, 0, "epilogue 0 stores"),
+    "f16_kb8_last_tile_past_out_kcores": (4, 2, 64, 0, 128, 15, "epilogue 4 stores"),
+    "resid_rows_overlap": (1, 1, 208, 192, 196, 0, "n_valid <= ldo"),
+    "resid_tma_rows_overlap": (8, 1, 208, 192, 196, 0, "n_valid <= ldo"),
+    "tanh_rows_overlap": (7, 1, 64, 40, 48, 0, "n_valid <= ldo"),
+    "glu_rows_overlap": (3, 1, 64, 20, 26, 0, "n_valid <= ldo"),
+}
+
+
+@pytest.mark.skipif(torch.cuda.is_available(), reason="on a GPU an accepted call would launch")
+@pytest.mark.parametrize("case", sorted(_OUT_OF_CONTRACT))
+def test_gemm_tc_rejects_out_of_contract_stores(lib_path, case):
+    from urgent2026_challenge_track1_b200 import _lib
+    epi, n_tiles, BN, ldo, n_valid, out_kcores, msg = _OUT_OF_CONTRACT[case]
+    h = _lib.lib()
+    p = 1 << 20                                          # never dereferenced: the call must fail its argument checks
+    rc = h.bsrnn_gemm_tc_ex(p, p, None, p, None, 2, n_tiles, 26, BN, epi, ldo, n_valid, out_kcores, 256, 2, 256, 1 << 40, 0, 1,
+                            0, 1, 0, None)
+    err = h.bsrnn_last_error().decode()
+    assert rc != 0 and msg in err, (rc, err)
+
+
+@pytest.mark.skipif(torch.cuda.is_available(), reason="on a GPU an accepted call would launch")
+@pytest.mark.parametrize("ksplit", [1, 4])
+def test_gemm_tc_scaled_rejects_overlapping_rows(lib_path, ksplit):
+    from urgent2026_challenge_track1_b200 import _lib
+    h = _lib.lib()
+    p = 1 << 20
+    rc = h.bsrnn_gemm_tc_scaled(p, p, None, p, 2, 1, 26, 208, 192, 196, 0.5, None, ksplit, 2, 256, 1 << 40, 0, 1, 0, None)
+    err = h.bsrnn_last_error().decode()
+    assert rc != 0 and "n_valid <= ldo" in err, (rc, err)
+
+
 def test_missing_library_raises(monkeypatch, tmp_path):
     from urgent2026_challenge_track1_b200 import _lib
     monkeypatch.setattr(_lib, "_lib", None)

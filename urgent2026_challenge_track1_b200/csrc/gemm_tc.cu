@@ -1243,6 +1243,15 @@ extern "C" int bsrnn_gemm_tc_ex(const void* A, const void* W, const float* bias,
   BSRNN_CHECK_ARG(tiles_per_step > 0 && seq_inner > 0 && tokens_per_sample > 0, "gemm_tc: bad row map");
   BSRNN_CHECK_ARG((epilogue != EPI_RESID_F32 && epilogue != EPI_TANH_F32 && epilogue != EPI_RESID_TMA) || (n_valid % 4 == 0 && ldo % 4 == 0),
                   "gemm_tc: the f32-row epilogues need n_valid and ldo to be multiples of 4 (got %d, %ld)", n_valid, ldo);
+  // the epilogues that do not clip at n_valid / out_kcores store every column of every N tile: reject a launch whose last tile
+  // would run into the next row (fp16 rows) or the next row tile (KB8), and row epilogues whose rows overlap
+  BSRNN_CHECK_ARG(epilogue != EPI_F16_ROWS || (long)n_tiles * BN <= ldo,
+                  "gemm_tc: epilogue 0 stores n_tiles*BN = %d columns per row, more than ldo = %ld", n_tiles * BN, ldo);
+  BSRNN_CHECK_ARG(epilogue != EPI_F16_KB8 || n_tiles * BN <= 8 * out_kcores,
+                  "gemm_tc: epilogue 4 stores n_tiles*BN = %d columns, more than 8*out_kcores = %d", n_tiles * BN, 8 * out_kcores);
+  BSRNN_CHECK_ARG((epilogue != EPI_RESID_F32 && epilogue != EPI_TANH_F32 && epilogue != EPI_RESID_TMA && epilogue != EPI_GLU_F32) ||
+                  (n_valid > 0 && ldo >= n_valid),
+                  "gemm_tc: the row epilogues need 0 < n_valid <= ldo (got %d, %ld)", n_valid, ldo);
   GemmTcArgs a{};
   a.A = reinterpret_cast<const __half*>(A);
   a.W = reinterpret_cast<const __half*>(W);
@@ -1357,6 +1366,7 @@ extern "C" int bsrnn_gemm_tc_scaled(const void* A, const void* W, const float* b
   BSRNN_CHECK_ARG(m_tiles > 0 && n_tiles > 0 && kcores > 0 && kcores % 2 == 0, "gemm_tc_scaled: bad tile counts (kcores=%d)", kcores);
   BSRNN_CHECK_ARG(BN >= 16 && BN <= 256 && BN % 16 == 0, "gemm_tc_scaled: BN=%d must be a multiple of 16 in [16,256]", BN);
   BSRNN_CHECK_ARG(tiles_per_step > 0 && seq_inner > 0 && n_valid % 4 == 0 && ldo % 4 == 0, "gemm_tc_scaled: bad row map / strides");
+  BSRNN_CHECK_ARG(n_valid > 0 && ldo >= n_valid, "gemm_tc_scaled: need 0 < n_valid <= ldo (got %d, %ld)", n_valid, ldo);
   GemmTcArgs a{};
   a.A = reinterpret_cast<const __half*>(A);
   a.W = reinterpret_cast<const __half*>(W);
