@@ -283,6 +283,17 @@ int bsrnn_blstm_fused768_tc(const void* xhat, const void* w_fused, const void* z
                             long y_stride, int R, int steps, int seq_tiles, int max_groups, int slots, void* sync_ws,
                             void* stream);
 int bsrnn_blstm_fused768_max_groups(void);
+/* bsrnn_blstm_fused768_train_tc: TRAINING forward of the H = 768 layer on the fused kernel: xhat, w_fused, zero_tile and
+ *     y_f / y_b / y_stride as bsrnn_blstm_fused768_tc (y_stride >= 96*1024, a multiple of 8), plus the activations BPTT
+ *     needs, written by the epilogue: gates rows [(step*seq_tiles + tile)*128 + r][8H] fp16 = ACTIVATED i, f, g, o at
+ *     column dir*4H + 4u + gate; c_f / c_b [step][seq_tiles*128][H] f32 -- the buffers bsrnn_blstm_train_bwd_tc reads
+ *     [autograd's saved tensors of nn.LSTM in FlowSEModel.training_step, flow_model.py:149-187].  sync_ws as
+ *     bsrnn_blstm_fused_tc; scratch as below. */
+int bsrnn_blstm_fused768_train_tc(const void* xhat, const void* w_fused, const void* zero_tile, void* y_f, void* y_b,
+                                  long y_stride, void* gates, float* c_f, float* c_b, void* scratch, int R, int steps,
+                                  int seq_tiles, int max_groups, int slots, void* sync_ws, void* stream);
+/* scratch of the call above in bytes (unit-major activations, as bsrnn_blstm_fused_train_scratch_bytes at H = 768). */
+long bsrnn_blstm_fused768_train_scratch_bytes(int steps, int seq_tiles);
 
 /* Debug / A-B timing: selects the recurrence schedule (4, 5, 6: 8-CTA clusters; 7: CTA pairs); any other value
  * returns to the BSRNN_LSTM_VER environment default. */

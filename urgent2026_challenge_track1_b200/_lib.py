@@ -61,6 +61,9 @@ PROTOTYPES = {
     "bsrnn_blstm_fused768_tc": [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_long, c_int, c_int, c_int, c_int, c_int,
                                 c_void_p, c_void_p],
     "bsrnn_blstm_fused768_max_groups": [],
+    "bsrnn_blstm_fused768_train_tc": [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_long, c_void_p, c_void_p, c_void_p,
+                                      c_void_p, c_int, c_int, c_int, c_int, c_int, c_void_p, c_void_p],
+    "bsrnn_blstm_fused768_train_scratch_bytes": [c_int, c_int],
     "bsrnn_blstm_fused7_tc": [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_void_p, c_void_p],
     "bsrnn_blstm_fused7_max_groups": [],
     "bsrnn_blstm_fused14_tc": [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_void_p, c_void_p],
@@ -139,6 +142,7 @@ def lib():
             fn.restype = c_int
         handle.bsrnn_launch_count.restype = C.c_long
         handle.bsrnn_blstm_fused_train_scratch_bytes.restype = C.c_long
+        handle.bsrnn_blstm_fused768_train_scratch_bytes.restype = C.c_long
         handle.bsrnn_last_error.restype = C.c_char_p
         handle.bsrnn_last_error.argtypes = []
         _lib = handle

@@ -52,6 +52,7 @@ namespace bsrnn {
 
 struct Geo392 {
   static constexpr bool SAVE = false;     // training forward: also write activated gates + c_t (the *S geometries)
+  static constexpr int H = 392;            // hidden size (unit-major stride of the saved activations)
   static constexpr int UPP = 49, BN = 208, PPG = 8, XKC = 26, HKC = 50, KS = 10, STAGES = 5;
   static constexpr int EPI_WARPS = 12, ACC = 256, NBUF = 2, EPI_REGS = 152, NC = 17;
   static constexpr int CLS = 2;             // cluster = one CTA pair
@@ -60,6 +61,7 @@ struct Geo392 {
 // direction of BASELINE config 2's time axis run 2-interleaved on 5 groups per direction instead of 3-interleaved on 3.
 struct Geo392x7 {
   static constexpr bool SAVE = false;     // training forward: also write activated gates + c_t (the *S geometries)
+  static constexpr int H = 392;
   static constexpr int UPP = 56, BN = 224, PPG = 7, XKC = 26, HKC = 50, KS = 10, STAGES = 4;
   static constexpr int EPI_WARPS = 16, ACC = 256, NBUF = 2, EPI_REGS = 104, NC = 14;
   static constexpr int CLS = 2;
@@ -70,12 +72,14 @@ struct Geo392x7 {
 // doubles - worthwhile only while few items are in flight (runtime_tc.fused_geometry).
 struct Geo392x14 {
   static constexpr bool SAVE = false;     // training forward: also write activated gates + c_t (the *S geometries)
+  static constexpr int H = 392;
   static constexpr int UPP = 28, BN = 112, PPG = 14, XKC = 26, HKC = 50, KS = 10, STAGES = 7;
   static constexpr int EPI_WARPS = 16, ACC = 128, NBUF = 4, EPI_REGS = 104, NC = 7;
   static constexpr int CLS = 2;
 };
 struct Geo768 {
   static constexpr bool SAVE = false;     // training forward: also write activated gates + c_t (the *S geometries)
+  static constexpr int H = 768;
   static constexpr int UPP = 32, BN = 128, PPG = 24, XKC = 50, HKC = 96, KS = 12, STAGES = 3;
   static constexpr int EPI_WARPS = 16, ACC = 128, NBUF = 4, EPI_REGS = 104, NC = 8;
   // -DBSRNN_FUSED768_CLS=4: clusters of 2 CTA pairs, the two CTAs of a parity fetch half of each ring stage and
@@ -89,6 +93,7 @@ struct Geo768 {
 struct Geo392x14M : Geo392x14 { static constexpr int CLS = 4; };
 struct Geo392x7S : Geo392x7 { static constexpr bool SAVE = true; };
 struct Geo392x14S : Geo392x14 { static constexpr bool SAVE = true; };
+struct Geo768S : Geo768 { static constexpr bool SAVE = true; };
 template <class G>
 struct Der {
   static constexpr int BH = G::BN / 2;                                  // B rows (gate columns) per CTA
@@ -127,7 +132,6 @@ struct FusedArgs {
   float* sv_c0;
   float* sv_c1;
 };
-constexpr int FH = 392;      // hidden size of the H = 392 geometries
 // saved activations, UNIT-major per (tile, direction): gates [tile][dir][unit][128 rows][4] fp16, c [tile][unit][128 rows] f32
 constexpr int SVG = 128 * 4, SVC = 128;
 
@@ -305,18 +309,20 @@ __device__ __forceinline__ void epif_item392x14(uint32_t t_col, __half* ycore, f
   }
 }
 // H = 768: thread = (row r, quarter T of the pair's 32 units): 8 units = 32 accumulator columns = one 16-byte row of
-// k-core 4q + T of the y tile.
-__device__ __forceinline__ void epif_item768(uint32_t t_col, __half* ycore, float (&c)[8], bool st) {
+// k-core 4q + T of the y tile.  SAVE: the activated gates / c_t of unit u0 + u (u0 = 32q + 8T) go to sg + 4*u / sc + u.
+template <bool SAVE = false>
+__device__ __forceinline__ void epif_item768(uint32_t t_col, __half* ycore, float (&c)[8], bool st, __half* sg = nullptr,
+                                             float* sc = nullptr) {
   float h[8];
   uint32_t accA[16], accB[16];
   tmem_ld_x16(t_col, accA);
   tmem_ld_wait();
   tmem_ld_x16(t_col + 16, accB);
   tmem_ld_pin16(accA);
-  epif_chunk<0>(accA, c, h);
+  epif_chunk_sv<0, 8, 8, SAVE>(accA, c, h, sg, sc, st);
   tmem_ld_wait();
   tmem_ld_pin16(accB);
-  epif_chunk<1>(accB, c, h);
+  epif_chunk_sv<1, 8, 8, SAVE>(accB, c, h, sg, sc, st);
   if (st)
     *reinterpret_cast<uint4*>(ycore) = make_uint4(pack_h2(h[0], h[1]), pack_h2(h[2], h[3]), pack_h2(h[4], h[5]), pack_h2(h[6], h[7]));
 }
@@ -366,8 +372,8 @@ __device__ __forceinline__ void epiloguef_role(const FusedArgs& a, uint32_t tmem
             __half* sg = nullptr; float* sc = nullptr;
             if constexpr (G::SAVE) {
               const int u0 = 56 * q + 14 * T;
-              sg = a.sv_gates + (((tile * 2 + GR.d) * FH + u0) * 128 + (size_t)r) * 4;
-              sc = (GR.d == 0 ? a.sv_c0 : a.sv_c1) + (tile * FH + u0) * 128 + (size_t)r;
+              sg = a.sv_gates + (((tile * 2 + GR.d) * G::H + u0) * 128 + (size_t)r) * 4;
+              sc = (GR.d == 0 ? a.sv_c0 : a.sv_c1) + (tile * G::H + u0) * 128 + (size_t)r;
             }
             if (k == 0) epif_item392x7<Q, G::SAVE>(t_lane + buf * G::ACC, ycore, c0, valid, sg, sc);
             else if (k == 1) epif_item392x7<Q, G::SAVE>(t_lane + buf * G::ACC, ycore, c1, valid, sg, sc);
@@ -376,16 +382,22 @@ __device__ __forceinline__ void epiloguef_role(const FusedArgs& a, uint32_t tmem
             __half* sg = nullptr; float* sc = nullptr;
             if constexpr (G::SAVE) {
               const int u0 = 28 * q + 7 * T;
-              sg = a.sv_gates + (((tile * 2 + GR.d) * FH + u0) * 128 + (size_t)r) * 4;
-              sc = (GR.d == 0 ? a.sv_c0 : a.sv_c1) + (tile * FH + u0) * 128 + (size_t)r;
+              sg = a.sv_gates + (((tile * 2 + GR.d) * G::H + u0) * 128 + (size_t)r) * 4;
+              sc = (GR.d == 0 ? a.sv_c0 : a.sv_c1) + (tile * G::H + u0) * 128 + (size_t)r;
             }
             if (k == 0) epif_item392x14<Q / 4, Q % 4, G::SAVE>(t_lane + buf * G::ACC, ycore, c0, valid, sg, sc);
             else if (k == 1) epif_item392x14<Q / 4, Q % 4, G::SAVE>(t_lane + buf * G::ACC, ycore, c1, valid, sg, sc);
             else epif_item392x14<Q / 4, Q % 4, G::SAVE>(t_lane + buf * G::ACC, ycore, c2, valid, sg, sc);
           } else {
-            if (k == 0) epif_item768(t_lane + buf * G::ACC, ycore, c0, valid);
-            else if (k == 1) epif_item768(t_lane + buf * G::ACC, ycore, c1, valid);
-            else epif_item768(t_lane + buf * G::ACC, ycore, c2, valid);
+            __half* sg = nullptr; float* sc = nullptr;
+            if constexpr (G::SAVE) {
+              const int u0 = 32 * q + 8 * T;
+              sg = a.sv_gates + (((tile * 2 + GR.d) * G::H + u0) * 128 + (size_t)r) * 4;
+              sc = (GR.d == 0 ? a.sv_c0 : a.sv_c1) + (tile * G::H + u0) * 128 + (size_t)r;
+            }
+            if (k == 0) epif_item768<G::SAVE>(t_lane + buf * G::ACC, ycore, c0, valid, sg, sc);
+            else if (k == 1) epif_item768<G::SAVE>(t_lane + buf * G::ACC, ycore, c1, valid, sg, sc);
+            else epif_item768<G::SAVE>(t_lane + buf * G::ACC, ycore, c2, valid, sg, sc);
           }
           tc_fence_before();
           __syncwarp();
@@ -858,6 +870,7 @@ extern "C" int bsrnn_blstm_fused768_max_groups(void) { return fused_max_groups<G
 
 namespace bsrnn {
 // unit-major scratch of the SAVE kernels -> the row-major buffers of bsrnn_blstm_train_bwd_tc.  grid (tiles, 2 directions).
+template <int H>
 __global__ void __launch_bounds__(256) saved_transpose_kernel(const uint2* __restrict__ gT, const float* __restrict__ cT0,
                                                              const float* __restrict__ cT1, uint2* __restrict__ gates,
                                                              float* __restrict__ c0, float* __restrict__ c1) {
@@ -865,16 +878,16 @@ __global__ void __launch_bounds__(256) saved_transpose_kernel(const uint2* __res
   __shared__ float tc[32][33];
   const int tile = blockIdx.x, d = blockIdx.y;
   const int tx = threadIdx.x & 31, ty = threadIdx.x >> 5;                 // 32 x 8
-  const uint2* sg = gT + ((size_t)(tile * 2 + d) * FH) * 128;             // [unit][row]
-  const float* sc = (d == 0 ? cT0 : cT1) + (size_t)tile * FH * 128;
-  uint2* dg = gates + (size_t)tile * 128 * (2 * FH) + (size_t)d * FH;     // row stride 2*FH uint2 (= 8H halves)
-  float* dc = (d == 0 ? c0 : c1) + (size_t)tile * 128 * FH;
-  for (int u0 = 0; u0 < FH; u0 += 32) {
+  const uint2* sg = gT + ((size_t)(tile * 2 + d) * H) * 128;              // [unit][row]
+  const float* sc = (d == 0 ? cT0 : cT1) + (size_t)tile * H * 128;
+  uint2* dg = gates + (size_t)tile * 128 * (2 * H) + (size_t)d * H;       // row stride 2*H uint2 (= 8H halves)
+  float* dc = (d == 0 ? c0 : c1) + (size_t)tile * 128 * H;
+  for (int u0 = 0; u0 < H; u0 += 32) {
     for (int r0 = 0; r0 < 128; r0 += 32) {
 #pragma unroll
       for (int k = 0; k < 4; ++k) {
         const int u = u0 + ty + 8 * k;
-        if (u < FH) {
+        if (u < H) {
           tg[ty + 8 * k][tx] = sg[(size_t)u * 128 + r0 + tx];
           tc[ty + 8 * k][tx] = sc[(size_t)u * 128 + r0 + tx];
         }
@@ -883,14 +896,39 @@ __global__ void __launch_bounds__(256) saved_transpose_kernel(const uint2* __res
 #pragma unroll
       for (int k = 0; k < 4; ++k) {
         const int r = r0 + ty + 8 * k, u = u0 + tx;
-        if (u < FH) {
-          dg[(size_t)r * (2 * FH) + u] = tg[tx][ty + 8 * k];
-          dc[(size_t)r * FH + u] = tc[tx][ty + 8 * k];
+        if (u < H) {
+          dg[(size_t)r * (2 * H) + u] = tg[tx][ty + 8 * k];
+          dc[(size_t)r * H + u] = tc[tx][ty + 8 * k];
         }
       }
       __syncthreads();
     }
   }
+}
+
+// scratch of a SAVE launch: unit-major gates (2 directions x 4H halves per row) + c_t (2 directions x H floats per row)
+template <int H>
+static long fused_train_scratch_bytes(int steps, int seq_tiles) {
+  return (long)steps * seq_tiles * 128 * H * (2 * 4 * 2 + 2 * 4);
+}
+
+// SAVE launch of geometry G, then the transpose of its scratch into gates / c_f / c_b
+template <class G>
+static int run_fused_train(const char* what, const void* xhat, const void* w_fused, const void* zero_tile, void* y_f, void* y_b,
+                           long y_stride, void* gates, float* c_f, float* c_b, void* scratch, int R, int steps, int seq_tiles,
+                           int max_groups, int slots, void* sync_ws, void* stream) {
+  static_assert(G::SAVE, "training forward needs a SAVE geometry");
+  const size_t m_all = (size_t)steps * seq_tiles;
+  __half* gT = reinterpret_cast<__half*>(scratch);
+  float* cT0 = reinterpret_cast<float*>(gT + m_all * 128 * 8 * G::H);
+  float* cT1 = cT0 + m_all * 128 * G::H;
+  const int rc = run_fused<G>(what, xhat, w_fused, zero_tile, y_f, y_b, y_stride, R, steps, seq_tiles, max_groups, slots, sync_ws,
+                              stream, gT, cT0, cT1);
+  if (rc) return rc;
+  saved_transpose_kernel<G::H><<<dim3((unsigned)m_all, 2), 256, 0, (cudaStream_t)stream>>>(
+      reinterpret_cast<const uint2*>(gT), cT0, cT1, reinterpret_cast<uint2*>(gates), c_f, c_b);
+  BSRNN_LAUNCH_OK();
+  return 0;
 }
 }  // namespace bsrnn
 
@@ -901,7 +939,7 @@ __global__ void __launch_bounds__(256) saved_transpose_kernel(const uint2* __res
 // bsrnn_blstm_train_bwd_tc reads [replaces autograd's saved tensors of nn.LSTM, d_model.py:61-95 / train_se.py:74-84].
 // scratch: (2 * steps*seq_tiles*128*4H halves) + (2 * steps*seq_tiles*128*H floats) = bsrnn_blstm_fused_train_scratch_bytes().
 extern "C" long bsrnn_blstm_fused_train_scratch_bytes(int steps, int seq_tiles) {
-  return (long)steps * seq_tiles * 128 * FH * (2 * 4 * 2 + 2 * 4);
+  return fused_train_scratch_bytes<392>(steps, seq_tiles);
 }
 extern "C" int bsrnn_blstm_fused_train_tc(int geo, const void* xhat, const void* w_fused, const void* zero_tile, void* y_f,
                                           void* y_b, long y_stride, void* gates, float* c_f, float* c_b, void* scratch, int R,
@@ -910,17 +948,25 @@ extern "C" int bsrnn_blstm_fused_train_tc(int geo, const void* xhat, const void*
   BSRNN_CHECK_ARG(R > 0 && steps > 0 && (long)seq_tiles * 128 >= R, "blstm_fused_train_tc: bad dims");
   BSRNN_CHECK_ARG(geo == 7 || geo == 14, "blstm_fused_train_tc: geo must be 7 or 14");
   BSRNN_CHECK_ARG(y_stride >= (long)Geo392x7::HKC * 128 * 8 && y_stride % 8 == 0, "blstm_fused_train_tc: bad y_stride");
-  const size_t m_all = (size_t)steps * seq_tiles;
-  __half* gT = reinterpret_cast<__half*>(scratch);
-  float* cT0 = reinterpret_cast<float*>(gT + m_all * 128 * 8 * FH);
-  float* cT1 = cT0 + m_all * 128 * FH;
-  const int rc = geo == 7 ? run_fused<Geo392x7S>("blstm_fused_train_tc", xhat, w_fused, zero_tile, y_f, y_b, y_stride, R, steps, seq_tiles,
-                                                 max_groups, slots, sync_ws, stream, gT, cT0, cT1)
-                          : run_fused<Geo392x14S>("blstm_fused_train_tc", xhat, w_fused, zero_tile, y_f, y_b, y_stride, R, steps, seq_tiles,
-                                                  max_groups, slots, sync_ws, stream, gT, cT0, cT1);
-  if (rc) return rc;
-  saved_transpose_kernel<<<dim3((unsigned)m_all, 2), 256, 0, (cudaStream_t)stream>>>(
-      reinterpret_cast<const uint2*>(gT), cT0, cT1, reinterpret_cast<uint2*>(gates), c_f, c_b);
-  BSRNN_LAUNCH_OK();
-  return 0;
+  return geo == 7 ? run_fused_train<Geo392x7S>("blstm_fused_train_tc", xhat, w_fused, zero_tile, y_f, y_b, y_stride, gates, c_f, c_b,
+                                               scratch, R, steps, seq_tiles, max_groups, slots, sync_ws, stream)
+                  : run_fused_train<Geo392x14S>("blstm_fused_train_tc", xhat, w_fused, zero_tile, y_f, y_b, y_stride, gates, c_f, c_b,
+                                                scratch, R, steps, seq_tiles, max_groups, slots, sync_ws, stream);
+}
+
+// Training forward of the BLSTM layer at H = 768 / N = 384 (BSRNN_flowse) on the fused kernel (Geo768S): xhat, w_fused,
+// zero_tile, y_f / y_b / y_stride as bsrnn_blstm_fused768_tc; gates [(step*seq_tiles + tile)*128 + r][8H] fp16 and c_f / c_b
+// [step][seq_tiles*128][H] f32 as bsrnn_blstm_fused_train_tc.  scratch: bsrnn_blstm_fused768_train_scratch_bytes().
+extern "C" long bsrnn_blstm_fused768_train_scratch_bytes(int steps, int seq_tiles) {
+  return fused_train_scratch_bytes<768>(steps, seq_tiles);
+}
+extern "C" int bsrnn_blstm_fused768_train_tc(const void* xhat, const void* w_fused, const void* zero_tile, void* y_f, void* y_b,
+                                             long y_stride, void* gates, float* c_f, float* c_b, void* scratch, int R, int steps,
+                                             int seq_tiles, int max_groups, int slots, void* sync_ws, void* stream) {
+  BSRNN_CHECK_ARG(xhat && w_fused && zero_tile && y_f && y_b && gates && c_f && c_b && sync_ws && scratch,
+                  "blstm_fused768_train_tc: null pointer");
+  BSRNN_CHECK_ARG(R > 0 && steps > 0 && (long)seq_tiles * 128 >= R, "blstm_fused768_train_tc: bad dims");
+  BSRNN_CHECK_ARG(y_stride >= (long)Geo768::HKC * 128 * 8 && y_stride % 8 == 0, "blstm_fused768_train_tc: bad y_stride");
+  return run_fused_train<Geo768S>("blstm_fused768_train_tc", xhat, w_fused, zero_tile, y_f, y_b, y_stride, gates, c_f, c_b,
+                                  scratch, R, steps, seq_tiles, max_groups, slots, sync_ws, stream);
 }

@@ -130,13 +130,18 @@ class FlowSEModel(nn.Module):
         assert clean.shape[1] == 1                                               # flow_model.py:153
         return flowse_forward_step(self, noisy, clean, lengths, int(fs), t=t, z=z)[0]
 
-    def configure_optimizers(self, process_group=None):
-        """AdamW(lr, eps=adam_epsilon, weight_decay) [flow_model.py:238-249] + EMA [:84] as one FlowSETrainer."""
+    def configure_optimizers(self, process_group=None, precision=None, cuda_graph=False):
+        """AdamW(lr, eps=adam_epsilon, weight_decay) [flow_model.py:238-249] + EMA [:84] as one FlowSETrainer.
+        precision: "fp32" (f32 recurrence kernels) or "fp16" / "bf16" (the BLSTM blocks on tensor cores); None reads
+        ``cfg.train_precision`` (default "fp32").  cuda_graph: replay forward + loss + backward as one CUDA graph."""
         from .training import FlowSETrainer
         cfg = self.cfg
+        if precision is None:
+            precision = getattr(cfg, "train_precision", "fp32")
         self.trainer_ = FlowSETrainer(self, weight_decay=getattr(cfg, "weight_decay", 1e-6),
                                       eps=getattr(cfg, "adam_epsilon", 1e-8),
-                                      gradient_clip=getattr(cfg, "gradient_clip", 0.5), process_group=process_group)
+                                      gradient_clip=getattr(cfg, "gradient_clip", 0.5), process_group=process_group,
+                                      precision=precision, cuda_graph=cuda_graph)
         return self.trainer_
 
     def training_step(self, batch, batch_idx=0):

@@ -1,8 +1,15 @@
-"""train_se — entry point mirroring ``baseline_code/train_se.py`` (reference train_se.py:37-84) for the discriminative
-BSRNN model: ``--config_file conf/models/BSRNN_baseline.yaml`` plus every Config field as a flag; one process per GPU
+"""train_se — entry point mirroring ``baseline_code/train_se.py`` (reference train_se.py:37-84) for both models it
+selects by ``model_type`` (:50-53): the discriminative BSRNN (``se``, default) and BSRNN-FlowSE (``flowse``).
+``--config_file conf/models/BSRNN_baseline.yaml`` plus every Config field as a flag; one process per GPU
 under torchrun (the reference lets Lightning spawn them), gradients averaged with ONE NCCL allreduce of the flat
 buffer per step; ``init_from`` accepts a raw or Lightning-style state_dict (:55-60); checkpoints are written in the
 reference's layout ``{"state_dict": ..., "hyper_parameters": {"cfg": cfg}}``.
+
+FlowSE (``model_type: flowse``) trains with the flow-matching loss, AdamW and the EMA fused into the optimizer tail, the
+forward + loss + backward replayed as one CUDA graph.  Its BLSTM blocks run at the precision of the YAML key
+``train_precision`` (default ``fp16``: tensor cores, f32 master weights; ``fp32``: the f32 recurrence kernels).  Its
+checkpoints carry the EMA weights under ``ema`` (flow_model.py:87-96), so FlowSEModel.load_from_checkpoint and
+inference.py read them as they read the reference's.
 
 The reference's data pipeline (dataset.py, dynamic mixing, simulation/) is out of scope (SURVEY.md §2 row 9): pass
 ``--data synthetic`` (default) for random (clean, noisy) pairs of the dataset contract — (clean (B,1,T), noisy (B,1,T),
@@ -48,6 +55,24 @@ def fit(model: SEModel, batches, cfg, rank=0, log_every=10, out_dir=None):
     return last
 
 
+def fit_flowse(model, batches, cfg, rank=0, log_every=10, out_dir=None):
+    """FlowSEModel training loop: FlowSETrainer steps (fp16 tensor-core blocks by default, CUDA-graph replay); at the
+    end rank 0 writes ``last-step<N>.ckpt`` with the EMA state (``trainer.sync_ema()`` first)."""
+    from .checkpoint import save_checkpoint
+    trainer = model.configure_optimizers(precision=getattr(cfg, "train_precision", "fp16"), cuda_graph=True)
+    last = None
+    for step, (clean, noisy, fs, lengths) in enumerate(batches):
+        last, _ = trainer.step(noisy, clean, lengths, fs)
+        if rank == 0 and step % log_every == 0:
+            print(f"step {step}: train_loss={float(last):.4g}", flush=True)
+    if out_dir and rank == 0:
+        trainer.sync_ema()
+        os.makedirs(out_dir, exist_ok=True)
+        save_checkpoint(os.path.join(out_dir, f"last-step{trainer.step_count:06d}.ckpt"), model, cfg,
+                        global_step=trainer.step_count, ema=model.ema.state_dict())
+    return last
+
+
 def main(argv=None):
     import torch.distributed as dist
     args = config_parser(argv)
@@ -62,9 +87,12 @@ def main(argv=None):
     dev = torch.device("cuda", local)
     if world > 1:
         dist.init_process_group("nccl", device_id=dev)
-    if getattr(cfg, "model_type", "se") == "flowse":
-        raise NotImplementedError("FlowSE training is not built yet (DESIGN.md §7); this entry point trains SEModel")
-    model = SEModel(cfg, precision="fp32")
+    flowse = getattr(cfg, "model_type", "se") == "flowse"
+    if flowse:
+        from .flow_model import FlowSEModel
+        model = FlowSEModel(cfg)
+    else:
+        model = SEModel(cfg, precision="fp32")
     if cfg.init_from != "none":
         sd = torch.load(cfg.init_from, map_location="cpu", weights_only=False)
         model.load_state_dict(sd.get("state_dict", sd))
@@ -74,7 +102,8 @@ def main(argv=None):
             dist.broadcast(p.data, 0)
     steps = int(getattr(cfg, "max_steps", 20))
     out_dir = os.path.join("exp", cfg.train_tag, cfg.train_name, f"version_{cfg.train_version}", "checkpoints")
-    fit(model, synthetic_batches(cfg, rank, world, steps, dev), cfg, rank, out_dir=out_dir if getattr(cfg, "save", False) else None)
+    (fit_flowse if flowse else fit)(model, synthetic_batches(cfg, rank, world, steps, dev), cfg, rank,
+                                    out_dir=out_dir if getattr(cfg, "save", False) else None)
     if world > 1:
         dist.destroy_process_group()
 

@@ -201,7 +201,46 @@ def mask_decoder_batched(md, skip, plan, F_bins):
     return outs[0], outs[1]
 
 
-BATCHED_BANDS = os.environ.get("BSRNN_TRAIN_BATCHED_BANDS", "1") == "1"   # 0: the per-band loops (band_split_diff, mask_decoder_diff)
+def grad_decoder_batched(gd, skip, plan, F_bins):
+    """grad_decoder_diff with the 2 x K' per-band GN -> Conv1d(N, 16 s) -> tanh as one set of reductions and one batched
+    GEMM per family.  Each band's 16 s output channels (channel c = 16-index * s + f) are padded per sub-channel to
+    16 smax, so that one reshape turns the GEMM output into (B,16,K smax,T); a gather then keeps the sum(s_k) real bins,
+    the padded tail of a truncated last band included (the 5x5 Conv2d sees it, as in the per-band loop).  The Conv2d +
+    GLU stays one torch op per family."""
+    B, T, K, N = skip.shape
+    sc = gd.sub_channel
+    tb = _band_tables(plan, skip.device)
+    smax = tb["smax"]
+    sel = tb.get("sel_all")
+    if sel is None:                                   # every bin of the K' bands (F' = sum s_k >= F), (band, bin) order
+        sel = tb["sel_all"] = torch.tensor([k * smax + f for k in range(K) for f in range(plan.subbands[k])], dtype=torch.long,
+                                           device=skip.device)
+    mean = skip.mean(dim=(1, 3), keepdim=True)
+    d = skip - mean
+    var = (d * d).mean(dim=(1, 3), keepdim=True)
+    outs = []
+    for mlps, conv in ((gd.mlp_mask, gd.conv_after_mask), (gd.mlp_residual, gd.conv_after_residual)):
+        gamma = torch.stack([mlps[k][0].weight for k in range(K)])              # (K,N)
+        beta = torch.stack([mlps[k][0].bias for k in range(K)])
+        xn = d * torch.rsqrt(var + mlps[0][0].eps) * gamma + beta               # (B,T,K,N)
+        W, b = [], []
+        for k in range(K):
+            s = plan.subbands[k]
+            W.append(F.pad(mlps[k][1].weight[:, :, 0].reshape(sc, s, N), (0, 0, 0, smax - s)).reshape(sc * smax, N))
+            b.append(F.pad(mlps[k][1].bias.reshape(sc, s), (0, smax - s)).reshape(sc * smax))
+        W, b = torch.stack(W), torch.stack(b)                                   # (K,16 smax,N), (K,16 smax)
+        h = torch.tanh(torch.bmm(xn.permute(2, 0, 1, 3).reshape(K, B * T, N), W.transpose(1, 2)) + b[:, None, :])
+        g = h.reshape(K, B, T, sc, smax).permute(1, 3, 0, 4, 2).reshape(B, sc, K * smax, T)[:, :, sel, :]   # (B,16,F',T)
+        g = F.glu(F.conv2d(g, conv[0].weight, conv[0].bias, padding=2), dim=1)   # (B,2,F',T)
+        g = g.permute(0, 3, 2, 1)                                                # (B,T,F',2)
+        if g.shape[2] < F_bins:
+            g = F.pad(g, (0, 0, 0, F_bins - g.shape[2]))
+        outs.append(torch.view_as_complex(g[:, :, :F_bins, :].contiguous()))
+    return outs[0], outs[1]
+
+
+# 0: the per-band loops (band_split_diff, mask_decoder_diff, grad_decoder_diff)
+BATCHED_BANDS = os.environ.get("BSRNN_TRAIN_BATCHED_BANDS", "1") == "1"
 
 
 def block_f32(x, rnn, fc, axis):
@@ -331,7 +370,7 @@ def flow_bsrnn_train_forward(dnn, x_btf, y_btf, t, blstm_fn=None):
         proj = t[:, None] * dnn.t_cond[i].W[None, :] * 2 * math.pi
         t_emb.append(torch.cat([torch.sin(proj), torch.cos(proj)], dim=-1))
     skip = dual_path_diff(dnn, skip, t_emb=t_emb, blstm_fn=blstm_fn)
-    m_c, r_c = grad_decoder_diff(dnn.grad_decoder, skip, plan, F_bins)
+    m_c, r_c = (grad_decoder_batched if BATCHED_BANDS else grad_decoder_diff)(dnn.grad_decoder, skip, plan, F_bins)
     return m_c * torch.view_as_complex(x_btf.contiguous()) + r_c
 
 

@@ -11,8 +11,9 @@ tcgen05 kernels of csrc/gemm_tc.cu with fp16 operands, f32 accumulation and f32 
             dG tiles (KB8) --gemm_tc_scaled--> dx ;  dW_ih = dG^T xhat, dW_hh = dG^T h_prev, dW_fc = d_out^T y through
             bsrnn_kb8_transpose (tokens become the K axis) + gemm_tc_scaled (1/S removed in f32).
 
-The recurrence is step-wise (one launch per time step, both directions), for any hidden size with H % 8 == 0 (K padded to 16) -- the
-same kernels serve BSRNN (H = 392) and FlowSE (H = 768).  Only bias gradients (two small reductions) use torch ops.
+The step-wise recurrence (one launch per time step, both directions) serves any hidden size with H % 8 == 0 (K padded to 16) -- the
+same kernels serve BSRNN (H = 392) and FlowSE (H = 768).  At the two published widths the forward instead runs on the persistent
+fused layer kernel (input projection + every step in one launch); BPTT stays step-wise.  Only bias gradients (two small reductions) use torch ops.
 Gradients are loss-scaled by a power of two chosen per call from max|d_out| so that fp16 neither overflows nor flushes.
 """
 from __future__ import annotations
@@ -63,14 +64,18 @@ def _gate_tables(H, dev):
 def pack_block(w_ih, w_hh, b_ih, b_hh, w_ih_r, w_hh_r, b_ih_r, b_hh_r, fc_w, narrow_bwd=False, fwd_steps=True):
     """All tensor-core operands of one block, from the f32 master weights (nn.LSTM / nn.Linear layouts).
     narrow_bwd: BPTT output tiles of 64 hidden units instead of up to 256 (few row tiles = small batch: more CTAs share a
-    step and each epilogue warp owns a single 32-unit chunk)."""
+    step and each epilogue warp owns a single 32-unit chunk).
+    fwd_steps=False (the fused forward): the input operand carries the constant-one bias column N, so kc_in and the
+    x^T tiles (bn_n x nt_n rows) cover N + 1 columns.  At N = 196 that column sits in the padding already; at N = 384
+    it needs two more k-cores (kc_in = 50), and every operand built on kc_in (dD, fcT, xT) follows."""
     H, N = w_hh.shape[1], w_ih.shape[1]
     if H % 8:
         raise NotImplementedError(f"tensor-core training BLSTM needs H % 8 == 0, got {H}")
     kc_h = (H + 15) // 16 * 2                        # k-cores of an h tile: K padded to a multiple of 16, pad core = 0
     dev = w_hh.device
     perm, gsc = _gate_tables(H, dev)
-    kc_in = (N + 15) // 16 * 2
+    n_in = N if fwd_steps else N + 1                 # + the constant-one column of the fused forward's operand
+    kc_in = (n_in + 15) // 16 * 2
     BN = _bn_div(4 * H, 32)
     bn_h, nt_h = _bn_cover(H, 32)                    # BPTT output tiles over the H hidden units (32-column chunks)
     if narrow_bwd and H > 64:
@@ -79,7 +84,7 @@ def pack_block(w_ih, w_hh, b_ih, b_hh, w_ih_r, w_hh_r, b_ih_r, b_hh_r, fc_w, nar
         bn_h = NARROW_BN if NARROW_BN > 0 else (32 if isinstance(narrow_bwd, int) and not isinstance(narrow_bwd, bool)
                                                  and 2 * narrow_bwd * ((H + 31) // 32) <= 148 else 64)
         nt_h = (H + bn_h - 1) // bn_h
-    bn_n, nt_n = _bn_cover(N, 16)
+    bn_n, nt_n = _bn_cover(n_in, 16)
     p = dict(H=H, N=N, kc_in=kc_in, kc_h=kc_h, BN=BN, n_tiles=4 * H // BN, bn_h=bn_h, nt_h=nt_h, bn_n=bn_n, nt_n=nt_n, perm=perm)
     wih, bias, whh, whhT, wihT = [], [], [], [], []
     for wi, wh, bi, bh in ((w_ih, w_hh, b_ih, b_hh), (w_ih_r, w_hh_r, b_ih_r, b_hh_r)):
@@ -102,18 +107,24 @@ def pack_block(w_ih, w_hh, b_ih, b_hh, w_ih_r, w_hh_r, b_ih_r, b_hh_r, fc_w, nar
     return p
 
 
-# BLSTM forward of the training step on the fused layer kernel (bsrnn_blstm_fused_train_tc, H = 392): one persistent launch per
-# block instead of one input-projection GEMM + one launch per time step.  BSRNN_TRAIN_FUSED=0: the step-wise forward.
+# BLSTM forward of the training step on the fused layer kernel (bsrnn_blstm_fused_train_tc at H = 392,
+# bsrnn_blstm_fused768_train_tc at H = 768 / N = 384): one persistent launch per block instead of one input-projection GEMM
+# + one launch per time step.  BSRNN_TRAIN_FUSED=0: the step-wise forward.
 FUSED_TRAIN = os.environ.get("BSRNN_TRAIN_FUSED", "1") == "1"
 _FUSED_IDX = {}
 
 
+FUSED_GEO = {7: (7, 56), 14: (14, 28), 768: (24, 32)}      # geometry -> (pairs per group, hidden units per pair)
+
+
 def pack_fused_train(ws, geo, kc_in, one_col):
-    """pack_lstm_fused7's layout ([dir][pair q][half e][kc_in + 50 k-cores][2U rows][8] fp16) from the 8 raw LSTM tensors
-    (w_ih, w_hh, b_ih, b_hh, and the reverse four) in a handful of batched ops: it runs inside every training step."""
+    """pack_lstm_fused7's / pack_lstm_fused768's layout ([dir][pair q][half e][kc_in + kc_h k-cores][2U rows][8] fp16,
+    kc_h = 50 at H = 392, 96 at H = 768) from the 8 raw LSTM tensors (w_ih, w_hh, b_ih, b_hh, and the reverse four) in a
+    handful of batched ops, without a host synchronisation: it runs inside every (captured) training step."""
     w_ih, w_hh, b_ih, b_hh, w_ih_r, w_hh_r, b_ih_r, b_hh_r = ws
     H, N = w_hh.shape[1], w_ih.shape[1]
-    P, U = (7, 56) if geo == 7 else (14, 28)
+    P, U = FUSED_GEO[geo]
+    kc_h = (H + 15) // 16 * 2
     dev = w_hh.device
     key = (H, P, U, str(dev))
     t = _FUSED_IDX.get(key)
@@ -125,17 +136,14 @@ def pack_fused_train(ws, geo, kc_in, one_col):
         gsc = torch.tensor(GATE_SCALE, device=dev).repeat(U)[None, None, :, None]
         t = _FUSED_IDX[key] = (rows, gsc)
     rows, gsc = t
-    ktot = (kc_in + LKC_H) * 8
+    ktot = (kc_in + kc_h) * 8
     full = torch.zeros(2, 4 * H, ktot, dtype=torch.float32, device=dev)
     for d, (wi, wh, bi, bh) in enumerate(((w_ih, w_hh, b_ih, b_hh), (w_ih_r, w_hh_r, b_ih_r, b_hh_r))):
         full[d, :, :N] = wi.detach().float()
         full[d, :, one_col] = (bi.detach() + bh.detach()).float()
         full[d, :, kc_in * 8: kc_in * 8 + H] = wh.detach().float()
     w = full[:, rows] * gsc                                               # (2, P, 4U, ktot)
-    return w.view(2, P, 2, 2 * U, kc_in + LKC_H, 8).permute(0, 1, 2, 4, 3, 5).contiguous().to(torch.float16)
-
-
-LKC_H = 50                    # k-cores of the H = 392 recurrent operand (K = 400)
+    return w.view(2, P, 2, 2 * U, kc_in + kc_h, 8).permute(0, 1, 2, 4, 3, 5).contiguous().to(torch.float16)
 
 
 def _geom(B, T, K, axis):
@@ -182,9 +190,10 @@ class BLSTMBlockTC(torch.autograd.Function):
         st = L.stream_ptr()
         R, steps, tiles, addr = _geom(B, T, K, axis)
         Hh, Nn = w_hh.shape[1], w_ih.shape[1]
-        fused = FUSED_TRAIN and Hh == 392 and Nn % 4 == 0 and Nn % 16 != 0
+        fused = FUSED_TRAIN and ((Hh == 392 and Nn % 4 == 0 and Nn % 16 != 0) or (Hh == 768 and Nn == 384))
         with torch.profiler.record_function("tc_pack_block"):
-            p = pack_block(w_ih, w_hh, b_ih, b_hh, w_ih_r, w_hh_r, b_ih_r, b_hh_r, fc_w, narrow_bwd=(tiles if tiles <= 16 else False), fwd_steps=not fused)
+            p = pack_block(w_ih, w_hh, b_ih, b_hh, w_ih_r, w_hh_r, b_ih_r, b_hh_r, fc_w, narrow_bwd=(tiles if tiles <= 16 else False),
+                           fwd_steps=not fused)
         H, BN, nt = p["H"], p["BN"], p["n_tiles"]
         m_all = steps * tiles
         x = x.contiguous().float()
@@ -193,21 +202,26 @@ class BLSTMBlockTC(torch.autograd.Function):
         y = [torch.zeros(m_all * tile_halves, dtype=torch.float16, device=dev) for _ in range(2)]     # pad k-core stays 0
         c_all = [torch.empty(steps, tiles * 128, H, dtype=torch.float32, device=dev) for _ in range(2)]
         zero = torch.zeros(tiles * tile_halves, dtype=torch.float16, device=dev)
-        assert not fused or (p["kc_h"] == LKC_H and N < p["kc_in"] * 8)
+        assert not fused or N < p["kc_in"] * 8
         if fused:
             # x -> operand tiles with the constant-one column (the bias rides in the weights), then ONE persistent launch:
             # input projection + recurrence, activated gates and c_t saved by the epilogue for BPTT
-            geo = 14 if (tiles + 1) // 2 <= 3 else 7
+            geo = 768 if H == 768 else 14 if (tiles + 1) // 2 <= 3 else 7
             xhat = torch.empty(m_all * p["kc_in"] * 1024, dtype=torch.float16, device=dev)
             L.call("bsrnn_norm_cast_kb8_ones", x.data_ptr(), None, None, xhat.data_ptr(), N, 0, N, p["kc_in"], m_all, tiles, R,
                    *addr, T * K, 1, N, st)
             wf = pack_fused_train((w_ih, w_hh, b_ih, b_hh, w_ih_r, w_hh_r, b_ih_r, b_hh_r), geo, p["kc_in"], N)
             sync = torch.empty(L.lib().bsrnn_blstm_fused_sync_bytes(), dtype=torch.uint8, device=dev)
-            scratch = torch.empty(m_all * 128 * H * 24, dtype=torch.uint8, device=dev)      # bsrnn_blstm_fused_train_scratch_bytes
+            scratch = torch.empty(m_all * 128 * H * 24, dtype=torch.uint8, device=dev)      # bsrnn_blstm_fused*_train_scratch_bytes
             with torch.profiler.record_function("tc_fwd_fused"):
-                L.call("bsrnn_blstm_fused_train_tc", geo, xhat.data_ptr(), wf.data_ptr(), zero.data_ptr(), y[0].data_ptr(),
-                       y[1].data_ptr(), tile_halves, gates.data_ptr(), c_all[0].data_ptr(), c_all[1].data_ptr(),
-                       scratch.data_ptr(), R, steps, tiles, 0, 0, sync.data_ptr(), st)
+                if geo == 768:
+                    L.call("bsrnn_blstm_fused768_train_tc", xhat.data_ptr(), wf.data_ptr(), zero.data_ptr(), y[0].data_ptr(),
+                           y[1].data_ptr(), tile_halves, gates.data_ptr(), c_all[0].data_ptr(), c_all[1].data_ptr(),
+                           scratch.data_ptr(), R, steps, tiles, 0, 0, sync.data_ptr(), st)
+                else:
+                    L.call("bsrnn_blstm_fused_train_tc", geo, xhat.data_ptr(), wf.data_ptr(), zero.data_ptr(), y[0].data_ptr(),
+                           y[1].data_ptr(), tile_halves, gates.data_ptr(), c_all[0].data_ptr(), c_all[1].data_ptr(),
+                           scratch.data_ptr(), R, steps, tiles, 0, 0, sync.data_ptr(), st)
         else:
             xhat = _cast_kb8(x, p["kc_in"], steps, tiles, R, addr, T * K)
             L.call("bsrnn_gemm_tc", xhat.data_ptr(), p["wih"].data_ptr(), p["bias"].data_ptr(), gates.data_ptr(), None, m_all,
