@@ -158,12 +158,12 @@ def _decode_fused_blocks(blocks, H, N, kc_in, kc_h, oc, U, prow_of, what):
 
 
 def decode_fused_pairs(wf, H, N, kc_in, oc):
-    """pack_lstm_fused7 (P/U = 7/56, 14/28), pack_lstm_fused768 (24/32) and training_tc.pack_fused_train:
-    [dir][pair q][half e][kc_in + kc_h k-cores][2U rows][8]; pair q's packed row 4*u_local + gate (half e = rows e*2U ..)
-    <- LSTM row gate*H + U*q + u_local, K = [W_ih | bias at column oc | pad | W_hh | pad]."""
+    """runtime_tc.pack_fused (P/U = 8/49, 7/56, 14/28, 24/32): [dir][pair q][half e][kc_in + kc_h k-cores][rh rows][8],
+    rh = ceil16(4U) / 2; pair q's packed row 4*u_local + gate (half e = rows e*rh ..) <- LSTM row gate*H + U*q + u_local,
+    rows >= 4U padding (208-row pairs at P = 8), K = [W_ih | bias at column oc | pad | W_hh | pad]."""
     _, P, _, kct, rh, _ = wf.shape
     U = H // P
-    assert U * P == H and rh == 2 * U
+    assert U * P == H and rh == (4 * U + 15) // 16 * 8
     kc_h = kct - kc_in
     g = torch.arange(4)
     out = []

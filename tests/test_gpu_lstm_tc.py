@@ -246,7 +246,7 @@ def unpack_step_w(W8, H, K):
 
 
 # ---------------------------------------------------------------------------------------------------- a. step kernels
-# (H, BN, n_tiles, m_tiles): every BN the packers choose (_bn_div / _bn_for: widest divisor; _bn_cover; narrow 32 / 64), one
+# (H, BN, n_tiles, m_tiles): every BN the packers choose (tile_width / _bn_for: widest divisor; _bn_cover; narrow 32 / 64), one
 # n_tiles*BN > 4H, padded k-cores at H = 40 and 392
 STEP_CASES = {
     "h32_bn128_m1": (32, 128, 1, 1),
@@ -579,28 +579,14 @@ GEOS = {   # geo -> (H, N, kc_in, kc_h, P, U)
 
 
 def fused_pack(geo, ws):
-    from urgent2026_challenge_track1_b200 import training_tc as TT
+    from urgent2026_challenge_track1_b200 import runtime_tc as TC
     H, N, kc_in, kc_h, P, U = GEOS[geo]
     flat = []
     for (wi, wh, b) in ws:
         flat += [wi, wh, b, torch.zeros_like(b)]
-    if geo == 8:
-        rnn = torch.nn.LSTM(N, H, bidirectional=True).to(DEV)
-        with torch.no_grad():
-            for (wi, wh, b), sfx in zip(ws, ("", "_reverse")):
-                getattr(rnn, "weight_ih_l0" + sfx).copy_(wi)
-                getattr(rnn, "weight_hh_l0" + sfx).copy_(wh)
-                getattr(rnn, "bias_ih_l0" + sfx).copy_(b)
-                getattr(rnn, "bias_hh_l0" + sfx).zero_()
-        from urgent2026_challenge_track1_b200 import runtime_tc as TC
-        p = TC.pack_lstm_tc(rnn)
-        dec = decode_lstm_tc({k: (v.cpu() if torch.is_tensor(v) else v) for k, v in p.items() if k != "_rnn"})["wfused"]
-        wf = p["wfused"]
-    else:
-        wf = TT.pack_fused_train(flat, 768 if geo == 768 else geo, kc_in, N)
-        dec = decode_fused_pairs(wf.cpu(), H, N, kc_in, N)
+    wf = TC.pack_fused(flat, geo, kc_in, N)
     W = []
-    for wi, wh, b in dec:
+    for wi, wh, b in decode_fused_pairs(wf.cpu(), H, N, kc_in, N):
         W.append((torch.cat([wi, b[:, None]], 1).to(DEV), wh.to(DEV)))     # x operand: columns 0..N-1 and the one column N
     return wf.contiguous(), W
 
@@ -852,7 +838,7 @@ def tc_inputs(g, R, steps, tiles):
             getattr(rnn, "bias_hh_l0" + sfx).zero_()
     p = TC.pack_lstm_tc(rnn)
     whh = p["whh"].to(DEV).contiguous()
-    W = [(None, w.to(DEV)) for w in decode_lstm_tc({k: v for k, v in p.items() if k != "_rnn"})["whh"]]
+    W = [(None, w.to(DEV)) for w in decode_lstm_tc(p)["whh"]]
     # gates_x [step][tile][dir][q][26][128][8] fp16, random (the pad columns 196..207 of each q too)
     gxt = (rand(g, steps * tiles * 2 * 8 * 26 * 1024, scale=1.5)).half()
     return whh, W, gxt

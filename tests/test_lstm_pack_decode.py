@@ -2,8 +2,10 @@
 
 The decoders (tests/lstm_packs.py) invert each packer's index map and remove GATE_SCALE.  The decoded tensors must equal
 fp16(w * scale) / scale of the nn.LSTM tensors bit for bit, and every padding row, column and k-core of the pack must be
-zero.  The existing pack tests compare the training packer with the inference packer; these compare both with nn.LSTM,
-and the GPU tests (test_gpu_lstm_tc.py) build their f64 references from the same decoders."""
+zero.  Training hands the packers nn.Parameters that require grad, inference packs under no_grad: both are decoded.  The
+GPU tests (test_gpu_lstm_tc.py) build their f64 references from the same decoders."""
+import itertools
+
 import pytest
 import torch
 
@@ -13,6 +15,9 @@ from urgent2026_challenge_track1_b200 import runtime_tc_steps as TS
 from urgent2026_challenge_track1_b200 import training_tc as TT
 
 
+GRAD = pytest.mark.parametrize("grad", [True, False], ids=["requires_grad", "no_grad"])
+
+
 def _lstm(N, H, seed):
     torch.manual_seed(seed)
     rnn = torch.nn.LSTM(N, H, batch_first=True, bidirectional=True)
@@ -20,11 +25,6 @@ def _lstm(N, H, seed):
         for p in rnn.parameters():           # magnitudes that exercise fp16 rounding, subnormals and the exponent range
             p.copy_(torch.randn_like(p) * torch.exp2(torch.randint(-16, 3, p.shape).float()))
     return rnn
-
-
-def _ws(rnn):
-    return (rnn.weight_ih_l0, rnn.weight_hh_l0, rnn.bias_ih_l0, rnn.bias_hh_l0, rnn.weight_ih_l0_reverse,
-            rnn.weight_hh_l0_reverse, rnn.bias_ih_l0_reverse, rnn.bias_hh_l0_reverse)
 
 
 def _same(a, b, what):
@@ -48,30 +48,43 @@ def test_pack_and_decode_lstm_tc():
         _same(fb, rounded(b), f"wfused[{d}] bias")
 
 
-@pytest.mark.parametrize("P,U", [(7, 56), (14, 28)])
-def test_pack_and_decode_lstm_fused7(P, U):
-    rnn = _lstm(196, 392, P)
-    wf = TC.pack_lstm_fused7(rnn, 26, 196, P=P, U=U)
-    assert tuple(wf.shape) == (2, P, 2, 76, 2 * U, 8)
-    for d, ((wi, wh, b), (dwi, dwh, db)) in enumerate(zip(lstm_tensors(rnn), decode_fused_pairs(wf, 392, 196, 26, 196))):
-        _same(dwi, rounded(wi), f"fused{P}[{d}] W_ih")
-        _same(dwh, rounded(wh), f"fused{P}[{d}] W_hh")
-        _same(db, rounded(b), f"fused{P}[{d}] bias")
+# geometry -> (N, H, kc_in, pairs, packed rows per pair): the fused layer kernel's four group geometries at their widths
+FUSED = {8: (196, 392, 26, 8, 208), 7: (196, 392, 26, 7, 224), 14: (196, 392, 26, 14, 112), 768: (384, 768, 50, 24, 128)}
+
+
+@GRAD
+@pytest.mark.parametrize("geo", sorted(FUSED))
+def test_pack_and_decode_fused(geo, grad):
+    N, H, kc_in, P, rows = FUSED[geo]
+    rnn = _lstm(N, H, geo)
+    with torch.set_grad_enabled(grad):
+        wf = TC.pack_fused(TC.lstm_ws(rnn), geo, kc_in, N)
+    assert tuple(wf.shape) == (2, P, 2, kc_in + (H + 15) // 16 * 2, rows // 2, 8) and wf.dtype == torch.float16
+    for d, ((wi, wh, b), (dwi, dwh, db)) in enumerate(zip(lstm_tensors(rnn), decode_fused_pairs(wf, H, N, kc_in, N))):
+        _same(dwi, rounded(wi), f"fused{geo}[{d}] W_ih")
+        _same(dwh, rounded(wh), f"fused{geo}[{d}] W_hh")
+        _same(db, rounded(b), f"fused{geo}[{d}] bias")
 
 
 def test_pack_and_decode_lstm_steps_and_fused768():
-    rnn = _lstm(384, 768, 3)
-    p = TS.pack_lstm_steps_tc(rnn)
-    assert tuple(p["wfused"].shape) == (2, 24, 2, 146, 64, 8)
-    steps = decode_lstm_steps(p)
-    fused = decode_fused_pairs(p["wfused"], 768, 384, 50, 384)
-    for d, (wi, wh, b) in enumerate(lstm_tensors(rnn)):
-        _same(steps[d][0], rounded(wi), f"steps wih[{d}]")
-        _same(steps[d][1], rounded(wh), f"steps whh[{d}]")
-        _same(steps[d][2], b.double(), f"steps bias[{d}] (f32, not rounded)")
-        _same(fused[d][0], rounded(wi), f"fused768[{d}] W_ih")
-        _same(fused[d][1], rounded(wh), f"fused768[{d}] W_hh")
-        _same(fused[d][2], rounded(b), f"fused768[{d}] bias")
+    """pack_lstm_steps_tc at the FlowSE width (with the fused layer kernel's weights) and at (N, H) = (64, 32), in both grad
+    modes."""
+    for (N, H), grad in itertools.product([(384, 768), (64, 32)], [True, False]):
+        rnn = _lstm(N, H, 3)
+        with torch.set_grad_enabled(grad):
+            p = TS.pack_lstm_steps_tc(rnn)
+        assert ("wfused" in p) == (H == 768)
+        steps = decode_lstm_steps(p)
+        for d, (wi, wh, b) in enumerate(lstm_tensors(rnn)):
+            _same(steps[d][0], rounded(wi), f"steps{H} wih[{d}]")
+            _same(steps[d][1], rounded(wh), f"steps{H} whh[{d}]")
+            _same(steps[d][2], b.double(), f"steps{H} bias[{d}] (f32, not rounded)")
+        if H == 768:
+            assert tuple(p["wfused"].shape) == (2, 24, 2, 146, 64, 8) and p["kc_fused"] == 50 and p["one_col"] == 384
+            for d, ((wi, wh, b), fused) in enumerate(zip(lstm_tensors(rnn), decode_fused_pairs(p["wfused"], 768, 384, 50, 384))):
+                _same(fused[0], rounded(wi), f"fused768[{d}] W_ih")
+                _same(fused[1], rounded(wh), f"fused768[{d}] W_hh")
+                _same(fused[2], rounded(b), f"fused768[{d}] bias")
 
 
 @pytest.mark.parametrize("N,H", [(196, 392), (384, 768), (36, 40)])
@@ -80,34 +93,26 @@ def test_pack_and_decode_lstm_steps_and_fused768():
 def test_pack_and_decode_pack_block(N, H, fwd_steps, narrow):
     rnn = _lstm(N, H, H + N)
     fc_w = torch.randn(N, 2 * H)
-    p = TT.pack_block(*_ws(rnn), fc_w, narrow_bwd=narrow, fwd_steps=fwd_steps)
-    assert p["nt_h"] * p["bn_h"] >= H and p["nt_n"] * p["bn_n"] >= N
-    dec = decode_pack_block(p)
-    for d, (wi, wh, b) in enumerate(lstm_tensors(rnn)):
-        _same(dec[d]["whhT"], rounded(wh, scale_rows=False), f"whhT[{d}]")
-        _same(dec[d]["wihT"], rounded(wi, scale_rows=False), f"wihT[{d}]")
-        if fwd_steps:
-            _same(dec[d]["whh"], rounded(wh), f"block whh[{d}]")
-            _same(dec[d]["wih"], rounded(wi), f"block wih[{d}]")
-            _same(dec[d]["b"], b.double(), f"block bias[{d}]")
-        else:
-            assert "whh" not in dec[d]
+    for grad in (True, False):
+        with torch.set_grad_enabled(grad):
+            p = TT.pack_block(*TC.lstm_ws(rnn), fc_w, narrow_bwd=narrow, fwd_steps=fwd_steps)
+        assert p["nt_h"] * p["bn_h"] >= H and p["nt_n"] * p["bn_n"] >= N
+        dec = decode_pack_block(p)
+        for d, (wi, wh, b) in enumerate(lstm_tensors(rnn)):
+            _same(dec[d]["whhT"], rounded(wh, scale_rows=False), f"whhT[{d}]")
+            _same(dec[d]["wihT"], rounded(wi, scale_rows=False), f"wihT[{d}]")
+            if fwd_steps:
+                _same(dec[d]["whh"], rounded(wh), f"block whh[{d}]")
+                _same(dec[d]["wih"], rounded(wi), f"block wih[{d}]")
+                _same(dec[d]["b"], b.double(), f"block bias[{d}]")
+            else:
+                assert "whh" not in dec[d]
 
 
-@pytest.mark.parametrize("geo,N,H,kc_in", [(7, 196, 392, 26), (14, 196, 392, 26), (768, 384, 768, 50)])
-def test_pack_and_decode_fused_train(geo, N, H, kc_in):
-    rnn = _lstm(N, H, geo)
-    wf = TT.pack_fused_train(_ws(rnn), geo, kc_in, N)
-    for d, ((wi, wh, b), (dwi, dwh, db)) in enumerate(zip(lstm_tensors(rnn), decode_fused_pairs(wf, H, N, kc_in, N))):
-        _same(dwi, rounded(wi), f"train{geo}[{d}] W_ih")
-        _same(dwh, rounded(wh), f"train{geo}[{d}] W_hh")
-        _same(db, rounded(b), f"train{geo}[{d}] bias")
-
-
-def test_pack_and_decode_rejects_a_corrupted_pack():
+def test_decoders_reject_a_corrupted_pack():
     """the decoders see a moved weight (wrong row), a non-zero padding element and a wrong scale."""
     rnn = _lstm(196, 392, 5)
-    wf = TC.pack_lstm_fused7(rnn, 26, 196, P=7, U=56)
+    wf = TC.pack_fused(TC.lstm_ws(rnn), 7, 26, 196)
     wi = lstm_tensors(rnn)[0][0]
     bad = wf.clone()
     bad[0, 0, 0, :, [0, 1]] = bad[0, 0, 0, :, [1, 0]]                 # i and f rows of unit 0 swapped

@@ -117,15 +117,3 @@ def test_batched_band_ops_equal_the_per_band_loops(fs):
     assert set(a[3]) == set(b[3])                       # bands the spectrum does not reach get no gradient in either
     assert max(rel(b[3][n], a[3][n]) for n in a[3]) < 1e-11
 
-
-@pytest.mark.parametrize("geo,P,U", [(7, 7, 56), (14, 14, 28)])
-def test_fused_training_weight_pack_equals_the_inference_pack(geo, P, U):
-    """training_tc.pack_fused_train (batched, runs inside every training step) builds bit-identical operands to
-    runtime_tc.pack_lstm_fused7 (the inference packer of the fused layer kernel)."""
-    from urgent2026_challenge_track1_b200 import runtime_tc as TC, training_tc as TT
-    torch.manual_seed(1)
-    rnn = torch.nn.LSTM(196, 392, bidirectional=True, batch_first=True)
-    ws = tuple(getattr(rnn, n + sfx) for sfx in ("", "_reverse") for n in ("weight_ih_l0", "weight_hh_l0", "bias_ih_l0", "bias_hh_l0"))
-    a = TC.pack_lstm_fused7(rnn, 26, 196, P=P, U=U)
-    b = TT.pack_fused_train(ws, geo, 26, 196)
-    assert a.shape == b.shape == (2, P, 2, 76, 2 * U, 8) and bool((a == b).all())

@@ -86,91 +86,122 @@ def from_kb8(t, rows, K):
     return t.permute(0, 2, 1, 3).reshape(n_tiles * rpt, kcores * 8)[:rows, :K].float()
 
 
-def _gate_perm(H, dev):
-    """row index into a (4H, .) LSTM matrix for packed position (q, c = 4*u + gate): gate*H + 49*q + u; -1 for pads."""
-    idx = torch.full((CL, LBN), -1, dtype=torch.long, device=dev)
-    for q in range(CL):
-        u = torch.arange(LU, device=dev)
-        for g in range(4):
-            idx[q, 4 * u + g] = g * H + LU * q + u
-    return idx
+def tile_width(cols, mult=16):
+    """widest multiple of `mult` <= 256 that divides cols: the N-tile width of a GEMM over cols output columns."""
+    for bn in range(256, mult - 1, -mult):
+        if cols % bn == 0:
+            return bn
+    raise NotImplementedError(f"no tile width for {cols} columns")
+
+
+# ------------------------------------------------------------------------------------------------ packed BLSTM weights
+# Every tensor-core BLSTM layout is cut from one block of gate rows per (direction, pair q): packed row 4*u + gate of pair q
+# is LSTM row gate*H + U*q + u (gates i, f, g, o), its i, f and o rows pre-halved by GATE_SCALE.  The step-wise kernels see a
+# single pair (P = 1, U = H).
+
+# fused layer kernel geometry -> (pairs per group P, hidden units per pair U): PPG / UPP of the csrc/lstm_fused.cu struct
+FUSED_PAIRS = {8: (8, 49),         # Geo392
+               7: (7, 56),         # Geo392x7
+               14: (14, 28),       # Geo392x14
+               768: (24, 32)}      # Geo768
+_GATE_ROWS = {}
+
+
+def lstm_ws(rnn):
+    """the 8 tensors of a one-layer bidirectional nn.LSTM in the packers' order: w_ih, w_hh, b_ih, b_hh, then the reverse four."""
+    return tuple(getattr(rnn, n + sfx) for sfx in ("", "_reverse") for n in ("weight_ih_l0", "weight_hh_l0", "bias_ih_l0", "bias_hh_l0"))
+
+
+def gate_row_map(H, P, U, dev):
+    """(rows (P, R) int64, scale (R, 1) f32), R = ceil16(4U): rows[q, 4*u + gate] = gate*H + U*q + u, and 4H (a zero row of
+    gate_rows' source) for the padding rows past 4U; scale = GATE_SCALE of each packed row.  Built once per (H, P, U, device):
+    an H2D copy from pageable memory is a stream synchronisation, and the training step packs inside every block."""
+    key = (H, P, U, str(dev))
+    t = _GATE_ROWS.get(key)
+    if t is None:
+        R = (4 * U + 15) // 16 * 16
+        q = torch.arange(P, device=dev)[:, None, None]
+        u = torch.arange(U, device=dev)[None, :, None]
+        g = torch.arange(4, device=dev)[None, None, :]
+        rows = torch.full((P, R), 4 * H, dtype=torch.long, device=dev)
+        rows[:, :4 * U] = (g * H + U * q + u).reshape(P, 4 * U)
+        scale = torch.zeros(R, device=dev)
+        scale[:4 * U] = torch.tensor(GATE_SCALE, device=dev).repeat(U)
+        t = _GATE_ROWS[key] = (rows, scale[:, None])
+    return t
+
+
+@torch.no_grad()
+def gate_rows(ws, P, U, kc_in, one_col=-1):
+    """The gate rows of the 8 LSTM tensors ws (lstm_ws order) for groups of P pairs x U units: (w (2, P, R, (kc_in + kc_h) * 8),
+    b (2, P, R)) f32, R = ceil16(4U), kc_h = ceil16(H) / 8, rows past 4U zero.  Columns of w: [W_ih | pad | W_hh | pad] over
+    kc_in + kc_h k-cores, and b_ih + b_hh in column one_col too when one_col >= 0 (the operand's constant-one column).  b is
+    the f32 bias.  Both carry GATE_SCALE.  A few batched ops without a host synchronisation: it runs in every training step."""
+    w_ih, w_hh, b_ih, b_hh, w_ih_r, w_hh_r, b_ih_r, b_hh_r = ws
+    H, N = w_hh.shape[1], w_ih.shape[1]
+    K = (kc_in + (H + 15) // 16 * 2) * 8
+    rows, scale = gate_row_map(H, P, U, w_hh.device)
+    src = torch.zeros(2, 4 * H + 1, K + 1, device=w_hh.device)         # row 4H stays zero; column K holds the bias
+    lstm = src[:, :4 * H]
+    lstm[..., :N] = torch.stack((w_ih, w_ih_r))
+    lstm[..., kc_in * 8: kc_in * 8 + H] = torch.stack((w_hh, w_hh_r))
+    lstm[..., K] = torch.stack((b_ih + b_hh, b_ih_r + b_hh_r))
+    if one_col >= 0:
+        src[:, :, one_col] = src[:, :, K]
+    w = src[:, rows] * scale                                             # (2, P, R, K + 1)
+    return w[..., :K], w[..., K]
+
+
+def pack_fused(ws, geo, kc_in, one_col):
+    """Weights of the fused layer kernel of geometry `geo` (FUSED_PAIRS): [dir][pair q][half e][kc_in + kc_h k-cores][R/2][8]
+    fp16, half e holding gate rows e*R/2 .. of pair q; the bias rides in operand column one_col."""
+    P, U = FUSED_PAIRS[geo]
+    w = gate_rows(ws, P, U, kc_in, one_col)[0]
+    R, K = w.shape[2:]
+    return w.view(2, P, 2, R // 2, K // 8, 8).permute(0, 1, 2, 4, 3, 5).contiguous().to(torch.float16)
+
+
+def pack_steps(ws, kc_in, BN):
+    """Operands of the step-wise kernels (one pair of U = H units, BN-row tiles): wih [2*4H/BN][kc_in][BN][8] (directions
+    stacked) for the input-projection GEMM, whose epilogue adds `bias` (2*4H) f32; whh per direction [4H/BN][kc_h][BN][8]."""
+    H = ws[1].shape[1]
+    kc_h = (H + 15) // 16 * 2
+    w, b = gate_rows(ws, 1, H, kc_in)
+    w, k0 = w[:, 0], kc_in * 8
+    return dict(wih=to_kb8(w[..., :k0].reshape(8 * H, k0), BN, kc_in), whh=[to_kb8(w[d, :, k0:], BN, kc_h) for d in (0, 1)],
+                bias=b.flatten().contiguous())
 
 
 def pack_lstm_tc(rnn):
-    """nn.LSTM(N, H=392, bidirectional) -> dict(wih [16][26][208][8], bih (16*208) f32, whh [2][8][50][208][8]).
+    """nn.LSTM(N, H=392, bidirectional) -> dict(wih [16][26][208][8], bih (16*208) f32, whh [2][8][50][208][8]): 8 CTAs of
+    49 units, 208 gate rows each.
 
     When the operand has a padding column (N < kc_in*8) the bias b_ih + b_hh is ALSO stored as weight column N
     (`one_col`): norm_cast_kb8_ones writes the constant 1 there and the input-projection GEMM runs without a bias
-    epilogue (its epilogue is then a pure convert-and-store at HBM write speed)."""
-    H, N = rnn.weight_hh_l0.shape[1], rnn.weight_ih_l0.shape[1]
+    epilogue (its epilogue is then a pure convert-and-store at HBM write speed).  The fused layer kernel needs that column:
+    only then are its weights packed (`wfused`, geometry 8; the others on first use, fused_weights)."""
+    ws = lstm_ws(rnn)
+    H, N = ws[1].shape[1], ws[0].shape[1]
     if H != CL * LU:
         raise NotImplementedError(f"tensor-core BLSTM kernel is specialised for H=392, got H={H}")
-    dev = rnn.weight_hh_l0.device
-    perm = _gate_perm(H, dev)
-    gsc = torch.tensor(GATE_SCALE, device=dev).repeat(LU)           # packed column c = 4*u + gate
-    gsc = torch.cat([gsc, torch.zeros(LBN - 4 * LU, device=dev)])
     kc_in = (N + 15) // 16 * 2
     one_col = N if (N % 4 == 0 and N < kc_in * 8) else -1
-    wih_rows, bih_rows, whh = [], [], []
-    for sfx in ("", "_reverse"):
-        wi = getattr(rnn, "weight_ih_l0" + sfx).float()
-        wh = getattr(rnn, "weight_hh_l0" + sfx).float()
-        b = (getattr(rnn, "bias_ih_l0" + sfx) + getattr(rnn, "bias_hh_l0" + sfx)).float()
-        for q in range(CL):
-            sel = perm[q].clamp_min(0)
-            valid = ((perm[q] >= 0).float() * gsc)[:, None]
-            wrow = wi[sel] * valid
-            brow = b[sel] * valid[:, 0]
-            if one_col >= 0:
-                wrow = torch.cat([wrow, torch.zeros(wrow.shape[0], kc_in * 8 - N, device=dev)], 1)
-                wrow[:, one_col] = brow
-            wih_rows.append(wrow)
-            bih_rows.append(brow)
-            whh.append(to_kb8(wh[sel] * valid, LBN, LKC)[0])
-    wih = to_kb8(torch.cat(wih_rows, 0), LBN, kc_in)                # 16 tiles of 208 rows
-    whh = torch.stack(whh).view(2, CL, LKC, LBN, 8).contiguous()
-    out = dict(wih=wih, bih=torch.cat(bih_rows).contiguous(), whh=whh, kc_in=kc_in, H=H, N=N, one_col=one_col)
+    w, b = gate_rows(ws, CL, LU, kc_in, one_col)
+    out = dict(wih=to_kb8(w[..., :kc_in * 8].reshape(-1, kc_in * 8), LBN, kc_in), bih=b.flatten().contiguous(),
+               whh=to_kb8(w[..., kc_in * 8:].reshape(-1, LKC * 8), LBN, LKC).view(2, CL, LKC, LBN, 8),
+               kc_in=kc_in, H=H, N=N, one_col=one_col)
     if one_col >= 0:
-        # bsrnn_blstm_fused_tc: [dir][pair q][half e][kc_in k-cores of W_ih (+ bias column) | 50 of W_hh][104 rows][8]
-        wf = torch.cat([wih.view(2, CL, kc_in, LBN, 8), whh], 2)
-        out["wfused"] = wf.view(2, CL, kc_in + LKC, 2, LBN // 2, 8).permute(0, 1, 3, 2, 4, 5).contiguous()
-        out["_rnn"] = rnn                   # the other group geometries are packed on first use (fused_weights)
+        out.update(wfused=pack_fused(ws, 8, kc_in, one_col), _ws=ws)
     return out
 
 
 def fused_weights(w, geo):
     """Packed weights of the fused layer kernel for group geometry `geo` (8, 7 or 14), built on first use and kept in the
     layer's pack dict (which PackedCache rebuilds whenever a parameter changes)."""
-    if geo == 8:
-        return w["wfused"]
-    key = f"wfused{geo}"
+    key = "wfused" if geo == 8 else f"wfused{geo}"
     if key not in w:
-        P, U = (7, 56) if geo == 7 else (14, 28)
-        w[key] = pack_lstm_fused7(w["_rnn"], w["kc_in"], w["one_col"], P=P, U=U)
+        w[key] = pack_fused(w["_ws"], geo, w["kc_in"], w["one_col"])
     return w[key]
-
-
-def pack_lstm_fused7(rnn, kc_in, one_col, P=7, U=56):
-    """bsrnn_blstm_fused7_tc / _fused14_tc: groups of P pairs x U units -> [dir][pair q][half e][kc_in + 50 k-cores][2U rows][8];
-    packed gate row c = 4*u_local + gate of pair q is LSTM row gate*H + U*q + u_local (i, f, o rows pre-halved)."""
-    H, N = rnn.weight_hh_l0.shape[1], rnn.weight_ih_l0.shape[1]
-    dev = rnn.weight_hh_l0.device
-    ul = torch.arange(U, device=dev)
-    gsc = torch.tensor(GATE_SCALE, device=dev).repeat(U)[:, None]
-    packs = []
-    for sfx in ("", "_reverse"):
-        wi = getattr(rnn, "weight_ih_l0" + sfx).float()
-        wh = getattr(rnn, "weight_hh_l0" + sfx).float()
-        b = (getattr(rnn, "bias_ih_l0" + sfx) + getattr(rnn, "bias_hh_l0" + sfx)).float()
-        for q in range(P):
-            rows = (torch.arange(4, device=dev)[None, :] * H + (U * q + ul)[:, None]).reshape(-1)        # 224 rows
-            w = torch.zeros(rows.numel(), (kc_in + LKC) * 8, device=dev)
-            w[:, :N] = wi[rows]
-            w[:, one_col] = b[rows]
-            w[:, kc_in * 8: kc_in * 8 + H] = wh[rows]
-            w = w * gsc
-            packs.append(w.view(2, rows.numel() // 2, kc_in + LKC, 8).permute(0, 2, 1, 3))              # [e][k-core][112][8]
-    return torch.stack(packs).view(2, P, 2, kc_in + LKC, 2 * U, 8).contiguous().to(torch.float16)
 
 
 def pack_fc_tc(fc, H):

@@ -17,7 +17,7 @@ from __future__ import annotations
 import torch
 
 from . import _lib as L
-from .runtime_tc import GATE_SCALE, to_kb8, FC_EPI
+from .runtime_tc import to_kb8, FC_EPI, lstm_ws, pack_fused, pack_steps, tile_width
 
 
 def _bn_for(cols, kcores=None):
@@ -29,41 +29,35 @@ def _bn_for(cols, kcores=None):
     forced = int(os.environ.get("BSRNN_STEP_BN", "0"))
     if forced:
         return forced
-    widths = (256, 224, 192, 160, 128, 96, 64, 32)
     if kcores is not None and os.environ.get("BSRNN_STEP_RESIDENT", "0") == "1":      # A/B switch, off: see launch_tc
-        for bn in widths:
-            if cols % bn == 0 and bn >= 64 and kcores * bn * 16 + 65536 + 1024 <= 225 * 1024:
+        for bn in range(256, 63, -32):
+            if cols % bn == 0 and kcores * bn * 16 + 65536 + 1024 <= 225 * 1024:
                 return bn
-    for bn in widths:
-        if cols % bn == 0:
-            return bn
-    return 256
+    return tile_width(cols, 32)
 
 
 def pack_lstm_steps_tc(rnn):
-    H, N = rnn.weight_hh_l0.shape[1], rnn.weight_ih_l0.shape[1]
+    """nn.LSTM(N, H, bidirectional), H % 16 == 0 -> the step-wise operands (runtime_tc.pack_steps) in BN-row tiles; at the
+    FlowSE width (N = 384, H = 768) also the fused layer kernel's weights (pack_lstm_fused768)."""
+    ws = lstm_ws(rnn)
+    H, N = ws[1].shape[1], ws[0].shape[1]
     if H % 16:
         raise NotImplementedError(f"step-wise tensor-core LSTM needs H % 16 == 0, got {H}")
-    dev = rnn.weight_hh_l0.device
-    u = torch.arange(H, device=dev)
-    perm = (torch.arange(4, device=dev)[None, :] * H + u[:, None]).reshape(-1)          # packed row 4u+g <- g*H + u
-    gsc = torch.tensor(GATE_SCALE, device=dev).repeat(H)[:, None]
     kc_in = (N + 15) // 16 * 2
     BN = _bn_for(4 * H, H // 8)
-    wih, bias, whh = [], [], []
-    for sfx in ("", "_reverse"):
-        wi = getattr(rnn, "weight_ih_l0" + sfx).float()[perm] * gsc
-        wh = getattr(rnn, "weight_hh_l0" + sfx).float()[perm] * gsc
-        b = (getattr(rnn, "bias_ih_l0" + sfx) + getattr(rnn, "bias_hh_l0" + sfx)).float()[perm] * gsc[:, 0]
-        wih.append(wi); bias.append(b); whh.append(to_kb8(wh, BN, H // 8))
-    out = dict(wih=to_kb8(torch.cat(wih, 0), BN, kc_in), bias=torch.cat(bias).contiguous(), whh=whh, BN=BN, H=H, N=N,
-               kc_in=kc_in, n_tiles=4 * H // BN)
+    out = dict(pack_steps(ws, kc_in, BN), BN=BN, H=H, N=N, kc_in=kc_in, n_tiles=4 * H // BN)
     if H == 768 and N == 384:
         out.update(pack_lstm_fused768(rnn))
     return out
 
 
-FUSED768 = dict(PPG=24, UPP=32, XKC=50, HKC=96)          # csrc/lstm_fused.cu Geo768
+def pack_lstm_fused768(rnn):
+    """nn.LSTM(384, 768, bidirectional) -> dict(wfused, kc_fused, one_col) for bsrnn_blstm_fused768_tc: runtime_tc.pack_fused
+    at geometry 768, the bias in operand column 384 (norm_cast_kb8_ones writes the constant 1 there) of kc_fused = 50 k-cores."""
+    N = rnn.weight_ih_l0.shape[1]
+    return dict(wfused=pack_fused(lstm_ws(rnn), 768, 50, N), kc_fused=50, one_col=N)
+
+
 # BSRNN_FLOWSE_FUSED=0 returns to the input-projection GEMM + one bsrnn_blstm_step_tc launch per time step
 import os as _os
 FLOWSE_FUSED = _os.environ.get("BSRNN_FLOWSE_FUSED", "1") == "1"
@@ -72,33 +66,6 @@ for _kv in _os.environ.get("BSRNN_FLOWSE_FUSED_SLOTS", "").split(","):
     if "=" in _kv:
         _ax, _sv = _kv.split("=")
         _FUSED_SLOTS[_ax] = int(_sv)
-
-
-def pack_lstm_fused768(rnn):
-    """nn.LSTM(384, 768, bidirectional) -> wfused [2][24 pairs][2 halves][50 + 96 k-cores][64 gate rows][8] fp16 for
-    bsrnn_blstm_fused768_tc: pair q owns hidden units [32q, 32q+32), packed gate row c = 4*u_local + gate (i, f, g, o; the
-    i/f/o rows pre-halved); operand column 384 carries b_ih + b_hh (norm_cast_kb8_ones writes the constant 1 there)."""
-    g = FUSED768
-    H, N = rnn.weight_hh_l0.shape[1], rnn.weight_ih_l0.shape[1]
-    dev = rnn.weight_hh_l0.device
-    ul = torch.arange(g["UPP"], device=dev)
-    gsc = torch.tensor(GATE_SCALE, device=dev).repeat(g["UPP"])[:, None]            # packed row c = 4*u + gate
-    packs = []
-    for sfx in ("", "_reverse"):
-        wi = getattr(rnn, "weight_ih_l0" + sfx).float()
-        wh = getattr(rnn, "weight_hh_l0" + sfx).float()
-        b = (getattr(rnn, "bias_ih_l0" + sfx) + getattr(rnn, "bias_hh_l0" + sfx)).float()
-        for q in range(g["PPG"]):
-            rows = (torch.arange(4, device=dev)[None, :] * H + (g["UPP"] * q + ul)[:, None]).reshape(-1)     # 128 rows
-            w = torch.zeros(rows.numel(), (g["XKC"] + g["HKC"]) * 8, device=dev)
-            w[:, :N] = wi[rows]
-            w[:, N] = b[rows]
-            w[:, g["XKC"] * 8: g["XKC"] * 8 + H] = wh[rows]
-            w = w * gsc
-            # [rows 128][K] -> [half e][k-core][64 rows][8]
-            packs.append(w.view(2, rows.numel() // 2, g["XKC"] + g["HKC"], 8).permute(0, 2, 1, 3))
-    wf = torch.stack(packs).view(2, g["PPG"], 2, g["XKC"] + g["HKC"], 64, 8).contiguous().to(torch.float16)
-    return dict(wfused=wf, kc_fused=g["XKC"], one_col=N)
 
 
 class StepsWorkspace:
@@ -147,8 +114,7 @@ def pack_dual_path_steps(mod):
             norm, rnn, fc = getattr(mod, f"norm_{axis}")[i], getattr(mod, f"rnn_{axis}")[i], getattr(mod, f"fc_{axis}")[i]
             p = pack_lstm_steps_tc(rnn)
             H, N = p["H"], fc.weight.shape[0]
-            bn = next(b for b in (256, 240, 224, 208, 192, 176, 160, 144, 128, 112, 96, 80, 64, 48, 32, 16)
-                      if ((N + 15) // 16 * 16) % b == 0)
+            bn = tile_width((N + 15) // 16 * 16)
             nt = ((N + 15) // 16 * 16) // bn
             w = fc.weight.float()
             bias = torch.zeros(nt * bn, device=w.device)
@@ -167,7 +133,7 @@ def pack_linear_tc(fc):
     """nn.Linear(K -> N) -> KB8 weight tiles + padded bias for bsrnn_gemm_tc (N tiles of bn columns, bn | ceil16(N))."""
     N, K = fc.weight.shape
     n16 = (N + 15) // 16 * 16
-    bn = next(b for b in (256, 240, 224, 208, 192, 176, 160, 144, 128, 112, 96, 80, 64, 48, 32, 16) if n16 % b == 0)
+    bn = tile_width(n16)
     bias = torch.zeros(n16, device=fc.weight.device)
     bias[:N] = fc.bias.float()
     return dict(w=to_kb8(fc.weight.float(), bn, (K + 7) // 8), b=bias, bn=bn, nt=n16 // bn)
@@ -294,7 +260,7 @@ def pack_grad_decoder_tc(gd):
         w, b, bn, nt = [], [], [], []
         for k, wk in enumerate(p["w1"]):                    # (16 s, N), rows already in c' order
             n16 = (wk.shape[0] + 15) // 16 * 16
-            bk = next(x for x in (256, 240, 224, 208, 192, 176, 160, 144, 128, 112, 96, 80, 64, 48, 32, 16) if n16 % x == 0)
+            bk = tile_width(n16)
             w.append(to_kb8(wk, bk, kc))
             bb = torch.zeros(n16, device=wk.device); bb[: wk.shape[0]] = p["b1"][k]
             b.append(bb); bn.append(bk); nt.append(n16 // bk)

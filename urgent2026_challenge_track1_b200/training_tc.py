@@ -24,17 +24,10 @@ import os
 import torch
 
 from . import _lib as L
-from .runtime_tc import GATE_SCALE, to_kb8, FC_EPI
+from .runtime_tc import to_kb8, FC_EPI, gate_row_map, lstm_ws, pack_steps, tile_width
+from .runtime_tc import pack_fused as pack_fused_train      # the fused forward's weights: the inference layout, repacked per step
 
 BIG = 1 << 40
-
-
-def _bn_div(cols, mult=16):
-    """largest tile width <= 256, multiple of `mult`, dividing cols (cols % mult == 0)."""
-    for bn in range(256, mult - 1, -mult):
-        if cols % bn == 0:
-            return bn
-    raise NotImplementedError(f"no tile width for {cols} columns")
 
 
 def _bn_cover(rows, mult=16):
@@ -44,23 +37,10 @@ def _bn_cover(rows, mult=16):
     return bn, nt
 
 
-_CONST = {}
 NARROW_BN = int(os.environ.get("BSRNN_BWD_BN", "0"))      # 0 = automatic (see pack_block)
 
 
-def _gate_tables(H, dev):
-    """(perm, gate scale column) for hidden size H on `dev`, built once: an H2D copy from pageable memory is a stream
-    synchronisation, and this runs in every block of every training step."""
-    key = (H, str(dev))
-    t = _CONST.get(key)
-    if t is None:
-        u = torch.arange(H, device=dev)
-        perm = (torch.arange(4, device=dev)[None, :] * H + u[:, None]).reshape(-1)      # packed row 4u+g <- g*H + u
-        gsc = torch.tensor(GATE_SCALE, device=dev).repeat(H)[:, None]
-        t = _CONST[key] = (perm, gsc)
-    return t
-
-
+@torch.no_grad()
 def pack_block(w_ih, w_hh, b_ih, b_hh, w_ih_r, w_hh_r, b_ih_r, b_hh_r, fc_w, narrow_bwd=False, fwd_steps=True):
     """All tensor-core operands of one block, from the f32 master weights (nn.LSTM / nn.Linear layouts).
     narrow_bwd: BPTT output tiles of 64 hidden units instead of up to 256 (few row tiles = small batch: more CTAs share a
@@ -72,11 +52,9 @@ def pack_block(w_ih, w_hh, b_ih, b_hh, w_ih_r, w_hh_r, b_ih_r, b_hh_r, fc_w, nar
     if H % 8:
         raise NotImplementedError(f"tensor-core training BLSTM needs H % 8 == 0, got {H}")
     kc_h = (H + 15) // 16 * 2                        # k-cores of an h tile: K padded to a multiple of 16, pad core = 0
-    dev = w_hh.device
-    perm, gsc = _gate_tables(H, dev)
     n_in = N if fwd_steps else N + 1                 # + the constant-one column of the fused forward's operand
     kc_in = (n_in + 15) // 16 * 2
-    BN = _bn_div(4 * H, 32)
+    BN = tile_width(4 * H, 32)
     bn_h, nt_h = _bn_cover(H, 32)                    # BPTT output tiles over the H hidden units (32-column chunks)
     if narrow_bwd and H > 64:
         # one BPTT step is a single wave of tiles x ceil(H / bn) x 2 CTAs that each stream the whole 4H-wide dG tile: the narrowest
@@ -85,24 +63,18 @@ def pack_block(w_ih, w_hh, b_ih, b_hh, w_ih_r, w_hh_r, b_ih_r, b_hh_r, fc_w, nar
                                                  and 2 * narrow_bwd * ((H + 31) // 32) <= 148 else 64)
         nt_h = (H + bn_h - 1) // bn_h
     bn_n, nt_n = _bn_cover(n_in, 16)
-    p = dict(H=H, N=N, kc_in=kc_in, kc_h=kc_h, BN=BN, n_tiles=4 * H // BN, bn_h=bn_h, nt_h=nt_h, bn_n=bn_n, nt_n=nt_n, perm=perm)
-    wih, bias, whh, whhT, wihT = [], [], [], [], []
-    for wi, wh, bi, bh in ((w_ih, w_hh, b_ih, b_hh), (w_ih_r, w_hh_r, b_ih_r, b_hh_r)):
-        wi_p, wh_p = wi.detach().float()[perm], wh.detach().float()[perm]               # interleaved rows, TRUE weights
-        if fwd_steps:                                  # operands of the step-wise forward (the fused forward packs its own)
-            wih.append(wi_p * gsc)
-            bias.append((bi.detach() + bh.detach()).float()[perm] * gsc[:, 0])
-            whh.append(to_kb8(wh_p * gsc, BN, kc_h))
-        whhT.append(to_kb8(wh_p.t().contiguous(), bn_h, 4 * H // 8))                    # rows = unit u, K = gate column
-        wihT.append(to_kb8(wi_p.t().contiguous(), bn_n, 4 * H // 8))                    # rows = input n, K = gate column
-    p.update(whhT=whhT, wihT=wihT)
-    if fwd_steps:
-        p.update(wih=to_kb8(torch.cat(wih, 0), BN, kc_in), bias=torch.cat(bias).contiguous(), whh=whh)
-    fw = fc_w.detach().float()                                                           # (N, 2H)
+    p = dict(H=H, N=N, kc_in=kc_in, kc_h=kc_h, BN=BN, n_tiles=4 * H // BN, bn_h=bn_h, nt_h=nt_h, bn_n=bn_n, nt_n=nt_n)
+    if fwd_steps:                                      # operands of the step-wise forward (the fused forward packs its own)
+        p.update(pack_steps((w_ih, w_hh, b_ih, b_hh, w_ih_r, w_hh_r, b_ih_r, b_hh_r), kc_in, BN))
+    # BPTT: TRUE weights, rows of the step-wise layout transposed (rows = unit u / input n, K = packed gate column)
+    perm = gate_row_map(H, 1, H, w_hh.device)[0][0]
+    p.update(whhT=[to_kb8(wh.float()[perm].t(), bn_h, 4 * H // 8) for wh in (w_hh, w_hh_r)],
+             wihT=[to_kb8(wi.float()[perm].t(), bn_n, 4 * H // 8) for wi in (w_ih, w_ih_r)])
+    fw = fc_w.float()                                                                    # (N, 2H)
     n16 = (N + 15) // 16 * 16
-    fc_bn = _bn_div(n16, 16)
+    fc_bn = tile_width(n16, 16)
     p.update(fc_bn=fc_bn, fc_nt=n16 // fc_bn, fcw=[to_kb8(fw[:, :H], fc_bn, kc_h), to_kb8(fw[:, H:], fc_bn, kc_h)])
-    bn_y = _bn_div(2 * H, 16)
+    bn_y = tile_width(2 * H, 16)
     p.update(bn_y=bn_y, nt_y=2 * H // bn_y, fcT=to_kb8(fw.t().contiguous(), bn_y, kc_in))   # rows = y column, K = n
     return p
 
@@ -111,39 +83,6 @@ def pack_block(w_ih, w_hh, b_ih, b_hh, w_ih_r, w_hh_r, b_ih_r, b_hh_r, fc_w, nar
 # bsrnn_blstm_fused768_train_tc at H = 768 / N = 384): one persistent launch per block instead of one input-projection GEMM
 # + one launch per time step.  BSRNN_TRAIN_FUSED=0: the step-wise forward.
 FUSED_TRAIN = os.environ.get("BSRNN_TRAIN_FUSED", "1") == "1"
-_FUSED_IDX = {}
-
-
-FUSED_GEO = {7: (7, 56), 14: (14, 28), 768: (24, 32)}      # geometry -> (pairs per group, hidden units per pair)
-
-
-def pack_fused_train(ws, geo, kc_in, one_col):
-    """pack_lstm_fused7's / pack_lstm_fused768's layout ([dir][pair q][half e][kc_in + kc_h k-cores][2U rows][8] fp16,
-    kc_h = 50 at H = 392, 96 at H = 768) from the 8 raw LSTM tensors (w_ih, w_hh, b_ih, b_hh, and the reverse four) in a
-    handful of batched ops, without a host synchronisation: it runs inside every (captured) training step."""
-    w_ih, w_hh, b_ih, b_hh, w_ih_r, w_hh_r, b_ih_r, b_hh_r = ws
-    H, N = w_hh.shape[1], w_ih.shape[1]
-    P, U = FUSED_GEO[geo]
-    kc_h = (H + 15) // 16 * 2
-    dev = w_hh.device
-    key = (H, P, U, str(dev))
-    t = _FUSED_IDX.get(key)
-    if t is None:
-        q = torch.arange(P, device=dev)[:, None, None]
-        u = torch.arange(U, device=dev)[None, :, None]
-        g = torch.arange(4, device=dev)[None, None, :]
-        rows = (g * H + U * q + u).reshape(P, 4 * U)                      # packed row 4*u_local + gate of pair q
-        gsc = torch.tensor(GATE_SCALE, device=dev).repeat(U)[None, None, :, None]
-        t = _FUSED_IDX[key] = (rows, gsc)
-    rows, gsc = t
-    ktot = (kc_in + kc_h) * 8
-    full = torch.zeros(2, 4 * H, ktot, dtype=torch.float32, device=dev)
-    for d, (wi, wh, bi, bh) in enumerate(((w_ih, w_hh, b_ih, b_hh), (w_ih_r, w_hh_r, b_ih_r, b_hh_r))):
-        full[d, :, :N] = wi.detach().float()
-        full[d, :, one_col] = (bi.detach() + bh.detach()).float()
-        full[d, :, kc_in * 8: kc_in * 8 + H] = wh.detach().float()
-    w = full[:, rows] * gsc                                               # (2, P, 4U, ktot)
-    return w.view(2, P, 2, 2 * U, kc_in + kc_h, 8).permute(0, 1, 2, 4, 3, 5).contiguous().to(torch.float16)
 
 
 def _geom(B, T, K, axis):
@@ -320,6 +259,4 @@ class BLSTMBlockTC(torch.autograd.Function):
 
 
 def blstm_block_tc(x, rnn, fc, axis):
-    return BLSTMBlockTC.apply(x, rnn.weight_ih_l0, rnn.weight_hh_l0, rnn.bias_ih_l0, rnn.bias_hh_l0,
-                              rnn.weight_ih_l0_reverse, rnn.weight_hh_l0_reverse, rnn.bias_ih_l0_reverse,
-                              rnn.bias_hh_l0_reverse, fc.weight, fc.bias, axis)
+    return BLSTMBlockTC.apply(x, *lstm_ws(rnn), fc.weight, fc.bias, axis)
