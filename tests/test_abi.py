@@ -105,3 +105,39 @@ def test_missing_library_raises(monkeypatch, tmp_path):
     monkeypatch.setattr(_lib, "LIB_PATH", str(tmp_path / "nope.so"))
     with pytest.raises(_lib.NativeLibraryError):
         _lib.lib()
+
+
+# Spectral calls the kernels cannot serve: each must fail its argument checks, with its message, before any launch.
+_P = 1 << 20                                             # never dereferenced
+_SPECTRAL_REJECTS = {
+    "stft_L_at_half_n_fft": ("bsrnn_stft_fwd", (_P, None, _P, _P, 1, 80, 160, 80, 0, 1.0, 1.0, None), "stft_fwd: bad dims"),
+    "stft_stats_L_at_half_n_fft": ("bsrnn_stft_stats_fwd", (_P, None, _P, _P, 1, 80, 160, 80, 0, 1.0, 1.0, _P, _P, 4, None),
+                                   "stft_stats_fwd: bad dims"),
+    "stft_prime_97": ("bsrnn_stft_fwd", (_P, None, _P, _P, 1, 1000, 97, 48, 0, 1.0, 1.0, None), "cannot factorise n_fft=97"),
+    "stft_stats_prime_101": ("bsrnn_stft_stats_fwd", (_P, None, _P, _P, 1, 1000, 101, 50, 0, 1.0, 1.0, _P, _P, 4, None),
+                             "cannot factorise n_fft=101"),
+    "istft_prime_194": ("bsrnn_istft_fwd", (_P, None, None, None, _P, _P, 1, 10, 1000, 194, 97, 0, 1.0, 1.0, None),
+                        "cannot factorise n_fft=194"),
+    "istft_prime_101": ("bsrnn_istft_fwd", (_P, None, None, None, _P, _P, 1, 10, 1000, 101, 50, 0, 1.0, 1.0, None),
+                        "cannot factorise n_fft=101"),
+    "istft_bwd_prime_97": ("bsrnn_istft_bwd", (_P, _P, _P, 1, 10, 1000, 97, 48, None), "cannot factorise n_fft=97"),
+    "istft_bwd_prime_194": ("bsrnn_istft_bwd", (_P, _P, _P, 1, 10, 1000, 194, 97, None), "cannot factorise n_fft=194"),
+    "istft_mask_without_resid": ("bsrnn_istft_fwd", (_P, _P, None, None, _P, _P, 1, 10, 1000, 160, 80, 0, 1.0, 1.0, None),
+                                 "mask and resid must come together"),
+    "mrl1_odd_window": ("bsrnn_mrl1_spec_fwd_bwd", (_P, _P, _P, _P, _P, 1, 1000, 255, 0.5, None),
+                        "mrl1_spec_fwd_bwd: bad dims"),
+    "mrl1_L_at_half_window": ("bsrnn_mrl1_spec_fwd_bwd", (_P, _P, _P, _P, _P, 1, 128, 256, 0.5, None),
+                              "mrl1_spec_fwd_bwd: bad dims"),
+    "mrl1_prime_194": ("bsrnn_mrl1_spec_fwd_bwd", (_P, _P, _P, _P, _P, 1, 1000, 194, 0.5, None), "cannot factorise window=194"),
+}
+
+
+@pytest.mark.skipif(torch.cuda.is_available(), reason="on a GPU an accepted call would launch")
+@pytest.mark.parametrize("case", sorted(_SPECTRAL_REJECTS))
+def test_spectral_calls_reject_what_the_kernels_cannot_serve(lib_path, case):
+    from urgent2026_challenge_track1_b200 import _lib
+    name, args, msg = _SPECTRAL_REJECTS[case]
+    h = _lib.lib()
+    rc = getattr(h, name)(*args)
+    err = h.bsrnn_last_error().decode()
+    assert rc != 0 and msg in err, (rc, err)
