@@ -141,3 +141,48 @@ def test_spectral_calls_reject_what_the_kernels_cannot_serve(lib_path, case):
     rc = getattr(h, name)(*args)
     err = h.bsrnn_last_error().decode()
     assert rc != 0 and msg in err, (rc, err)
+
+
+# CUDA-core calls the kernels cannot serve: each must fail its argument checks, with its message, before any launch.
+# bsrnn_band_split_fwd reads its host channel offsets: bands of 8 channels and, last, one of 224 at N = 256 (over 227 KB), so
+# the check must run before the first band's launch.
+_C_OFF = (ctypes.c_int32 * 4)(0, 8, 16, 240)
+_BS = lambda N, ldo, out_width, out_col: (_P, _P, _P, _P, _P, _P, _P, _P, _P, ctypes.addressof(_C_OFF), 3, 1000, 10, 600, N,
+                                          224, ldo, out_width, out_col, None)
+_CORE_REJECTS = {
+    "band_split_N_not_4": ("bsrnn_band_split_fwd", _BS(198, 600, 200, 0), "multiples of 4"),
+    "band_split_out_col_not_4": ("bsrnn_band_split_fwd", _BS(196, 600, 200, 2), "multiples of 4"),
+    "band_split_out_width_not_4": ("bsrnn_band_split_fwd", _BS(196, 600, 198, 0), "multiples of 4"),
+    "band_split_ldo_not_4": ("bsrnn_band_split_fwd", _BS(196, 602, 200, 0), "multiples of 4"),
+    "band_split_wide_band_last": ("bsrnn_band_split_fwd", _BS(256, 768, 256, 0), "band of 224 channels does not fit"),
+    "band_cast_cmax_too_large": ("bsrnn_band_norm_cast_kb8", (_P, _P, _P, _P, _P, _P, _P, _P, 3, 1000, 10, 600, 900, None),
+                                 "band of 900 channels does not fit"),
+    "gn_stats_rows_0": ("bsrnn_gn_stats", (_P, _P, 2, 0, 196, 196, None), "gn_stats: bad arguments"),
+    "gn_stats_C_0": ("bsrnn_gn_stats", (_P, _P, 2, 10, 0, 196, None), "gn_stats: bad arguments"),
+    "gn_stats_B_neg": ("bsrnn_gn_stats", (_P, _P, -1, 10, 196, 196, None), "gn_stats: bad arguments"),
+    "band_stats_T_0": ("bsrnn_band_stats", (_P, _P, 2, 0, 392, _P, _P, 2, None), "band_stats: bad arguments"),
+    "gn_finalize_G_0": ("bsrnn_gn_finalize", (_P, _P, _P, None, _P, _P, 0, 196, _P, 1e-5, 1, None), "gn_finalize: bad arguments"),
+    "gn_finalize_C_0": ("bsrnn_gn_finalize", (_P, _P, _P, None, _P, _P, 4, 0, _P, 1e-5, 1, None), "gn_finalize: bad arguments"),
+    "gn_finalize_G_inner_0": ("bsrnn_gn_finalize", (_P, _P, _P, None, _P, _P, 4, 196, _P, 1e-5, 0, None),
+                              "gn_finalize: bad arguments"),
+    "conv5x5_T_0": ("bsrnn_conv5x5_glu", (_P, _P, _P, _P, 1, 0, 32, 32, None), "conv5x5_glu: bad arguments"),
+    "conv5x5_Fp_0": ("bsrnn_conv5x5_glu", (_P, _P, _P, _P, 1, 4, 0, 32, None), "conv5x5_glu: bad arguments"),
+    "conv5x5_F_neg": ("bsrnn_conv5x5_glu", (_P, _P, _P, _P, 1, 4, 32, -1, None), "conv5x5_glu: bad arguments"),
+    "blstm_recurrence_seq_inner_0": ("bsrnn_blstm_recurrence_f32", (_P, _P, _P, _P, 4, 3, 8, 0, 3, 1, 1, None),
+                                     "blstm_recurrence_f32: bad dims"),
+    "blstm_train_fwd_seq_inner_neg": ("bsrnn_blstm_train_fwd_f32", (_P, _P, _P, _P, _P, 4, 3, 8, -1, 3, 1, 1, None),
+                                      "blstm_train_fwd_f32: bad dims"),
+    "blstm_train_bwd_seq_inner_0": ("bsrnn_blstm_train_bwd_f32", (_P, _P, _P, _P, _P, _P, 4, 3, 8, 0, 3, 1, 1, None),
+                                    "blstm_train_bwd_f32: bad dims"),
+}
+
+
+@pytest.mark.skipif(torch.cuda.is_available(), reason="on a GPU an accepted call would launch")
+@pytest.mark.parametrize("case", sorted(_CORE_REJECTS))
+def test_cuda_core_calls_reject_what_the_kernels_cannot_serve(lib_path, case):
+    from urgent2026_challenge_track1_b200 import _lib
+    name, args, msg = _CORE_REJECTS[case]
+    h = _lib.lib()
+    rc = getattr(h, name)(*args)
+    err = h.bsrnn_last_error().decode()
+    assert rc == 1 and msg in err, (rc, err)

@@ -157,6 +157,9 @@ extern "C" int bsrnn_band_split_fwd(const float* spec, const float* scale, const
                   "band_split_fwd: bad dims (N, out_col, out_width and ldo must be multiples of 4)");
   BandSplitArgs a{spec, scale, shift, wT, bias, out, c_off, bin0, width2, rows, T, F2, N, K, cmax, 0, ldo, out_width, out_col};
   auto smem_of = [&](int C) { const int Cp = (C + 3) & ~3; return (size_t)Cp * N * 4 + (size_t)kBsRows * Cp * 4; };
+  for (int j = 0; j < K; ++j)                         // every band fits before the first run launches
+    BSRNN_CHECK_ARG(smem_of(c_off_host[j + 1] - c_off_host[j]) <= 227 * 1024,
+                    "band_split_fwd: band of %d channels does not fit in shared memory", c_off_host[j + 1] - c_off_host[j]);
   // consecutive runs of bands whose shared-memory need is within 2x of the run's maximum share one launch
   int k = 0;
   while (k < K) {
@@ -168,7 +171,6 @@ extern "C" int bsrnn_band_split_fwd(const float* spec, const float* scale, const
       if (s > need) need = s;
       ++e;
     }
-    BSRNN_CHECK_ARG(need <= 227 * 1024, "band_split_fwd: band of %d channels does not fit in shared memory", c_off_host[k + 1] - c_off_host[k]);
     BSRNN_CUDA_OK(cudaFuncSetAttribute(band_split_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)need));
     a.k_lo = k;
     dim3 grid(e - k, (unsigned)((rows + kBsRows - 1) / kBsRows));

@@ -135,33 +135,36 @@ namespace bsrnn {
 //   dh      = dy[p, d] + dh_rec[d]            (dh_rec = dG_{next} W_hh from the step processed just before)
 //   dc      = dh * o * (1 - tanh(c)^2) + dc_carry[d]     ; dc_carry <- dc * f
 //   dG      = (dc*g*i(1-i), dc*c_prev*f(1-f), dc*i*(1-g^2), dh*tanh(c)*o(1-o))   -> dgates[p, d] (grad of gates_x)
-// grid (ceil(H/256), R, 2), block 256
+// grid (ceil(H/256), min(R, 65535), 2), block 256: sequences r = blockIdx.y + j * gridDim.y (R = B*T on the band axis
+// can exceed the 65535 limit of grid.y)
 __global__ void __launch_bounds__(256)
 lstm_bwd_gates_kernel(const float* __restrict__ dy, const float* __restrict__ saved, const float* __restrict__ dh_rec,
                       float* __restrict__ dc_carry, float* __restrict__ dgates, int R, int H, int q, int steps,
                       SeqAddr addr) {
   const int u = blockIdx.x * 256 + threadIdx.x;
-  const int r = blockIdx.y, d = blockIdx.z;
+  const int d = blockIdx.z;
   if (u >= H) return;
   const int p = d == 0 ? steps - 1 - q : q;
   const int p_prev = d == 0 ? p - 1 : p + 1;                 // forward-order predecessor
-  const long tok = addr.token(r, p);
-  const float* sv = saved + (tok * 2 + d) * (5L * H) + u;
-  const float ig = sv[0], fg = sv[H], gg = sv[2L * H], og = sv[3L * H], c = sv[4L * H];
-  float c_prev = 0.f;
-  if (p_prev >= 0 && p_prev < steps) c_prev = saved[(addr.token(r, p_prev) * 2 + d) * (5L * H) + 4L * H + u];
-  const long si = ((long)d * R + r) * H + u;
-  float dh = dy[tok * (2L * H) + (long)d * H + u];
-  float dc = 0.f;
-  if (q > 0) { dh += dh_rec[si]; dc = dc_carry[si]; }
-  const float tc = tanhf(c);
-  dc += dh * og * (1.f - tc * tc);
-  dc_carry[si] = dc * fg;
-  float* dg = dgates + (tok * 2 + d) * (4L * H) + u;
-  dg[0] = dc * gg * ig * (1.f - ig);
-  dg[H] = dc * c_prev * fg * (1.f - fg);
-  dg[2L * H] = dc * ig * (1.f - gg * gg);
-  dg[3L * H] = dh * tc * og * (1.f - og);
+  for (int r = blockIdx.y; r < R; r += gridDim.y) {
+    const long tok = addr.token(r, p);
+    const float* sv = saved + (tok * 2 + d) * (5L * H) + u;
+    const float ig = sv[0], fg = sv[H], gg = sv[2L * H], og = sv[3L * H], c = sv[4L * H];
+    float c_prev = 0.f;
+    if (p_prev >= 0 && p_prev < steps) c_prev = saved[(addr.token(r, p_prev) * 2 + d) * (5L * H) + 4L * H + u];
+    const long si = ((long)d * R + r) * H + u;
+    float dh = dy[tok * (2L * H) + (long)d * H + u];
+    float dc = 0.f;
+    if (q > 0) { dh += dh_rec[si]; dc = dc_carry[si]; }
+    const float tc = tanhf(c);
+    dc += dh * og * (1.f - tc * tc);
+    dc_carry[si] = dc * fg;
+    float* dg = dgates + (tok * 2 + d) * (4L * H) + u;
+    dg[0] = dc * gg * ig * (1.f - ig);
+    dg[H] = dc * c_prev * fg * (1.f - fg);
+    dg[2L * H] = dc * ig * (1.f - gg * gg);
+    dg[3L * H] = dh * tc * og * (1.f - og);
+  }
 }
 
 // dh_rec[d, r, k] = sum_n dgates[p, d, r, n] * W_hh[d, n, k]      (R x 4H) @ (4H x H); 64x64x16 tiles
@@ -235,7 +238,7 @@ extern "C" int bsrnn_blstm_train_bwd_f32(const float* dy, const float* saved, co
   BSRNN_CHECK_ARG(R > 0 && steps > 0 && H > 0 && seq_inner > 0, "blstm_train_bwd_f32: bad dims");
   SeqAddr addr{seq_inner, seq_outer, seq_inner_stride, step_stride};
   cudaStream_t st = (cudaStream_t)stream;
-  dim3 g1(cdiv(H, 256), R, 2), g2(cdiv(H, 64), cdiv(R, 64), 2);
+  dim3 g1(cdiv(H, 256), R < 65535 ? R : 65535, 2), g2(cdiv(H, 64), cdiv(R, 64), 2);
   for (int q = 0; q < steps; ++q) {
     lstm_bwd_gates_kernel<<<g1, 256, 0, st>>>(dy, saved, dh_rec, dc_carry, dgates, R, H, q, steps, addr);
     if (q + 1 < steps) lstm_bwd_dh_kernel<<<g2, 256, 0, st>>>(dgates, w_hh, dh_rec, R, H, q, steps, addr);
