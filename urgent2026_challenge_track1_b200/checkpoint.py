@@ -54,9 +54,11 @@ def from_reference_config(obj):
     return Config(**(dict(obj) if isinstance(obj, dict) else vars(obj)))
 
 
-def save_checkpoint(path, model, cfg, *, global_step=0, epoch=0, ema=None, optimizer_states=None, lr_schedulers=None):
+def save_checkpoint(path, model, cfg, *, global_step=0, epoch=0, ema=None, optimizer_states=None, lr_schedulers=None,
+                    extra=None):
     """Writes the dict Lightning's ModelCheckpoint writes.  ``model``: SEModel / FlowSEModel (keys ``se_model.*`` /
-    ``dnn.*``).  ``ema``: torch_ema-style state_dict (FlowSEModel.on_save_checkpoint, flow_model.py:95-96)."""
+    ``dnn.*``).  ``ema``: torch_ema-style state_dict (FlowSEModel.on_save_checkpoint, flow_model.py:95-96).  ``extra``:
+    further top-level keys (the training loop's ``b200_trainer`` state)."""
     sd = {k: v.detach().cpu().clone() for k, v in model.state_dict().items()}
     ckpt = {"epoch": int(epoch), "global_step": int(global_step), "pytorch-lightning_version": LIGHTNING_VERSION,
             "state_dict": sd, "loops": {}, "callbacks": {}, "optimizer_states": optimizer_states or [],
@@ -72,6 +74,7 @@ def save_checkpoint(path, model, cfg, *, global_step=0, epoch=0, ema=None, optim
             if e.get(k) is not None:
                 e[k] = [t.detach().cpu().clone() for t in e[k]]
         ckpt["ema"] = e
+    ckpt.update(extra or {})
     torch.save(ckpt, path)
     return path
 

@@ -43,8 +43,15 @@ def _str2bool(v):
     raise argparse.ArgumentTypeError("Boolean value expected.")
 
 
+# keys of this package that have no reference default: a flag sets them, and without the flag (or the YAML key) the
+# attribute stays absent, so every getattr(cfg, key, default) keeps its default
+_OPTIONAL_FLAGS = dict(train_precision=str, max_steps=int)
+
+
 def config_parser(argv=None):
     parser = argparse.ArgumentParser()
     for name, default in vars(Config()).items():
         parser.add_argument(f"--{name}", type=_str2bool if isinstance(default, bool) else type(default), default=default)
+    for name, typ in _OPTIONAL_FLAGS.items():
+        parser.add_argument(f"--{name}", type=typ, default=argparse.SUPPRESS)
     return parser.parse_args(argv)

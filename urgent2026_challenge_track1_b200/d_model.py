@@ -26,13 +26,20 @@ class SEModel(nn.Module):
         return self.se_model(noisy_speech, speech_length, fs)
 
     # ------------------------------------------------------------------------------------------------ training
-    def configure_optimizers(self, process_group=None):
+    def configure_optimizers(self, process_group=None, precision=None, cuda_graph=None):
         """AdamW(lr, eps=adam_epsilon, weight_decay) + StepLR(lr_step_size epochs, lr_gamma) + clip 0.5
-        [d_model.py:102-113, train_se.py:78] as one SETrainer (flat parameters, one allreduce, fused update)."""
+        [d_model.py:102-113, train_se.py:78] as one SETrainer (flat parameters, one allreduce, fused update).
+        precision None reads ``cfg.train_precision`` (default "fp32": the f32 kernels); cuda_graph None replays the
+        step as a CUDA graph exactly when the BLSTM blocks run on tensor cores ("fp16" / "bf16")."""
         from .training import SETrainer
         cfg = self.cfg
+        if precision is None:
+            precision = getattr(cfg, "train_precision", "fp32")
+        if cuda_graph is None:
+            cuda_graph = precision != "fp32"
         self.trainer_ = SETrainer(self.se_model, lr=cfg.learning_rate, weight_decay=cfg.weight_decay,
-                                  eps=cfg.adam_epsilon, gradient_clip=cfg.gradient_clip, process_group=process_group)
+                                  eps=cfg.adam_epsilon, gradient_clip=cfg.gradient_clip, process_group=process_group,
+                                  precision=precision, cuda_graph=cuda_graph)
         self.epoch_ = 0
         return self.trainer_
 

@@ -144,6 +144,12 @@ class FlowSEModel(nn.Module):
                                       precision=precision, cuda_graph=cuda_graph)
         return self.trainer_
 
+    def on_train_epoch_end(self):
+        """StepLR(step_size=lr_step_size, gamma=lr_gamma) of configure_optimizers [flow_model.py:238-249]."""
+        self.epoch_ = getattr(self, "epoch_", 0) + 1
+        if self.epoch_ % max(1, int(getattr(self.cfg, "lr_step_size", 1))) == 0:
+            self.trainer_.set_lr(self.trainer_.lr * getattr(self.cfg, "lr_gamma", 1.0))
+
     def training_step(self, batch, batch_idx=0):
         clean, noisy, fs, lengths = batch
         if not hasattr(self, "trainer_"):

@@ -16,32 +16,10 @@ import numpy as np
 import torch
 
 from .d_model import SEModel
+from .data import _probe_wav, _read_wav, read_scp
 from .flow_model import FlowSEModel
 from .pipeline import StreamedEnhancer
 from .sharding import shard_utterances
-
-
-def _to_float(x):
-    if x.dtype.kind == "i":
-        x = x.astype(np.float32) / float(np.iinfo(x.dtype).max + 1)
-    elif x.dtype.kind == "u":
-        x = (x.astype(np.float32) - 128.0) / 128.0
-    if x.ndim > 1:
-        x = x[:, 0]
-    return np.ascontiguousarray(x, dtype=np.float32)
-
-
-def _read_wav(path):
-    from scipy.io import wavfile
-    sr, x = wavfile.read(path)
-    return _to_float(x), int(sr)
-
-
-def _probe_wav(path):
-    """(n_samples, sample_rate) from the header only (memory-mapped read: no sample is touched)."""
-    from scipy.io import wavfile
-    sr, x = wavfile.read(path, mmap=True)
-    return int(x.shape[0]), int(sr)
 
 
 def _write_wav(path, x, sr):
@@ -56,16 +34,6 @@ def load_model(ckpt_path, device, precision=None):
     except KeyError:
         model = FlowSEModel.load_from_checkpoint(ckpt_path, map_location=device)
     return model.eval()
-
-
-def read_scp(path):
-    utts = []
-    with open(path) as f:
-        for line in f:
-            if line.strip():
-                uid, wav = line.strip().split()
-                utts.append((uid, wav))
-    return utts
 
 
 def _peak_normalise(y):

@@ -349,7 +349,12 @@ def bsrnn_se_train_forward(model, wav, lens, fs, blstm_fn=None):
     skip = dual_path_diff(core, skip, blstm_fn=blstm_fn)
     m_c, r_c = (mask_decoder_batched if BATCHED_BANDS else mask_decoder_diff)(core.mask_decoder, skip, plan, F_bins)
     est = m_c * torch.view_as_complex(spec) + r_c                               # (B,T,F)
-    L_out = int(torch.as_tensor(lens).max()) if not (torch.is_tensor(lens) and lens.is_cuda) else int(lens.max())
+    if torch.cuda.is_current_stream_capturing():
+        # reading device lengths would be a sync inside the capture: the output is the padded width, which is
+        # max(lengths) for every batch SETrainer replays (it checks that on the host)
+        L_out = wav.shape[1]
+    else:
+        L_out = int(torch.as_tensor(lens).max()) if not (torch.is_tensor(lens) and lens.is_cuda) else int(lens.max())
     wav_out = ISTFTFunction.apply(torch.view_as_real(est), L_out, n_fft, hop)
     return wav_out, est
 
@@ -448,7 +453,11 @@ class SETrainer:
         self.precision = precision
         self.block_fn = BLOCKS[precision]
         self.cuda_graph = bool(cuda_graph)
-        self._graphs = {}
+        self._graphs = {}                  # (noisy shape, clean shape, fs) -> captured step
+        self.captures = 0
+        self._seen = {}                    # shape -> peak device bytes of its first (eager) step
+        self._eager_only = set()           # shapes that did not fit beside the graphs kept
+        self.pool_bytes = {}               # signature -> device bytes of the private pool its capture took
         self.model = se_model
         self.loss_fn = loss_fn             # (model, noisy, clean, lengths, fs) -> (loss, logged scalar): other criteria
         self.flat = FlatParams(se_model)
@@ -488,6 +497,9 @@ class SETrainer:
     def step(self, noisy, clean, lengths, fs):
         if self.cuda_graph:
             return self._step_graphed(noisy, clean, lengths, fs)
+        return self._step_eager(noisy, clean, lengths, fs)
+
+    def _step_eager(self, noisy, clean, lengths, fs):
         self.flat.zero_grad()
         loss, sisnr = self.loss(noisy, clean, lengths, fs)
         loss.backward()
@@ -496,44 +508,101 @@ class SETrainer:
         return loss.detach(), sisnr
 
     # ---- CUDA-graph replay of forward + loss + backward (the step is launch-bound: ~8 700 kernels, profiles/r02 call05) ----
+    # Graphs are kept per (batch shape, rate), and a corpus with utterances shorter than max_duration has many shapes.  Each
+    # graph pins a private pool about as large as the eager step's peak, which depends on the model AND the rate (config 5
+    # on a B200: SE up to 9.7 GB; FlowSE at the published width 20.6 GB at 48 kHz, 67 GB at 8 kHz), so what fits is decided
+    # at run time from free device memory.  Evicting graphs to capture others thrashes when a corpus has more shapes than
+    # fit (measured on a seven-rate set: 420 ms per step against 90 ms eager), so graphs are kept and a shape that does not
+    # fit runs eager.
+    MAX_GRAPHS = 8
+
     def _step_graphed(self, noisy, clean, lengths, fs):
-        """One captured graph per batch signature (shapes, fs, lengths): zero_grad + forward + loss + backward + gather are
-        replayed; the allreduce and the fused optimizer tail stay eager (two kernels and one collective).  Random draws
-        inside the loss (FlowSE's t and z) use the graph-safe CUDA generator, so every replay draws afresh."""
-        lens_key = tuple(int(v) for v in torch.as_tensor(lengths).tolist())
-        key = (tuple(noisy.shape), tuple(clean.shape), int(fs), lens_key)
+        """One captured graph per batch shape and rate: zero_grad + forward + loss + backward + gather are replayed; the
+        allreduce and the fused optimizer tail stay eager (two kernels and one collective).  The lengths are device data
+        of the graph (a static buffer written before each replay), so one graph serves every batch of that shape; the
+        padded width must be the longest length, which the training collate guarantees (checked on the host for host
+        lengths; device lengths are checked once, at the first step of a shape, and must keep it after).
+
+        The first batch of a shape runs eager and measures its peak device memory (resetting the allocator's peak
+        statistics), so a width seen once costs no capture.  The second is captured if MAX_GRAPHS allows it and the free
+        device memory holds that peak (for the graph's pool) plus the largest eager peak seen (for the shapes that keep
+        running eager); otherwise that shape runs eager from then on.  Random draws inside the loss (FlowSE's t and z)
+        use the graph-safe CUDA generator, so every replay draws afresh."""
+        dev = self.flat.flat.device
+        lens_src = lengths if (torch.is_tensor(lengths) and lengths.is_cuda) else torch.as_tensor(lengths)
+        key = (tuple(noisy.shape), tuple(clean.shape), int(fs))
         entry = self._graphs.get(key)
+        if not lens_src.is_cuda or key not in self._seen:      # (host lengths: pinned from the loader, so the copy is async)
+            longest = int(lens_src.max())
+            if longest != noisy.shape[-1]:
+                raise ValueError(f"graphed step: max(lengths) = {longest} but the batch is padded to {noisy.shape[-1]}")
+        if entry is None and key not in self._seen:
+            torch.cuda.reset_peak_memory_stats(dev)
+            base = torch.cuda.memory_allocated(dev)
+            out = self._step_eager(noisy, clean, lengths, fs)
+            self._seen[key] = torch.cuda.max_memory_allocated(dev) - base
+            return out
+        if entry is None and key in self._eager_only:
+            return self._step_eager(noisy, clean, lengths, fs)
         if entry is None:
-            dev = self.flat.flat.device
+            torch.cuda.synchronize(dev)
+            torch.cuda.empty_cache()
+            need = self._seen[key] + max(self._seen.values())
+            if len(self._graphs) >= self.MAX_GRAPHS or torch.cuda.mem_get_info(dev)[0] < need:
+                self._eager_only.add(key)
+                return self._step_eager(noisy, clean, lengths, fs)
             n_s, c_s = torch.empty_like(noisy, device=dev), torch.empty_like(clean, device=dev)
-            n_s.copy_(noisy); c_s.copy_(clean)
+            l_s = torch.empty(lens_src.shape, dtype=torch.int32, device=dev)
+            n_s.copy_(noisy); c_s.copy_(clean); l_s.copy_(lens_src)
             side = torch.cuda.Stream(dev)
             side.wait_stream(torch.cuda.current_stream(dev))
             with torch.cuda.stream(side):                     # warm-up on a side stream (allocator, caches, lazy inits)
                 for _ in range(2):
                     self.flat.zero_grad()
-                    l0, _ = self.loss(n_s, c_s, lengths, fs)
+                    l0, _ = self.loss(n_s, c_s, l_s, fs)
                     l0.backward()
                     self.flat.gather_grads()
             torch.cuda.current_stream(dev).wait_stream(side)
             torch.cuda.synchronize(dev)
             touched = list(self.flat.touched)                  # hooks do not run at replay: the set is part of the signature
+            del l0
+            torch.cuda.empty_cache()                           # the warm-up's blocks go back before the pool is filled
+            free0 = torch.cuda.mem_get_info(dev)[0]
             g = torch.cuda.CUDAGraph()
             with torch.cuda.graph(g):
                 self.flat.zero_grad()
-                loss, logged = self.loss(n_s, c_s, lengths, fs)
+                loss, logged = self.loss(n_s, c_s, l_s, fs)
                 loss.backward()
                 self.flat.gather_grads()
-            if len(self._graphs) >= 4:
-                self._graphs.pop(next(iter(self._graphs)))
-            entry = self._graphs[key] = (g, n_s, c_s, loss, logged, touched)
-        g, n_s, c_s, loss, logged, touched = entry
+            torch.cuda.synchronize(dev)
+            self.pool_bytes[key] = free0 - torch.cuda.mem_get_info(dev)[0]
+            self.captures += 1
+            entry = self._graphs[key] = (g, n_s, c_s, l_s, loss, logged, touched)
+        g, n_s, c_s, l_s, loss, logged, touched = entry
         n_s.copy_(noisy, non_blocking=True)
         c_s.copy_(clean, non_blocking=True)
+        l_s.copy_(lens_src, non_blocking=True)
         g.replay()
         self.flat.touched = list(touched)
         self.apply_gradients()
         return loss.detach().clone(), logged.detach().clone()
+
+    # ---- trainer state (checkpoints, resume) ----
+    def state_dict(self):
+        """Optimizer state beside the weights: the flat AdamW moments, the flat EMA, the device counters, the lr."""
+        cpu = lambda t: None if t is None else t.detach().cpu().clone()
+        return {"numel": self.flat.numel, "exp_avg": cpu(self.exp_avg), "exp_avg_sq": cpu(self.exp_avg_sq),
+                "ema": cpu(self.ema), "stats": cpu(self.stats), "lr": float(self.lr)}
+
+    def load_state_dict(self, state):
+        if int(state["numel"]) != self.flat.numel or state["exp_avg"].numel() != self.exp_avg.numel():
+            raise ValueError(f"trainer state for {state['numel']} parameters, this model has {self.flat.numel}")
+        self.exp_avg.copy_(state["exp_avg"])
+        self.exp_avg_sq.copy_(state["exp_avg_sq"])
+        if self.ema is not None and state.get("ema") is not None:
+            self.ema.copy_(state["ema"])
+        self.stats.copy_(state["stats"])
+        self.lr = float(state["lr"])
 
     def allreduce_gradients(self):
         """ONE collective over the flat gradient buffer (sum; the 1/world factor is folded into the optimizer kernel).
@@ -642,3 +711,12 @@ class FlowSETrainer(SETrainer):
             for p, off in zip(self.flat.params, self.flat.offsets):
                 shadow[by_id[id(p)]].copy_(self.ema[off:off + p.numel()].view_as(p))
         self.model.ema.num_updates = n_upd
+
+    def load_ema_from_model(self):
+        """The inverse of sync_ema: ``model.ema`` (e.g. a checkpoint's ``ema`` entry) into the flat EMA and its counter."""
+        shadow = self.model.ema.shadow_params
+        by_id = {id(p): i for i, p in enumerate(self.model.parameters())}
+        with torch.no_grad():
+            for p, off in zip(self.flat.params, self.flat.offsets):
+                self.ema[off:off + p.numel()].copy_(shadow[by_id[id(p)]].reshape(-1))
+        self.stats[3] = float(self.model.ema.num_updates or 0)
