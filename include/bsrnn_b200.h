@@ -421,6 +421,36 @@ int bsrnn_axpy_complex(float* out, const float* y, const float* z, float sigma, 
 int bsrnn_complex_mask(float* out, const float* x, const float* mask, const float* resid, float sign, long n_complex,
                        void* stream);
 
+/* ---------------------------------------------------------------------------------------------- dynamic mixing
+ * The simulation chain of mixing.simulate (reverberation -> noise at an SNR -> bandwidth limitation -> clipping -> packet
+ * loss -> peak normalisation) [replaces the simulator's host-side functions that dataset.py:154-335 calls per utterance].
+ * Signals are (B, T) f32 rows, valid on [0, len[b]); every output is written as exact zeros on [len[b], T) and no padded
+ * input sample is read.  No floating-point atomics: the same inputs give bitwise-identical outputs.
+ * bsrnn_mix_conv: uniformly partitioned overlap-save FFT convolution (P = 1024, FFT 2048; twiddle from
+ *   bsrnn_fft_twiddle(2048)).  For each filter f < nfilt: y (nfilt, B, T), y[f, b, s] = sum_m h[b, m] x[b, s + off_b - m]
+ *   with h (B, Lh) zero at and beyond h_len[b * nfilt + f], x zero outside [0, x_len[b]); off_b = (h_len[b * nfilt] - 1)/2
+ *   if `centered` (a zero-phase FIR), else 0.  h_len 0 copies x.  The filters of one utterance share its input spectrum.
+ *   scratch: bsrnn_mix_conv_scratch_bytes(B, T, Lh, nfilt) bytes = (B ceil(T/1024) + nfilt B ceil(Lh/1024)) 2048 complex64.
+ * bsrnn_mix_snr: noisy = speech + g noise, g = 10^(-snr_db/20) sqrt(P_s / max(P_n, 1e-10)), P the active-level power: the
+ *   mean of the 1024-sample frames' (hop 512) mean squares that exceed 0.01 x their mean over the utterance (an utterance
+ *   shorter than a frame is one frame).  gain (B) f32 receives g (may be NULL).  scratch:
+ *   bsrnn_mix_snr_scratch_bytes(B, T) bytes.
+ * bsrnn_mix_quantiles: thr (B, 2) f32 = np.quantile(x[b, :len[b]], q[b, i], method="linear") for q (B, 2) f64, by radix
+ *   select over the order-preserving uint32 image; one CTA per utterance.
+ * bsrnn_mix_finish: in place, over s < len[b]: noisy = clamp(noisy, thr[b, 0], thr[b, 1]), zeroed where lost (B, npk)
+ *   uint8 marks packet s / pkt (lost may be NULL); then noisy and clean are scaled by 0.9 / peak when the joint peak of
+ *   |noisy| and |clean| exceeds 0.9.  peak: B uint32 of scratch.
+ */
+long bsrnn_mix_conv_scratch_bytes(int B, int T, int Lh, int nfilt);
+int bsrnn_mix_conv(const float* x, const int32_t* x_len, const float* h, const int32_t* h_len, float* y, float* scratch,
+                   const float* twiddle, int B, int T, int Lh, int nfilt, int centered, void* stream);
+long bsrnn_mix_snr_scratch_bytes(int B, int T);
+int bsrnn_mix_snr(const float* speech, const float* noise, const int32_t* len, const float* snr_db, float* noisy,
+                  float* gain, double* scratch, int B, int T, void* stream);
+int bsrnn_mix_quantiles(const float* x, const int32_t* len, const double* q, float* thr, int B, int T, void* stream);
+int bsrnn_mix_finish(float* noisy, float* clean, const int32_t* len, const float* thr, const uint8_t* lost, int npk, int pkt,
+                     uint32_t* peak, int B, int T, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

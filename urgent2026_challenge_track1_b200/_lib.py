@@ -102,6 +102,12 @@ PROTOTYPES = {
     "bsrnn_euler_step": [c_void_p, c_void_p, c_void_p, c_float, c_long, c_void_p],
     "bsrnn_axpy_complex": [c_void_p, c_void_p, c_void_p, c_float, c_long, c_void_p],
     "bsrnn_complex_mask": [c_void_p, c_void_p, c_void_p, c_void_p, c_float, c_long, c_void_p],
+    "bsrnn_mix_conv_scratch_bytes": [c_int, c_int, c_int, c_int],
+    "bsrnn_mix_conv": [c_void_p] * 7 + [c_int, c_int, c_int, c_int, c_int, c_void_p],
+    "bsrnn_mix_snr_scratch_bytes": [c_int, c_int],
+    "bsrnn_mix_snr": [c_void_p] * 7 + [c_int, c_int, c_void_p],
+    "bsrnn_mix_quantiles": [c_void_p] * 4 + [c_int, c_int, c_void_p],
+    "bsrnn_mix_finish": [c_void_p] * 5 + [c_int, c_int, c_void_p, c_int, c_int, c_void_p],
 }
 
 # mirrors `bsrnn_gemm_desc` (include/bsrnn_b200.h); 144 bytes
@@ -143,6 +149,8 @@ def lib():
         handle.bsrnn_launch_count.restype = C.c_long
         handle.bsrnn_blstm_fused_train_scratch_bytes.restype = C.c_long
         handle.bsrnn_blstm_fused768_train_scratch_bytes.restype = C.c_long
+        handle.bsrnn_mix_conv_scratch_bytes.restype = C.c_long
+        handle.bsrnn_mix_snr_scratch_bytes.restype = C.c_long
         handle.bsrnn_last_error.restype = C.c_char_p
         handle.bsrnn_last_error.argtypes = []
         _lib = handle

@@ -183,19 +183,21 @@ def make_loader(corpus, batches, max_len, train, num_workers, seed=0, epoch=0):
 
 
 def prefetch_to_device(batches, device):
-    """Copies clean / noisy of batch i+1 to the device on a side stream while the caller works on batch i (the pattern of
-    pipeline.StreamedEnhancer).  fs and lengths stay on the host: the training step reads them there."""
+    """Copies the leading tensors of batch i+1 (all but the last two entries: clean / noisy of a pair batch, the signals
+    of a mixing batch) to the device on a side stream while the caller works on batch i (the pattern of
+    pipeline.StreamedEnhancer).  The last two entries (fs and lengths, or fs and the mixing parameters) stay on the host:
+    the caller reads them there."""
     copy = torch.cuda.Stream(device)
     cur = torch.cuda.current_stream(device)
 
     def submit(b):
-        clean, noisy, fs, lens = b
+        *lead, fs, tail = b
         with torch.cuda.stream(copy):
             copy.wait_stream(cur)               # blocks the allocator may hand out could still be read by queued work
-            c, n = clean.to(device, non_blocking=True), noisy.to(device, non_blocking=True)
+            lead = [t.to(device, non_blocking=True) for t in lead]
             ev = torch.cuda.Event()
             ev.record(copy)
-        return (c, n, fs, lens), ev
+        return (*lead, fs, tail), ev
 
     pending = None
     for b in batches:
@@ -208,11 +210,11 @@ def prefetch_to_device(batches, device):
 
 
 def _ready(pending, cur):
-    (c, n, fs, lens), ev = pending
+    b, ev = pending
     cur.wait_event(ev)
-    c.record_stream(cur)
-    n.record_stream(cur)
-    return c, n, fs, lens
+    for t in b[:-2]:
+        t.record_stream(cur)
+    return b
 
 
 # ------------------------------------------------------------------------------------------------ checkpoint files

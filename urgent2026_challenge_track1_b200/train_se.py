@@ -18,8 +18,11 @@ length-bucketed batches of ``batch_size`` cropped to ``max_duration`` samples, r
 ``valid_set_path`` adds a validation pass every ``val_check_interval`` global steps and at the end; rank 0 keeps the best
 ``save_top_k`` checkpoints by ``val_loss`` under ``exp/<train_tag>/<train_name>/version_<v>/checkpoints/``, named
 ``best_epoch=EE-step=SSSSSS-val_loss=V.VVV.ckpt``, with the optimizer state under ``b200_trainer``; ``resume: true``
-continues from the newest of them.  StepLR (``lr_step_size`` epochs, ``lr_gamma``) runs at each epoch end.  Dynamic
-mixing (``train_set_dynamic_mixing: true``) is not built.  With ``train_set_path: none`` the run trains ``max_steps``
+continues from the newest of them.  StepLR (``lr_step_size`` epochs, ``lr_gamma``) runs at each epoch end.  With
+``train_set_dynamic_mixing: true`` the training set is a dynamic-mixing set instead (``speech.scp``, ``noise.scp``,
+optional ``rir.scp``; mixing.py): the workers read speech, noise and RIRs, and mixing.simulate makes a new noisy / clean
+pair per utterance and epoch on the GPU, with the parameters of the optional ``dynamic_mixing:`` YAML mapping; validation
+stays a pre-simulated set.  With ``train_set_path: none`` the run trains ``max_steps``
 steps on synthetic (clean, noisy) pairs of the dataset contract -- (clean (B,1,T), noisy (B,1,T), fs int32 scalar,
 lengths (B,) int32), one fs per batch (dataset.py:417,441) -- and ``save: true`` writes ``last-step<N>.ckpt``.
 """
@@ -138,19 +141,24 @@ def validate(model, trainer, corpus, cfg, rank, world, dev, flowse):
 
 
 def fit_corpus(model, cfg, rank, world, dev, flowse, out_dir, log_every=10):
-    """Epochs over the pre-simulated set of ``train_set_path`` with periodic validation, top-k checkpoints and resume.
+    """Epochs over the set of ``train_set_path`` (pre-simulated pairs, or dynamic mixing) with periodic validation, top-k
+    checkpoints and resume.
     -> {"global_step", "epoch", "val": [logged dicts with "step" and "epoch"], "checkpoints": [paths kept]}."""
     import warnings
     from . import data as D
     from . import runtime as R
     from .checkpoint import load_checkpoint, save_checkpoint
-    if cfg.train_set_dynamic_mixing:
-        raise NotImplementedError("dynamic mixing is not built: a pre-simulated set (wav.scp + spk1.scp) needs "
-                                  "train_set_dynamic_mixing: false")
+    from . import mixing as M
+    mixing = bool(cfg.train_set_dynamic_mixing)
+    if mixing and not M.is_mix_set(cfg.train_set_path):
+        raise NotImplementedError(f"{cfg.train_set_path}: dynamic mixing reads a set of speech.scp + noise.scp (+ optional "
+                                  "rir.scp); a pre-simulated set (wav.scp + spk1.scp) needs train_set_dynamic_mixing: false")
+    mix_params = M.mix_params(cfg) if mixing else None
     if rank == 0 and getattr(cfg, "use_high_pass", False):
-        print("note: use_high_pass is not applied by the pre-simulated corpus loader", flush=True)
+        print(f"note: use_high_pass is not applied by {'dynamic mixing' if mixing else 'the pre-simulated corpus loader'}",
+              flush=True)
     max_len = int(cfg.max_duration)
-    train = D.PairCorpus(cfg.train_set_path)
+    train = M.MixCorpus(cfg.train_set_path) if mixing else D.PairCorpus(cfg.train_set_path)
     valid = D.PairCorpus(cfg.valid_set_path) if cfg.valid_set_path != "none" else None
     trainer = _configure(model, cfg, flowse)
     epoch, global_step, skip, last_val = 0, 0, 0, -1
@@ -206,9 +214,13 @@ def fit_corpus(model, cfg, rank, world, dev, flowse, out_dir, log_every=10):
         batches, dropped = D.train_batches(train, cfg.batch_size, max_len, rank, world, epoch, cfg.seed)
         if rank == 0 and skip == 0:
             print(f"epoch {epoch}: {len(batches)} batches per rank, {dropped} utterances dropped (uneven tail)", flush=True)
-        loader = D.make_loader(train, batches[skip:], max_len, True, cfg.num_worker, seed=cfg.seed, epoch=epoch)
+        if mixing:
+            loader = M.make_loader(train, batches[skip:], max_len, mix_params, cfg.num_worker, cfg.seed, epoch)
+        else:
+            loader = D.make_loader(train, batches[skip:], max_len, True, cfg.num_worker, seed=cfg.seed, epoch=epoch)
         done = skip
-        for clean, noisy, fs, lens in D.prefetch_to_device(loader, dev):
+        for batch in D.prefetch_to_device(loader, dev):
+            clean, noisy, fs, lens = M.simulate(batch, dev) if mixing else batch
             loss, _ = trainer.step(noisy, clean, lens, fs)
             done += 1
             global_step += 1
