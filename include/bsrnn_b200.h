@@ -195,8 +195,7 @@ int bsrnn_gemm_tc_grouped(const void* A, const void* W, const float* bias, void*
                           long tokens_per_sample, int tiles_per_step, int R, long seq_inner, long seq_outer,
                           long seq_inner_stride, long step_stride, void* stream);
 /* bsrnn_gemm_tc_limit_ctas: upper bound on the persistent CTAs of the following bsrnn_gemm_tc* launches of this process (0 =
- *     every SM); returns the previous bound.  The mask decoder's two MLP families [espnet2 MaskDecoder: mlp_mask /
- *     mlp_residual] run on two streams with half of the SMs each. */
+ *     every SM); returns the previous bound.  With a few CTAs, each CTA walks many tiles of one launch. */
 int bsrnn_gemm_tc_limit_ctas(int n);
 int bsrnn_band_norm_cast_kb8(const float* spec, const float* scale, const float* shift, void* out, const int32_t* c_off,
                              const int32_t* bin0, const int32_t* width2, const long long* a_off, int K, long rows, int T,

@@ -20,9 +20,9 @@ swapped rows, one element 3x its bound off) and asserts that the checker rejects
 
 Each GEMM case runs on the default persistent grid and under bsrnn_gemm_tc_limit_ctas (3 CTAs, or n_tiles for the
 weight-resident schedule) so that every CTA walks many tiles: both TMEM accumulators and their phase flips, the row-buffer
-refill of epilogue 8, and the later steps of the tile iterator (reverse M, band innermost, grouped).  Launcher switches
-that select other device code, and the BSRNN_GEMM_DEBUG modes that break the result on purpose, are read once per process:
-they run in child pytest processes of this file (the switches must pass, the debug modes must fail).
+refill of epilogue 8, and the later steps of the tile iterator (reverse M, band innermost, grouped).  The BSRNN_GEMM_DEBUG
+modes that break the result on purpose are read once per process: they run in child pytest processes of this file, and
+each must fail.
 """
 import math
 import os
@@ -577,25 +577,6 @@ def run_child(env_var, value, kexpr):
 
 
 child_only = pytest.mark.skipif(os.environ.get(CHILD) == "1", reason="runs in the parent process only")
-
-# launcher switches that select other device code -> the cases whose path they change
-AB_SWITCHES = [
-    ("BSRNN_FC_TMAP", "0", "epi8 or grouped or store"),
-    ("BSRNN_FC_RUNS", "0", "time and (epi8 or store)"),
-    ("BSRNN_FC_BAND_INNER", "0", "epi8_band"),
-    ("BSRNN_TANH_BULK", "0", "tanhkb8"),
-    ("BSRNN_GLU_REVERSE", "0", "glu"),
-    ("BSRNN_GEMM_KS", "4", "epi1_band or f16rows_h768"),          # the two cases whose 4-stage ring becomes 8 x 4 k-cores
-    ("BSRNN_GEMM_STAGES", "4", "f16rows or generic or glu or tanh32 or epi1"),
-]
-
-
-@child_only
-@pytest.mark.parametrize("env_var,value,kexpr", AB_SWITCHES, ids=[f"{a}={b}" for a, b, _ in AB_SWITCHES])
-def test_launcher_switch_passes(env_var, value, kexpr):
-    rc, tail = run_child(env_var, value, kexpr)
-    print(tail)
-    assert rc == 0 and " passed" in tail, f"{env_var}={value}: child exit {rc}\n{tail}"
 
 
 # BSRNN_GEMM_DEBUG modes that break the result on purpose (all stay in bounds) -> a case that must catch it

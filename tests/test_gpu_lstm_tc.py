@@ -257,7 +257,7 @@ STEP_CASES = {
     "h392_bn224_m2": (392, 224, 7, 2),
     "h392_bn256_cover_m1": (392, 256, 7, 1),          # 1792 > 1568
     "h768_bn256_m3": (768, 256, 12, 3),
-    "h768_bn96_m5": (768, 96, 32, 5),                 # the shape whose launch takes the resident / multicast path when enabled
+    "h768_bn96_m5": (768, 96, 32, 5),
 }
 
 
@@ -952,13 +952,7 @@ def run_child(env, kexpr):
 
 child_only = pytest.mark.skipif(os.environ.get(CHILD) == "1", reason="runs in the parent process only")
 SWITCHES = [
-    # resident W_hh + h multicast (gemm_tc.cu launch_tc): 2 x 32 N tiles of 96 and 5 row tiles per direction qualify
-    ({"BSRNN_STEP_RESIDENT": "1", "BSRNN_STEP_MC": "1"}, "h768_bn96_m5 and not single"),
-    ({"BSRNN_STEP_RESIDENT": "1", "BSRNN_STEP_MC": "2"}, "h768_bn96_m5 and not single"),
-    ({"BSRNN_STEP_RESIDENT": "1", "BSRNN_STEP_MC": "4"}, "h768_bn96_m5 and not single"),
     ({"BSRNN_FUSED14_CLS": "4"}, "fused_layer and g14 and not g14S"),
-    ({"BSRNN_GEMM_STAGES": "4"}, "(step_kernel and h768) or bwd_step"),
-    ({"BSRNN_GEMM_KS": "4"}, "step_kernel and h768_bn256"),
 ]
 
 

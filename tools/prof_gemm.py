@@ -54,4 +54,4 @@ for _ in range(a.reps):
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record(); run(); e1.record(); torch.cuda.synchronize()
     ms = e0.elapsed_time(e1)
-    print(f"[gemm {a.which} {a.axis}{' nobias' if a.nobias else ''}{' tma' if a.tma else ''} stages={os.environ.get('BSRNN_GEMM_STAGES', '8')}] {ms:.3f} ms  {bytes_alg / ms / 1e6:.0f} GB/s algorithmic  {flops / ms / 1e9:.0f} TFLOP/s", flush=True)
+    print(f"[gemm {a.which} {a.axis}{' nobias' if a.nobias else ''}{' tma' if a.tma else ''}] {ms:.3f} ms  {bytes_alg / ms / 1e6:.0f} GB/s algorithmic  {flops / ms / 1e9:.0f} TFLOP/s", flush=True)

@@ -25,16 +25,14 @@
 namespace bsrnn {
 using namespace umma;
 
-constexpr int TC_STAGES = 8;       // barrier slots; a launch uses a.stages (4 or 8) of them
-constexpr int TC_KS = 8;            // default k-cores (8 halves each) per pipeline stage -> K = 64 per stage (a.ks: 8 or 4)
+constexpr int TC_STAGES = 8;       // barrier slots; a launch uses a.stages (<= 8, chosen by shared-memory fit) of them
+constexpr int TC_KS = 8;            // k-cores (8 halves each) per pipeline stage -> K = 64 per stage
 constexpr int TC_EPI_WARPS = 8;
 // Epilogue warps per CTA.  The residual epilogue (Linear + skip) runs 12 (16 would cap the kernel at 96 registers and spill 4 KB): it is a scattered-row read-modify-write of the f32
 // residual stream whose cost is set by the bytes its warps keep in flight (profiles/r02 call43: 0.81 ms without the
-// residual traffic, 1.45 ms store-only, 1.80 ms full, all with 8 warps).  -DBSRNN_RESID_EPI_WARPS=8 restores 8.
-#ifndef BSRNN_RESID_EPI_WARPS
-#define BSRNN_RESID_EPI_WARPS 12
-#endif
-__host__ __device__ constexpr int tc_epi_warps(int epi) { return (epi == 1 /* EPI_RESID_F32 */ || epi == 8 /* EPI_RESID_TMA */) ? BSRNN_RESID_EPI_WARPS : TC_EPI_WARPS; }
+// residual traffic, 1.45 ms store-only, 1.80 ms full, all with 8 warps).
+constexpr int TC_RESID_EPI_WARPS = 12;
+__host__ __device__ constexpr int tc_epi_warps(int epi) { return (epi == 1 /* EPI_RESID_F32 */ || epi == 8 /* EPI_RESID_TMA */) ? TC_RESID_EPI_WARPS : TC_EPI_WARPS; }
 __host__ __device__ constexpr int tc_threads(int epi) { return (2 + tc_epi_warps(epi)) * 32; }
 constexpr int TC_SCR_LD = 36;                                   // floats per scratch row (32 + 4: conflict-free 16 B rows)
 constexpr int TC_SCR_BYTES = tc_epi_warps(1) * 32 * TC_SCR_LD * 4;  // residual epilogue only
@@ -74,30 +72,24 @@ struct GemmTcArgs {
   int out_kcores;                   // EPI_TANH_KB8: k-cores of the destination operand
   int b_resident;                   // 1: each CTA keeps ONE weight tile in shared memory and streams A tiles only
   int pf_dist;                      // A tile this many tiles ahead is bulk-prefetched into L2 (0 = off)
-  int ks;                           // k-cores per pipeline stage (TC_KS, or 4: twice the stages in the same shared memory)
   const __half* gx;                 // EPI_LSTM_STEP: input projection rows [m*128 + r][ld_gx] fp16 (this step, this direction)
   float* cstate;                    // EPI_LSTM_STEP: cell state [m*128 + r][H] f32 (this direction), updated in place
   long ld_gx;
   int H;
-  // EPI_LSTM_STEP, both directions in one launch: row tiles m >= dir_tiles belong to the second direction and use the
-  // *2 pointers with m - dir_tiles (0 = single direction)
+  // EPI_LSTM_STEP / EPI_LSTM_BWD, both directions in one launch (streaming schedule): row tiles m >= dir_tiles belong to
+  // the second direction and use the *2 pointers with m - dir_tiles (0 = single direction)
   int dir_tiles;
   const __half* A2; const __half* W2; const __half* gx2; float* cstate2; void* out2;
   int debug;                        // BSRNN_GEMM_DEBUG (A/B experiments on the input projection): 1 = every tile
                                     // writes the first tile's output block (stores stay in L2), 2 = no stores
   int stages;                       // pipeline depth: 8 when the shared memory allows (short-K GEMMs: one tile is 4 stages,
-                                    // and a ring of one tile exposes the HBM latency of every A tile), else 4
+                                    // and a ring of one tile exposes the HBM latency of every A tile), else 4 (3 if 4 do not fit)
   RowMap rows;
   float out_scale;                  // EPI_RESID_F32: the accumulator is multiplied by this before it is added (0 = 1)
   const float* out_scale_ptr;       // ... or by *out_scale_ptr (device scalar: no host sync to learn the loss scale)
   // split-K (EPI_RESID_F32 with atomic adds; weight-gradient GEMMs: few output tiles, K = tokens): the launch iterates
   // over m_tiles = m_log * ksplit tiles; tile m' = split * m_log + m covers k-cores [split*kps, split*kps + kps)
   int ksplit, kps, m_log;
-  // A-tile multicast (weight-resident schedule): the launch runs in clusters of `mc` CTAs that own consecutive N tiles of
-  // the same M-tile walk; each fetches 1/mc of every A stage and multicasts it into all mc shared memories, so the L2->SM
-  // traffic of the operand every N tile re-reads drops by mc (the input projection re-read xhat 16 times: 14.5 GB of L2
-  // reads per launch next to 13.9 GB of writes -- the kernel sat on the L2, not on HBM)
-  int mc;
   // training (EPI_LSTM_STEP with save_gates, EPI_LSTM_BWD)
   int save_gates;                   // EPI_LSTM_STEP: write the ACTIVATED gates i,f,g,o back over gx (fp16, same columns) and
                                     // c_t to cstate_out (c_{t-1} is read from cstate; null = zeros): what BPTT needs
@@ -115,10 +107,6 @@ struct GemmTcArgs {
   // adjacent 784-byte segments of the same output rows.
   const long long* groups;
   int n_groups;
-  // L2 residency of the MaskDecoder's hidden activation (the same 100 MB buffer is written by every band's Conv1d+Tanh and
-  // read back by its Conv1d+GLU): bit 0 = bulk stores of the output (EPI_TANH_KB8 / BNC = 208), bit 1 = bulk loads of the A
-  // operand carry the evict_last policy, so the buffer stays in the 126 MB L2 instead of making a DRAM round trip per band
-  int l2_keep;
   // streaming launches with one N tile walk the M tiles from the LAST one down: the MaskDecoder's Conv1d+GLU GEMM reads the 100 MB
   // hidden tile its predecessor has just written in ascending order, so the most recently written (still L2-resident) tiles come
   // first instead of the evicted ones
@@ -436,25 +424,12 @@ __device__ __forceinline__ void epilogue_chunk(const GemmTcArgs& a, int m, int n
 // The schedule above as an iterator without a division per tile: the control warps have ~1 350 cycles of MMA per tile at
 // K = 208 and every dependent integer division costs them ~150 (profiles/r01/call32: the MMA warp spent more time
 // between tiles than issuing).
-// Weight-resident mode with two directions in one launch (dir_tiles > 0: M tiles [0, dir_tiles) use W, the rest W2): a CTA
-// owns the VIRTUAL N tile (direction, n) -- blockIdx % (2 n_tiles) -- and walks only its direction's M tiles.
 struct TileIter {
   int m, n;
-  int dm, dn, n_tiles, m_tiles;     // m_tiles = end of this CTA's M range
+  int dm, dn, n_tiles, m_tiles;
   bool resident;
   __device__ __forceinline__ TileIter(const GemmTcArgs& a) {
     n_tiles = a.n_tiles; m_tiles = a.m_tiles; resident = a.b_resident != 0;
-    if (resident && a.dir_tiles > 0) {
-      const int nt2 = 2 * n_tiles;
-      const int vn = (int)blockIdx.x % nt2;
-      const int dir = vn / n_tiles;
-      n = vn - dir * n_tiles;
-      dm = (int)gridDim.x / nt2;
-      m = dir * a.dir_tiles + (int)blockIdx.x / nt2;
-      m_tiles = dir == 0 ? a.dir_tiles : a.m_tiles;
-      dn = 0;
-      return;
-    }
     n = (int)blockIdx.x % n_tiles;
     m = (int)blockIdx.x / n_tiles;
     dm = (int)gridDim.x / n_tiles;
@@ -523,7 +498,7 @@ template <int EPI, int BNC = 0>
 __global__ void __launch_bounds__(tc_threads(EPI), 1) gemm_tc_kernel(const __grid_constant__ GemmTcArgs a) {
   extern __shared__ __align__(128) uint8_t smem[];
   const int BN = a.BN;
-  const int KS = a.ks;
+  constexpr int KS = TC_KS;
   const uint32_t a_stage_bytes = KS * 128 * 16;
   const uint32_t b_stage_bytes = KS * BN * 16;
   uint8_t* sA = smem;
@@ -542,7 +517,7 @@ __global__ void __launch_bounds__(tc_threads(EPI), 1) gemm_tc_kernel(const __gri
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   if (threadIdx.x == 0) {
-    for (int i = 0; i < TC_STAGES; ++i) { mbar_init(full + i, 1); mbar_init(empty + i, a.mc > 1 ? a.mc : 1); }
+    for (int i = 0; i < TC_STAGES; ++i) { mbar_init(full + i, 1); mbar_init(empty + i, 1); }
     for (int i = 0; i < 2; ++i) { mbar_init(acc_full + i, 1); mbar_init(acc_empty + i, BNC ? TC_EPI_WARPS / 2 : tc_epi_warps(EPI)); }
     mbar_init(b_full, 1);
     mbar_init(res_full, 128);
@@ -551,11 +526,8 @@ __global__ void __launch_bounds__(tc_threads(EPI), 1) gemm_tc_kernel(const __gri
   if (warp == 2) tmem_alloc(tmem_slot, 2 * TC_ACC_COLS);
   tc_fence_before();
   __syncthreads();
-  if (a.mc > 1) cluster_sync();          // every CTA's barriers exist before a peer multicasts into it
   tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
-  const uint32_t crank = a.mc > 1 ? cluster_ctarank() : 0u;
-  const uint16_t cmask = (uint16_t)((1u << (a.mc > 1 ? a.mc : 1)) - 1u);
 
   // Control warps: the whole role runs inside ONE `if (elect_one())` region.  The compiler then knows a single
   // thread executes it and emits back-to-back UTCHMMA / UBLKCP / UTCBAR with descriptors in uniform registers.  Under
@@ -573,8 +545,7 @@ __global__ void __launch_bounds__(tc_threads(EPI), 1) gemm_tc_kernel(const __gri
         pf_mod = t3.m % a.n_tiles; pf_dmod = ti.dm % a.n_tiles;
       }
       if (a.b_resident && ti.valid()) {
-        const uint8_t* gB = reinterpret_cast<const uint8_t*>((a.dir_tiles > 0 && ti.m >= a.dir_tiles) ? a.W2 : a.W) +
-                            (size_t)ti.n * a.kcores * BN * 16;
+        const uint8_t* gB = reinterpret_cast<const uint8_t*>(a.W) + (size_t)ti.n * a.kcores * BN * 16;
         const uint32_t bytes = (uint32_t)a.kcores * BN * 16;
         mbar_expect_tx(b_full, bytes);
         for (uint32_t off = 0; off < bytes; off += 32768) bulk_g2s(sB + off, gB + off, min(32768u, bytes - off), b_full);
@@ -606,13 +577,6 @@ __global__ void __launch_bounds__(tc_threads(EPI), 1) gemm_tc_kernel(const __gri
           const int nk = min(KS, kcnt - kc0);
           mbar_wait(empty + stage, phase ^ 1);
           mbar_expect_tx(full + stage, (uint32_t)nk * (2048 + (a.b_resident ? 0 : BN * 16)));
-          if (a.mc > 1) {                  // my 1/mc of the stage, into the same ring slot of every CTA of the cluster
-            const uint32_t slice = (uint32_t)nk * 2048 / (uint32_t)a.mc;
-            bulk_g2s_multicast(sA + stage * a_stage_bytes + crank * slice, gA + (size_t)kc0 * 2048 + crank * slice, slice,
-                               full + stage, cmask);
-          } else if (a.l2_keep & 2)
-            bulk_g2s_hint(sA + stage * a_stage_bytes, gA + (size_t)kc0 * 2048, nk * 2048, full + stage, l2_policy_evict_last());
-          else
           bulk_g2s(sA + stage * a_stage_bytes, gA + (size_t)kc0 * 2048, nk * 2048, full + stage);
           if (!a.b_resident)
             bulk_g2s(sB + stage * b_stage_bytes, gB + (size_t)kc0 * BN * 16, nk * BN * 16, full + stage);
@@ -647,8 +611,7 @@ __global__ void __launch_bounds__(tc_threads(EPI), 1) gemm_tc_kernel(const __gri
             const uint64_t da = da0 + (uint64_t)(stage * (a_stage_bytes >> 4));
             const uint64_t db = db0 + (uint64_t)(a.b_resident ? (uint32_t)ks * (KS / 2) * b_step : stage * (b_stage_bytes >> 4));
             for (int j = 0; j < nk / 2; ++j) mma_f16_ss(d_tmem, da + (uint64_t)(j * a_step), db + (uint64_t)(j * b_step), idesc, (ks | j) != 0);
-            if (a.mc > 1) mma_commit_multicast(empty + stage, cmask);     // the slot is free once ALL mc CTAs have read it
-            else mma_commit(empty + stage);
+            mma_commit(empty + stage);
             if (++stage == NST) { stage = 0; phase ^= 1; }
           }
           mma_commit(acc_full + buf);
@@ -714,10 +677,7 @@ __global__ void __launch_bounds__(tc_threads(EPI), 1) gemm_tc_kernel(const __gri
         store_kb8_cores_smem<2>(my_stg + 12 * 2048, v3);
         fence_proxy_async_shared();                                     // generic-proxy smem writes -> the bulk copy's reads
         named_bar_sync(bar_id, 128);
-        if (leader && do_store && nA) {
-          if (EPI == EPI_TANH_KB8 && (a.l2_keep & 1)) bulk_s2g_hint(gdst, stg, nA * 2048, l2_policy_evict_last());
-          else bulk_s2g(gdst, stg, nA * 2048);
-        }
+        if (leader && do_store && nA) bulk_s2g(gdst, stg, nA * 2048);
         tmem_ld_x32(t_row + 112, v0);
         tmem_ld_x32(t_row + 144, v1);
         tmem_ld_x32(t_row + 176, v2);
@@ -735,10 +695,7 @@ __global__ void __launch_bounds__(tc_threads(EPI), 1) gemm_tc_kernel(const __gri
         else store_kb8_cores_smem<3>(my_stg + 8 * 2048, v2);            // core 25 (columns 200..207) is padding nobody reads
         fence_proxy_async_shared();
         named_bar_sync(bar_id, 128);
-        if (leader && do_store && nB) {
-          if (EPI == EPI_TANH_KB8 && (a.l2_keep & 1)) bulk_s2g_hint(gdst + 14 * 2048, stg, nB * 2048, l2_policy_evict_last());
-          else bulk_s2g(gdst + 14 * 2048, stg, nB * 2048);
-        }
+        if (leader && do_store && nB) bulk_s2g(gdst + 14 * 2048, stg, nB * 2048);
       }
       if (leader) bulk_store_wait_all();
     } else if constexpr (EPI == EPI_RESID_TMA) {
@@ -1001,16 +958,15 @@ __global__ void __launch_bounds__(tc_threads(EPI), 1) gemm_tc_kernel(const __gri
   }
   tc_fence_before();
   __syncthreads();
-  if (a.mc > 1) cluster_sync();          // no CTA exits while peers may still multicast into it / arrive on its barriers
   if (warp == 2) {
     tc_fence_after();
     tmem_dealloc(tmem_base, 2 * TC_ACC_COLS);
   }
 }
 
-static size_t tc_smem_bytes(int BN, int kcores, bool resident, bool scratch, int stages, int ksz = TC_KS, size_t extra = 0) {
-  const size_t b = resident ? (size_t)kcores * BN * 16 : (size_t)stages * ksz * BN * 16;
-  return (size_t)stages * ksz * 128 * 16 + b + (2 * TC_STAGES + 8) * 8 + (scratch ? TC_SCR_BYTES : 0) + extra;
+static size_t tc_smem_bytes(int BN, int kcores, bool resident, bool scratch, int stages, size_t extra = 0) {
+  const size_t b = resident ? (size_t)kcores * BN * 16 : (size_t)stages * TC_KS * BN * 16;
+  return (size_t)stages * TC_KS * 128 * 16 + b + (2 * TC_STAGES + 8) * 8 + (scratch ? TC_SCR_BYTES : 0) + extra;
 }
 // EPI_RESID_TMA: 128 residual rows of min(BN, n_valid) floats, row stride padded to 4 (mod 8) floats
 static size_t tc_resbuf_bytes(int BN, int n_valid) {
@@ -1019,17 +975,13 @@ static size_t tc_resbuf_bytes(int BN, int n_valid) {
   return (size_t)128 * ldr * 4;
 }
 
-// Upper bound on the persistent CTAs of the following bsrnn_gemm_tc* launches (0 = every SM).  The mask decoder runs its two
-// MLP families on two streams: with each launch on half of the SMs the Conv1d+Tanh GEMM of one family (MUFU / store path)
-// and the Conv1d+GLU GEMM of the other (HBM reads) share the chip instead of taking turns on all of it.
+// Upper bound on the persistent CTAs of the following bsrnn_gemm_tc* launches (0 = every SM): with a few CTAs every CTA
+// walks many tiles of the same launch.
 static int g_cta_limit = 0;
 
-static bool tanh_bulk_enabled() {         // BSRNN_TANH_BULK=0: the generic epilogue for EPI_TANH_KB8 (A/B timing)
-  static int v = -1;
-  if (v < 0) { const char* e = getenv("BSRNN_TANH_BULK"); v = (e && e[0] == '0') ? 0 : 1; }
-  return v != 0;
-}
-
+// One launch shape per call: a plain launch of gemm_tc_kernel<EPI> (streaming or weight-resident schedule, chosen below), or
+// of the specialised straight-line kernel gemm_tc_kernel<EPI, 208> for the input projection (EPI_F16_KB8) and the
+// MaskDecoder's Conv1d+Tanh (EPI_TANH_KB8) at BN = 208, K = 208, bias folded into the weights.
 template <int EPI>
 static int launch_tc(GemmTcArgs a, cudaStream_t st) {
   static int sms = 0;                     // one process per GPU: the SM count is queried once
@@ -1039,86 +991,37 @@ static int launch_tc(GemmTcArgs a, cudaStream_t st) {
     if (cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess || sms <= 0) sms = 148;
   }
   // weight-resident schedule when several N tiles exist, the tile fits beside the A ring, and there is enough M work
+  // (the LSTM step kernels run both directions in one launch: dir_tiles > 0 keeps them streaming; measured resident
+  // with A-tile multicast: 52 vs 34 us per step at H = 768, profiles/r02 call13)
   a.b_resident = (a.n_tiles > 1 && a.n_tiles <= sms && (size_t)a.kcores * a.BN * 16 <= 120 * 1024 &&
                   a.m_tiles >= 2 * (sms / a.n_tiles) && a.ksplit <= 1 && a.dir_tiles == 0) ? 1 : 0;
-  int step_mc = 1;
-  if (EPI == EPI_LSTM_STEP && a.n_tiles > 1) {
-    // LSTM step (any H): keep the W_hh tile resident whenever it fits beside a 4-stage A ring (H = 768: BN = 96 -> 147 KB)
-    // and multicast the h tiles across clusters of N-tile CTAs: un-multicast, every step re-streams its W tile AND its A
-    // tile per output tile (4.4 GB of L2->SM traffic per band-axis step of FlowSE config 4: 830 us, profiles/r02 call12)
-    // MEASURED (profiles/r02 call13, FlowSE config-4 shapes): BN = 96 resident + multicast 52 us / 1 130 us per step (time /
-    // band axis) against 33.6 / 830 us for BN = 256 streaming, identical for multicast 1 / 2 / 4 -- the step GEMM is paced
-    // by the per-K-stage producer/MMA handshake (~400 cycles per 64-wide stage), not by L2->SM bandwidth.  Default OFF.
-    static int res_env = -1, mc_env = -1;               // BSRNN_STEP_RESIDENT=0|1 (default 0), BSRNN_STEP_MC=1|2|4 (default 4)
-    if (res_env < 0) { const char* e = getenv("BSRNN_STEP_RESIDENT"); res_env = (e && e[0] == '1') ? 1 : 0; }
-    if (mc_env < 0) { const char* e = getenv("BSRNN_STEP_MC"); mc_env = (e && (e[0] == '1' || e[0] == '2' || e[0] == '4')) ? e[0] - '0' : 4; }
-    const int ndir = a.dir_tiles > 0 ? 2 : 1;
-    const int nt_all = a.n_tiles * ndir;
-    const int per_dir = a.dir_tiles > 0 ? a.dir_tiles : a.m_tiles;
-    if (res_env && nt_all <= sms && tc_smem_bytes(a.BN, a.kcores, true, false, 4) <= 227 * 1024 && per_dir >= 2 * (sms / nt_all) &&
-        (a.dir_tiles == 0 || a.m_tiles == 2 * a.dir_tiles)) {
-      a.b_resident = 1;
-      if (mc_env > 1 && a.n_tiles % mc_env == 0) step_mc = mc_env;
-    }
-  }
-  if (EPI == EPI_GLU_F32) {
-    static int rev_env = -1;              // BSRNN_GLU_REVERSE=0: ascending tile order (A/B timing)
-    if (rev_env < 0) { const char* e = getenv("BSRNN_GLU_REVERSE"); rev_env = (e && e[0] == '0') ? 0 : 1; }
-    a.reverse_m = rev_env;
-  }
-  if (EPI == EPI_TANH_KB8 || EPI == EPI_GLU_F32) {
-    // MEASURED (profiles/r02 call51, launch lists with / without): no effect -- Conv1d+GLU 32.1 us per band either way; the
-    // policy does not keep the 100 MB buffer resident against the streaming traffic around it.  Default off.
-    static int keep_env = -1;             // BSRNN_HIDDEN_L2=1: evict_last policy on the hidden activation (A/B timing)
-    if (keep_env < 0) { const char* e = getenv("BSRNN_HIDDEN_L2"); keep_env = (e && e[0] == '1') ? 1 : 0; }
-    a.l2_keep = keep_env ? (EPI == EPI_TANH_KB8 ? 1 : 2) : 0;
-  }
+  if (EPI == EPI_GLU_F32) a.reverse_m = 1;
   const size_t extra_smem = EPI == EPI_RESID_TMA ? tc_resbuf_bytes(a.BN, a.n_valid) + 128 : 0;
   if (EPI == EPI_RESID_TMA) {
     // matrix view of the output for the tensor-map path: address = seq * row_stride + step * col_step (+ group offset)
-    static int tmap_env = -1;             // BSRNN_FC_TMAP=0: 1-D bulk copies per row / run (A/B timing)
-    if (tmap_env < 0) { const char* e = getenv("BSRNN_FC_TMAP"); tmap_env = (e && e[0] == '0') ? 0 : 1; }
     long row_stride = 0, col_step = 0;
     if (a.rows.seq_inner == 1) { row_stride = a.rows.seq_outer * a.ldo; col_step = a.rows.step_stride * a.ldo; }
     else if (a.rows.seq_inner >= (long)a.rows.R) { row_stride = a.rows.seq_inner_stride * a.ldo; col_step = a.rows.step_stride * a.ldo; }
     const long steps = (a.groups ? a.m_tiles / a.n_groups : a.m_tiles) / a.rows.tiles_per_step;
     a.use_tmap = 0;
-    if (tmap_env && a.n_tiles == 1 && a.n_valid <= a.BN && a.n_valid % 8 == 4 && row_stride > 0 && a.ksplit <= 1 &&
+    if (a.n_tiles == 1 && a.n_valid <= a.BN && a.n_valid % 8 == 4 && row_stride > 0 && a.ksplit <= 1 &&
         a.out_scale == 0.f && a.out_scale_ptr == nullptr && (steps - 1) * col_step + a.n_valid <= row_stride &&
         (!a.groups || col_step == 0) && col_step < (1L << 30) &&
         make_tmap_2d_f32(&a.tmap, a.out, (uint64_t)row_stride, (uint64_t)a.rows.R, (uint64_t)row_stride * 4, (uint32_t)a.n_valid, 128)) {
       a.use_tmap = 1;
       a.tm_col_step = (int)col_step;
-      static int inner_env = -1;          // BSRNN_FC_BAND_INNER=0: step-major tile order on the band axis (A/B timing)
-      if (inner_env < 0) { const char* e = getenv("BSRNN_FC_BAND_INNER"); inner_env = (e && e[0] == '0') ? 0 : 1; }
-      if (inner_env && !a.groups && steps > 1 && col_step > 0 && a.m_tiles == steps * a.rows.tiles_per_step) a.m_inner = (int)steps;
+      if (!a.groups && steps > 1 && col_step > 0 && a.m_tiles == steps * a.rows.tiles_per_step) a.m_inner = (int)steps;
     }
   }
   // (the same band-innermost walk without a tensor map -- FlowSE, N = 384 = two N tiles of 192, one bulk copy per row -- measures
   // no difference: 5.75 vs 5.73 s on config 4, profiles/r02 call72; it stays step-major there)
-  if (EPI == EPI_RESID_TMA && !a.use_tmap) {
-    static int runs_env = -1;             // BSRNN_FC_RUNS=0: one bulk copy per row (A/B timing)
-    if (runs_env < 0) { const char* e = getenv("BSRNN_FC_RUNS"); runs_env = (e && e[0] == '0') ? 0 : 1; }
-    a.run_merge = (runs_env && a.n_tiles == 1 && a.n_valid <= a.BN && a.ldo == a.n_valid && a.n_valid % 8 == 4) ? 1 : 0;
-  }
-  a.stages = tc_smem_bytes(a.BN, a.kcores, a.b_resident, EPI == EPI_RESID_F32, 8, TC_KS, extra_smem) <= 227 * 1024 ? 8 : 4;
-  while (a.stages > 2 && tc_smem_bytes(a.BN, a.kcores, a.b_resident, EPI == EPI_RESID_F32, a.stages, TC_KS, extra_smem) > 227 * 1024) --a.stages;
-  static int force4 = -1;                 // BSRNN_GEMM_STAGES=4: previous pipeline depth (A/B timing)
-  if (force4 < 0) { const char* e = getenv("BSRNN_GEMM_STAGES"); force4 = (e && e[0] == '4') ? 1 : 0; }
-  if (force4) a.stages = 4;
-  a.ks = TC_KS;
-  // Streaming mode with a ring that only fits 4 stages of 8 k-cores (Linear 4N->N: the 333 KB weight tile rides beside every
-  // 205 KB activation tile): 8 stages of 4 k-cores hold the same bytes, but 7/8 instead of 3/4 of them are in flight while
-  // one stage is being consumed -- the loads, not the tensor pipe, pace this GEMM (ncu profiles/r02 call24: DRAM 53 %).
-  // MEASURED (profiles/r02 call41): no gain -- Linear+skip 25.6 vs 25.5 ms per step at config 2, FlowSE 38.0 vs 38.0 ms per
-  // evaluation: the ring is not what paces this GEMM.  Default stays 8 k-cores per stage.
-  static int ks_env = -1;                 // BSRNN_GEMM_KS=4 selects the 8 x 4 ring (A/B timing)
-  if (ks_env < 0) { const char* e = getenv("BSRNN_GEMM_KS"); ks_env = (e && e[0] == '4') ? 4 : 8; }
-  if (ks_env == 4 && a.stages == 4 && !a.b_resident && a.mc <= 1 && a.ksplit <= 1 && a.kcores >= 32 && a.kcores % 4 == 0 &&
-      tc_smem_bytes(a.BN, a.kcores, false, EPI == EPI_RESID_F32, 8, 4, extra_smem) <= 227 * 1024) {
-    a.ks = 4;
-    a.stages = 8;
-  }
+  if (EPI == EPI_RESID_TMA && !a.use_tmap)
+    a.run_merge = (a.n_tiles == 1 && a.n_valid <= a.BN && a.ldo == a.n_valid && a.n_valid % 8 == 4) ? 1 : 0;
+  // Streaming GEMMs whose ring only fits 4 stages of 8 k-cores (Linear 4N->N: the 333 KB weight tile rides beside every
+  // 205 KB activation tile) keep 4: 8 stages of 4 k-cores measured no gain (profiles/r02 call41: Linear+skip 25.6 vs 25.5 ms
+  // per step at config 2, FlowSE 38.0 vs 38.0 ms per evaluation).
+  a.stages = tc_smem_bytes(a.BN, a.kcores, a.b_resident, EPI == EPI_RESID_F32, 8, extra_smem) <= 227 * 1024 ? 8 : 4;
+  while (a.stages > 2 && tc_smem_bytes(a.BN, a.kcores, a.b_resident, EPI == EPI_RESID_F32, a.stages, extra_smem) > 227 * 1024) --a.stages;
   // L2 prefetch distance of the A tiles.  Streaming mode has one prefetcher per CTA: at K = 800 (Linear 4N->N, A tile
   // 205 KB) three tiles ahead on 148 CTAs is 91 MB of prefetched lines in a 126 MB L2 that also carries the residual
   // stream -- they were evicted before use and fetched twice (ncu: 9.3 GB read for 5.2 GB algorithmic,
@@ -1130,99 +1033,35 @@ static int launch_tc(GemmTcArgs a, cudaStream_t st) {
   static int dbg = -1;
   if (dbg < 0) { const char* e = getenv("BSRNN_GEMM_DEBUG"); dbg = (e && e[0] >= '0' && e[0] <= '9') ? atoi(e) : 0; }
   a.debug = dbg;
-  static int pfd = -2;                    // BSRNN_GEMM_PFDIST=0..3 overrides (A/B timing)
-  if (pfd == -2) { const char* e = getenv("BSRNN_GEMM_PFDIST"); pfd = (e && e[0] >= '0' && e[0] <= '9') ? e[0] - '0' : -1; }
-  if (pfd >= 0) a.pf_dist = pfd;
-  const size_t smem = tc_smem_bytes(a.BN, a.kcores, a.b_resident, EPI == EPI_RESID_F32, a.stages, a.ks, extra_smem);
+  const int total = a.m_tiles * a.n_tiles;
+  const int sms_use = (g_cta_limit > 0 && g_cta_limit < sms) ? g_cta_limit : sms;
+  int grid = total < sms_use ? total : sms_use;
+  if (a.b_resident) {
+    grid = (sms_use / a.n_tiles) * a.n_tiles;
+    if (grid < a.n_tiles) grid = a.n_tiles;
+  }
+  if constexpr (EPI == EPI_F16_KB8 || EPI == EPI_TANH_KB8) {
+    // Specialised kernel: 5 ring stages + two 28 KB staging blocks for the bulk stores.  Conv1d(N->4N)+Tanh runs on it too
+    // (straight-line epilogue, tile staged in shared memory in the destination layout): the st.global path of the generic
+    // epilogue paced it.  (A-tile multicast over clusters of N-tile CTAs measured 42.1 / 43.3 / 45.6 ms per step for
+    // 1 / 2 / 4, profiles/r02 call11: the L2->SM re-reads are not what bounds this GEMM.)
+    const bool fits = EPI == EPI_F16_KB8 ? a.out_kcores >= a.n_tiles * 26 : a.out_kcores > (a.n_tiles - 1) * 26;
+    if (a.BN == 208 && a.kcores == 26 && a.bias == nullptr && a.b_resident && fits) {
+      a.stages = 5;
+      const size_t smem_ip = tc_smem_bytes(a.BN, a.kcores, true, false, a.stages) + 2 * 14 * 2048;
+      BSRNN_CUDA_OK(cudaFuncSetAttribute(gemm_tc_kernel<EPI, 208>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_ip));
+      gemm_tc_kernel<EPI, 208><<<grid, tc_threads(EPI), smem_ip, st>>>(a);
+      BSRNN_LAUNCH_OK();
+      return 0;
+    }
+  }
+  const size_t smem = tc_smem_bytes(a.BN, a.kcores, a.b_resident, EPI == EPI_RESID_F32, a.stages, extra_smem);
   static size_t smem_set = 0;             // per instantiation: the attribute only ever needs to grow (step-wise launches
   if (smem > smem_set) {                  // call this thousands of times per training step)
     BSRNN_CUDA_OK(cudaFuncSetAttribute(gemm_tc_kernel<EPI>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     smem_set = smem;
   }
-  const int total = a.m_tiles * a.n_tiles;
-  const int sms_use = (g_cta_limit > 0 && g_cta_limit < sms) ? g_cta_limit : sms;
-  int grid = total < sms_use ? total : sms_use;
-  if (a.b_resident) {
-    const int nt_all = a.n_tiles * (a.dir_tiles > 0 ? 2 : 1);
-    grid = (sms_use / nt_all) * nt_all;
-    if (grid < nt_all) grid = nt_all;
-    if (a.dir_tiles > 0) a.pf_dist = 0;             // the A-tile L2 prefetcher is not direction-aware
-  }
-  if (EPI == EPI_F16_KB8 && a.BN == 208 && a.kcores == 26 && a.bias == nullptr && a.b_resident &&
-      a.out_kcores >= a.n_tiles * 26) {
-    // specialised input-projection kernel: 5 ring stages + two 28 KB staging blocks for the bulk stores
-    a.stages = 5;
-    const size_t smem_ip = tc_smem_bytes(a.BN, a.kcores, true, false, a.stages) + 2 * 14 * 2048;
-    BSRNN_CUDA_OK(cudaFuncSetAttribute(gemm_tc_kernel<EPI_F16_KB8, 208>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_ip));
-    static int mc_env = -1;               // BSRNN_GEMM_MC=1|2|4: A-tile multicast cluster size (default 1 = off: measured 42.1 / 43.3 / 45.6 ms per step for 1 / 2 / 4, profiles/r02 call11 -- the L2->SM re-reads are not what bounds this GEMM)
-    if (mc_env < 0) { const char* e = getenv("BSRNN_GEMM_MC"); mc_env = (e && (e[0] == '1' || e[0] == '2' || e[0] == '4')) ? e[0] - '0' : 1; }
-    int mc = mc_env;
-    if (mc > 1 && (a.n_tiles % mc != 0 || a.m_tiles < 2 * (sms / a.n_tiles))) mc = 1;
-    if (mc > 1) {
-      cudaLaunchConfig_t cfg = {};
-      cfg.gridDim = dim3(grid); cfg.blockDim = dim3(tc_threads(EPI)); cfg.dynamicSmemBytes = smem_ip; cfg.stream = st;
-      cudaLaunchAttribute at[1];
-      at[0].id = cudaLaunchAttributeClusterDimension;
-      at[0].val.clusterDim.x = mc; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
-      cfg.attrs = at; cfg.numAttrs = 1;
-      static int max_cl[5] = {0, 0, 0, 0, 0};           // co-resident clusters of this size (whole N-tile groups only)
-      if (max_cl[mc] == 0) {
-        int n = 0;
-        if (cudaOccupancyMaxActiveClusters(&n, gemm_tc_kernel<EPI_F16_KB8, 208>, &cfg) != cudaSuccess || n <= 0) { cudaGetLastError(); n = -1; }
-        max_cl[mc] = n;
-      }
-      if (max_cl[mc] > 0) {
-        const int groups = (max_cl[mc] * mc) / a.n_tiles;          // the persistent CTAs must all be resident at once
-        if (groups >= 1) {
-          if (groups * a.n_tiles < grid) grid = groups * a.n_tiles;
-          cfg.gridDim = dim3(grid);
-          a.mc = mc;
-          BSRNN_CUDA_OK(cudaLaunchKernelEx(&cfg, gemm_tc_kernel<EPI_F16_KB8, 208>, a));
-          BSRNN_LAUNCH_OK();
-          return 0;
-        }
-      }
-    }
-    a.mc = 1;
-    gemm_tc_kernel<EPI_F16_KB8, 208><<<grid, tc_threads(EPI_F16_KB8), smem_ip, st>>>(a);
-  } else if (EPI == EPI_TANH_KB8 && a.BN == 208 && a.kcores == 26 && a.bias == nullptr && a.b_resident &&
-             a.out_kcores > (a.n_tiles - 1) * 26 && tanh_bulk_enabled()) {
-    // MaskDecoder Conv1d(N->4N)+Tanh on the specialised kernel of the input projection (straight-line epilogue, tile staged in
-    // shared memory in the destination layout, bulk stores): the st.global path of the generic epilogue paced it
-    a.stages = 5;
-    a.mc = 1;
-    const size_t smem_ip = tc_smem_bytes(a.BN, a.kcores, true, false, a.stages) + 2 * 14 * 2048;
-    BSRNN_CUDA_OK(cudaFuncSetAttribute(gemm_tc_kernel<EPI_TANH_KB8, 208>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_ip));
-    gemm_tc_kernel<EPI_TANH_KB8, 208><<<grid, tc_threads(EPI_TANH_KB8), smem_ip, st>>>(a);
-  } else if (step_mc > 1) {
-    // cluster launch: mc consecutive CTAs = mc consecutive N tiles of the same (direction, M walk)
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3(grid); cfg.blockDim = dim3(tc_threads(EPI)); cfg.dynamicSmemBytes = smem; cfg.stream = st;
-    cudaLaunchAttribute at[1];
-    at[0].id = cudaLaunchAttributeClusterDimension;
-    at[0].val.clusterDim.x = step_mc; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
-    cfg.attrs = at; cfg.numAttrs = 1;
-    static int max_cl = 0;
-    static size_t max_cl_smem = 0;
-    if (max_cl == 0 || smem > max_cl_smem) {
-      int n = 0;
-      if (cudaOccupancyMaxActiveClusters(&n, gemm_tc_kernel<EPI>, &cfg) != cudaSuccess || n <= 0) { cudaGetLastError(); n = -1; }
-      max_cl = n; max_cl_smem = smem;
-    }
-    const int nt_all = a.n_tiles * (a.dir_tiles > 0 ? 2 : 1);
-    const int groups = max_cl > 0 ? (max_cl * step_mc) / nt_all : 0;     // persistent CTAs: all must be resident at once
-    if (groups >= 1) {
-      if (groups * nt_all < grid) grid = groups * nt_all;
-      cfg.gridDim = dim3(grid);
-      a.mc = step_mc;
-      BSRNN_CUDA_OK(cudaLaunchKernelEx(&cfg, gemm_tc_kernel<EPI>, a));
-    } else {
-      a.mc = 1;
-      gemm_tc_kernel<EPI><<<grid, tc_threads(EPI), smem, st>>>(a);
-    }
-  } else {
-    gemm_tc_kernel<EPI><<<grid, tc_threads(EPI), smem, st>>>(a);
-  }
+  gemm_tc_kernel<EPI><<<grid, tc_threads(EPI), smem, st>>>(a);
   BSRNN_LAUNCH_OK();
   return 0;
 }

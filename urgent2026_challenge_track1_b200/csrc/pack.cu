@@ -6,7 +6,6 @@
 #include "umma.cuh"
 #include "tmap.cuh"
 #include <cuda_fp16.h>
-#include <stdlib.h>
 
 namespace bsrnn {
 
@@ -22,8 +21,8 @@ struct PackArgs {
   long tokens_per_sample;  // scale row = (token / tokens_per_sample) * g_inner + (g_inner > 1 ? token % g_inner : 0)
   int g_inner;
   int one_col;           // >= C: this operand column is the constant 1 (bias row of the weights); -1 = none
-  int bulk;              // async kernel: rows arrive by cp.async.bulk (1; 2 = contiguous runs of rows merged), by ONE 2-D tensor
-                         // copy per tile (3, band axis, tmap.cuh) or by 16-byte cp.async (0, BSRNN_PACK_BULK=0)
+  int bulk;              // async kernel: rows arrive by one cp.async.bulk per row (1), per run of contiguous rows (2), or by
+                         // ONE 2-D tensor copy per block (3, band axis, tmap.cuh)
   int m_inner;           // bulk == 3: blocks walk the tiles with the step (= band) innermost: co-running blocks read adjacent
                          // segments of the same rows of the residual stream
   int tm_col_step;       // bulk == 3: the tile is rows [j*128, +128) x cols [step*tm_col_step, +C) of the matrix view `tmap`
@@ -122,16 +121,19 @@ __global__ void __launch_bounds__(256) norm_cast_kb8_kernel(const PackArgs a, in
 }
 
 
-// Asynchronous variant (vectorisable shapes): every thread fires its share of the tile's 16-byte global->shared
-// cp.async copies at once (no registers held, ~100 KB in flight per block, 2 blocks per SM), waits once, and then
-// converts from the f32 shared-memory tile: thread = (k-core, row) reads 8 floats, applies the affine and stores one
-// 16-byte KB8 core entry (a warp = 512 contiguous bytes).  The register-staged kernel above held at most 8 loads per
-// thread and measured 0.885 ms = 2.9 TB/s at BASELINE config 2 whatever that count (profiles/r01/call26, call42).
+// Asynchronous variant (vectorisable shapes): the block's rows arrive in an f32 shared-memory tile by bulk copies (no
+// registers held), and the block then converts from there: thread = (k-core, row) reads 8 floats, applies the affine and
+// stores one 16-byte KB8 core entry.  The register-staged kernel above held at most 8 loads per thread and measured
+// 0.885 ms = 2.9 TB/s at BASELINE config 2 whatever that count (profiles/r01/call26, call42).
 // Row stride LD floats with LD % 8 == 4 (C itself for N = 196, C + 4 for N = 384 / 768): consecutive rows start 4 banks
-// apart, so the 8 rows of one 16-byte-access phase cover all 32 banks.  ROWS = 128 (one block per tile) or 64 (two blocks
-// per tile, each owning half of the rows of every k-core) so that the f32 staging tile fits twice per SM at any width.
-template <int ROWS>
+// apart, so the 8 rows of one 16-byte-access phase cover all 32 banks.
+// A block owns PACK_ROWS = 32 rows of every k-core of a tile (four blocks per tile): a block loads, waits, then converts, and
+// only co-resident blocks overlap those phases.  MEASURED (profiles/r02 call53 / call54, N = 196, config 2): 128-row blocks
+// (2 per SM) 595 / 614 us per call (time / band axis), 64-row blocks 463 / 541 us, 32-row blocks (8 per SM) 402 / 447 us;
+// FlowSE config 4 5.78 s (32) vs 5.84 s (64).
+constexpr int PACK_ROWS = 32;
 __global__ void __launch_bounds__(256) norm_cast_kb8_async_kernel(const __grid_constant__ PackArgs a, int ld) {
+  constexpr int ROWS = PACK_ROWS;
   extern __shared__ __align__(128) unsigned char smem_raw[];
   float* tile = reinterpret_cast<float*>(smem_raw);                    // [ROWS][ld]
   PackRow* rows = reinterpret_cast<PackRow*>(smem_raw + (size_t)ROWS * ld * 4);
@@ -151,59 +153,42 @@ __global__ void __launch_bounds__(256) norm_cast_kb8_async_kernel(const __grid_c
     rows[r] = pr;
   }
   __syncthreads();
-  if (a.bulk) {
-    // one bulk (1-D TMA) copy per row: C*4 contiguous bytes, completion counted on one mbarrier.  The DMA engine issues
-    // whole-row bursts instead of 6 272 separate 16-byte cp.async requests per tile.
-    __shared__ uint64_t bar;
-    if (threadIdx.x == 0) { umma::mbar_init(&bar, ROWS); umma::fence_barrier_init(); }
-    __syncthreads();
-    if (a.bulk == 3) {
-      if (threadIdx.x < ROWS) {
-        if (threadIdx.x == 0) {
-          umma::mbar_expect_tx(&bar, (uint32_t)ROWS * (uint32_t)a.C * 4);
-          tma_load_2d(tile, &a.tmap, step * a.tm_col_step, j * 128 + r0, &bar);
-        } else {
-          umma::mbar_arrive(&bar);
-        }
-      }
-    } else
+  // one bulk (1-D TMA) copy per row: C*4 contiguous bytes, completion counted on one mbarrier.  The DMA engine issues
+  // whole-row bursts instead of separate 16-byte requests.
+  __shared__ uint64_t bar;
+  if (threadIdx.x == 0) { umma::mbar_init(&bar, ROWS); umma::fence_barrier_init(); }
+  __syncthreads();
+  if (a.bulk == 3) {
     if (threadIdx.x < ROWS) {
-      const int r = threadIdx.x;
-      const long tok = rows[r].tok;
-      // dense rows (ldx == C == ld, time axis: the K bands of a frame are consecutive tokens): the rows of a warp whose
-      // tokens are consecutive are one contiguous run in HBM and in the tile and arrive by ONE bulk copy
-      uint32_t nr = tok >= 0 ? 1u : 0u;
-      if (a.bulk == 2) {
-        const int lane = threadIdx.x & 31;
-        const long ptok = __shfl_up_sync(0xffffffffu, tok, 1);
-        const bool head = tok >= 0 && (lane == 0 || ptok < 0 || tok != ptok + 1);
-        const unsigned heads = __ballot_sync(0xffffffffu, head), oks = __ballot_sync(0xffffffffu, tok >= 0);
-        const unsigned above = lane == 31 ? 0u : ((heads | ~oks) & ~((2u << lane) - 1u));
-        nr = head ? (uint32_t)((above ? __ffs(above) - 1 : 32) - lane) : 0u;
-      }
-      if (nr) {
-        umma::mbar_expect_tx(&bar, nr * (uint32_t)a.C * 4);
-        umma::bulk_g2s(tile + (size_t)r * ld, a.x + tok * a.ldx + a.col0, nr * (uint32_t)a.C * 4, &bar);
+      if (threadIdx.x == 0) {
+        umma::mbar_expect_tx(&bar, (uint32_t)ROWS * (uint32_t)a.C * 4);
+        tma_load_2d(tile, &a.tmap, step * a.tm_col_step, j * 128 + r0, &bar);
       } else {
         umma::mbar_arrive(&bar);
       }
     }
-    umma::mbar_wait(&bar, 0);
-  } else {
-  const int q4 = a.C >> 2;                                             // 16-byte pieces per row
-  const int items = ROWS * q4;
-  const uint32_t tile_s = (uint32_t)__cvta_generic_to_shared(tile);
-  for (int idx = threadIdx.x; idx < items; idx += 256) {
-    const int r = idx / q4, c4 = idx - r * q4;
+  } else if (threadIdx.x < ROWS) {
+    const int r = threadIdx.x;
     const long tok = rows[r].tok;
-    if (tok >= 0) {
-      const float* src = a.x + tok * a.ldx + a.col0 + 4 * c4;
-      asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(tile_s + (uint32_t)(r * ld + 4 * c4) * 4), "l"(src) : "memory");
+    // dense rows (ldx == C == ld, time axis: the K bands of a frame are consecutive tokens): the rows of a warp whose
+    // tokens are consecutive are one contiguous run in HBM and in the tile and arrive by ONE bulk copy
+    uint32_t nr = tok >= 0 ? 1u : 0u;
+    if (a.bulk == 2) {
+      const int lane = threadIdx.x & 31;
+      const long ptok = __shfl_up_sync(0xffffffffu, tok, 1);
+      const bool head = tok >= 0 && (lane == 0 || ptok < 0 || tok != ptok + 1);
+      const unsigned heads = __ballot_sync(0xffffffffu, head), oks = __ballot_sync(0xffffffffu, tok >= 0);
+      const unsigned above = lane == 31 ? 0u : ((heads | ~oks) & ~((2u << lane) - 1u));
+      nr = head ? (uint32_t)((above ? __ffs(above) - 1 : 32) - lane) : 0u;
+    }
+    if (nr) {
+      umma::mbar_expect_tx(&bar, nr * (uint32_t)a.C * 4);
+      umma::bulk_g2s(tile + (size_t)r * ld, a.x + tok * a.ldx + a.col0, nr * (uint32_t)a.C * 4, &bar);
+    } else {
+      umma::mbar_arrive(&bar);
     }
   }
-  asm volatile("cp.async.commit_group;" ::: "memory");
-  asm volatile("cp.async.wait_group 0;" ::: "memory");
-  }
+  umma::mbar_wait(&bar, 0);
   __syncthreads();
   __half* dst = a.out + (size_t)m * a.kcores * 128 * 8;
   for (int i = threadIdx.x; i < a.kcores * ROWS; i += 256) {
@@ -253,53 +238,23 @@ extern "C" int bsrnn_norm_cast_kb8_ones(const float* x, const float* scale, cons
   const int vec_ok = (C % 4 == 0 && col0 % 4 == 0 && ldx % 4 == 0 && (reinterpret_cast<uintptr_t>(x) & 15) == 0 &&
                       (!scale || ((reinterpret_cast<uintptr_t>(scale) & 15) == 0 && (reinterpret_cast<uintptr_t>(shift) & 15) == 0)))
                          ? 1 : 0;
-  // asynchronous kernel: vectorisable shapes whose f32 tile fits twice per SM and whose row stride is bank-friendly
-  static int force_old = -1;              // BSRNN_PACK_SYNC=1: the register-staged kernel (A/B timing)
-  if (force_old < 0) { const char* e = getenv("BSRNN_PACK_SYNC"); force_old = (e && e[0] == '1') ? 1 : 0; }
+  // asynchronous kernel: vectorisable shapes whose f32 block tile fits (bank-friendly row stride)
   const int ld = (C % 8 == 4) ? C : C + 4;              // bank-friendly row stride of the staging tile
-  static int bulk_env = -1;
-  if (bulk_env < 0) { const char* e = getenv("BSRNN_PACK_BULK"); bulk_env = (e && e[0] == '0') ? 0 : 1; }
-  a.bulk = bulk_env;
-  static int runs_env = -1;               // BSRNN_PACK_RUNS=0: one bulk copy per row even where rows are contiguous (A/B timing)
-  if (runs_env < 0) { const char* e = getenv("BSRNN_PACK_RUNS"); runs_env = (e && e[0] == '0') ? 0 : 1; }
-  if (a.bulk && runs_env && ld == C && ldx == C && col0 == 0) a.bulk = 2;
-  const size_t smem128 = (size_t)128 * ld * 4 + 128 * sizeof(PackRow), smem64 = (size_t)64 * ld * 4 + 64 * sizeof(PackRow);
-  const size_t smem32 = (size_t)32 * ld * 4 + 32 * sizeof(PackRow);
-  // band axis (seq_inner == 1: token = seq * seq_outer + step * step_stride): the tile is a box of the row-major matrix
-  // [R rows][seq_outer * ldx floats] -> one tensor copy (the box is ROWS x C; full tiles only: ROWS = 128)
-  static int tmap_env = -1;               // BSRNN_PACK_TMAP=0: per-row bulk copies on the band axis (A/B timing)
-  if (tmap_env < 0) { const char* e = getenv("BSRNN_PACK_TMAP"); tmap_env = (e && e[0] == '0') ? 0 : 1; }
-  // rows per block: 128 when the f32 tile fits twice per SM, else 64 / 32.  BSRNN_PACK_ROWS=64|32 forces smaller blocks
-  // (more blocks per SM: a block loads, waits, then converts -- only co-resident blocks overlap those phases)
-  // MEASURED (profiles/r02 call53, N = 196, config 2): 128-row blocks (2 per SM) 595 / 614 us per call (time / band axis),
-  // 64-row blocks (4 per SM) 463 / 541 us -- the kernel was bound by the load-wait-convert sequence of too few resident blocks,
-  // not by HBM or by the number of bulk copies.  Default: 32-row blocks.
-  static int rows_env = -1;
-  if (rows_env < 0) { const char* e = getenv("BSRNN_PACK_ROWS"); rows_env = e ? atoi(e) : 0; }
-  const int rows_fit = smem128 <= 110 * 1024 ? 128 : (smem64 <= 110 * 1024 ? 64 : 32);
-  int rows_sel = 32;                      // call54: 32-row blocks (8 per SM at N = 196) 402 / 447 us; FlowSE config 4 5.78 s (32) vs 5.84 s (64)
-  if ((rows_env == 128 || rows_env == 64 || rows_env == 32) && rows_env <= rows_fit) rows_sel = rows_env;
-  if (a.bulk && tmap_env && ld == C && col0 == 0 && seq_inner == 1 && seq_inner_stride == 0 &&
+  a.bulk = (ld == C && ldx == C && col0 == 0) ? 2 : 1;
+  const size_t smem_async = (size_t)PACK_ROWS * ld * 4 + PACK_ROWS * sizeof(PackRow);
+  // band axis (seq_inner == 1: token = seq * seq_outer + step * step_stride): the block's rows are a box of the row-major
+  // matrix [R rows][seq_outer * ldx floats] -> one tensor copy (the box is PACK_ROWS x C)
+  if (ld == C && col0 == 0 && seq_inner == 1 && seq_inner_stride == 0 &&
       (long)(m_tiles / tiles_per_step - 1) * step_stride * ldx + C <= seq_outer * ldx && step_stride * ldx < (1L << 30) &&
       make_tmap_2d_f32(&a.tmap, x, (uint64_t)(seq_outer * ldx), (uint64_t)R, (uint64_t)(seq_outer * ldx) * 4, (uint32_t)C,
-                       (uint32_t)rows_sel)) {
+                       (uint32_t)PACK_ROWS)) {
     a.bulk = 3;
     a.tm_col_step = (int)(step_stride * ldx);
-    static int inner_env = -1;            // BSRNN_PACK_BAND_INNER=0: step-major block order (A/B timing)
-    if (inner_env < 0) { const char* e = getenv("BSRNN_PACK_BAND_INNER"); inner_env = (e && e[0] == '0') ? 0 : 1; }
-    if (inner_env && m_tiles % tiles_per_step == 0 && m_tiles / tiles_per_step > 1) a.m_inner = m_tiles / tiles_per_step;
+    if (m_tiles % tiles_per_step == 0 && m_tiles / tiles_per_step > 1) a.m_inner = m_tiles / tiles_per_step;
   }
-  if (vec_ok && !force_old && C % 4 == 0 && smem32 <= 110 * 1024 && (one_col < 0 || one_col % 4 == 0)) {
-    if (rows_sel == 128) {
-      BSRNN_CUDA_OK(cudaFuncSetAttribute(norm_cast_kb8_async_kernel<128>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem128));
-      norm_cast_kb8_async_kernel<128><<<m_tiles, 256, smem128, (cudaStream_t)stream>>>(a, ld);
-    } else if (rows_sel == 64) {           // wide rows (N = 384: 196 KB per tile): half tiles, still two blocks per SM
-      BSRNN_CUDA_OK(cudaFuncSetAttribute(norm_cast_kb8_async_kernel<64>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem64));
-      norm_cast_kb8_async_kernel<64><<<2 * m_tiles, 256, smem64, (cudaStream_t)stream>>>(a, ld);
-    } else {                               // 2N = 768 (condition_fc operand): quarter tiles
-      BSRNN_CUDA_OK(cudaFuncSetAttribute(norm_cast_kb8_async_kernel<32>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem32));
-      norm_cast_kb8_async_kernel<32><<<4 * m_tiles, 256, smem32, (cudaStream_t)stream>>>(a, ld);
-    }
+  if (vec_ok && C % 4 == 0 && smem_async <= 110 * 1024 && (one_col < 0 || one_col % 4 == 0)) {
+    BSRNN_CUDA_OK(cudaFuncSetAttribute(norm_cast_kb8_async_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_async));
+    norm_cast_kb8_async_kernel<<<(128 / PACK_ROWS) * m_tiles, 256, smem_async, (cudaStream_t)stream>>>(a, ld);
     BSRNN_LAUNCH_OK();
     return 0;
   }

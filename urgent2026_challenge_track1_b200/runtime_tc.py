@@ -342,7 +342,6 @@ def dual_path_tc(skip, layers, t_emb=None, max_clusters=0, stats_ready=False, ba
 
 # ------------------------------------------------------------------------------------------------ band split
 BAND_SPLIT_TC = os.environ.get("BSRNN_BAND_SPLIT_TC", "1") == "1"      # 0: the f32 CUDA-core kernel (A/B, bandsplit.cu)
-BAND_SPLIT_GROUPED = os.environ.get("BSRNN_BAND_SPLIT_GROUPED", "1") == "1"   # 0: one GEMM launch per band (A/B)
 
 
 def pack_band_split_tc(bs):
@@ -366,7 +365,7 @@ def pack_band_split_tc(bs):
 
 def band_split_tc(spec, plan, bs_pack, bs_tc, N, stats):
     """spec (B,T,F,2) -> skip (B,T,K',N) f32 on tensor cores [reference bsrnn_flowse.py:65-86]: one operand-builder launch
-    (per-band GroupNorm applied on the fly) + one store-only tcgen05 GEMM per band.  The GEMM epilogues also accumulate the
+    (per-band GroupNorm applied on the fly) + one store-only tcgen05 GEMM launch for all bands.  The GEMM epilogue also accumulates the
     per-sample sums of the result into workspace(...).stats: the first dual-path GroupNorm needs no pass of its own."""
     from .runtime import _i32, _const_table
     B, T, F, _ = spec.shape
@@ -394,30 +393,19 @@ def band_split_tc(spec, plan, bs_pack, bs_tc, N, stats):
            bs_pack["c_off"].data_ptr(), bin0.data_ptr(), wid.data_ptr(), a_off_d.data_ptr(), K, B * T, T, 2 * F, cmax, st)
     out = torch.empty(B, T, K, N, dtype=torch.float32, device=dev)
     ws.stats.zero_()
-    if BAND_SPLIT_GROUPED and bs_tc["BN"] >= N:
-        # one launch for all bands, band innermost in the tile order: co-running CTAs write adjacent 4N-byte segments of the
-        # same rows of the (B,T,K,N) stream
-        desc = []
-        for k in range(K):
-            desc += [offs[k], bs_tc["w_off"][k], k * N, k * bs_tc["BN"], bs_tc["kcs"][k]]
-        groups = _const_table(desc, torch.int64, dev)
-        L.call("bsrnn_gemm_tc_grouped", xhat.data_ptr(), bs_tc["w"].data_ptr(), bs_tc["bias"].data_ptr(), out.data_ptr(),
-               ws.stats.data_ptr(), groups.data_ptr(), K, tiles, max(bs_tc["kcs"][:K]), bs_tc["BN"], K * N, N, T, tiles,
-               B * T, BIG, 0, 1, 0, st)
-        return out
+    # one launch for all bands, band innermost in the tile order: co-running CTAs write adjacent 4N-byte segments of the
+    # same rows of the (B,T,K,N) stream
+    desc = []
     for k in range(K):
-        L.call("bsrnn_gemm_tc_ex", xhat.data_ptr() + 2 * offs[k], bs_tc["w"].data_ptr() + 2 * bs_tc["w_off"][k],
-               bs_tc["bias"][k].data_ptr(), out.data_ptr() + 4 * k * N, ws.stats.data_ptr(), tiles, 1, bs_tc["kcs"][k],
-               bs_tc["BN"], L.TC_RESID_TMA, K * N, N, 0, T, tiles, B * T, BIG, 0, 1, 0, 1, 1, st)
+        desc += [offs[k], bs_tc["w_off"][k], k * N, k * bs_tc["BN"], bs_tc["kcs"][k]]
+    groups = _const_table(desc, torch.int64, dev)
+    L.call("bsrnn_gemm_tc_grouped", xhat.data_ptr(), bs_tc["w"].data_ptr(), bs_tc["bias"].data_ptr(), out.data_ptr(),
+           ws.stats.data_ptr(), groups.data_ptr(), K, tiles, max(bs_tc["kcs"][:K]), bs_tc["BN"], K * N, N, T, tiles,
+           B * T, BIG, 0, 1, 0, st)
     return out
 
 
 # ------------------------------------------------------------------------------------------------ mask decoder
-MASKDEC_ONES = os.environ.get("BSRNN_MASKDEC_ONES", "1") == "1"      # 0: separate bias vector, generic tanh epilogue (A/B)
-MASKDEC_SMS = int(os.environ.get("BSRNN_MASKDEC_SMS", "0"))          # persistent CTAs per mask-decoder GEMM launch (0 = all SMs)
-MASKDEC_SHARED_NORM = os.environ.get("BSRNN_MASKDEC_SHARED_NORM", "1") == "1"   # 0: one normalised operand per MLP family
-
-
 def pack_mask_decoder_tc(md):
     """espnet2-style MaskDecoder for the tensor-core path: Conv1d(N,4N) as 208-column tiles, Conv1d(4N,4s) with rows
     interleaved (value, gate) so the GLU pairs sit in adjacent accumulator columns."""
@@ -431,18 +419,16 @@ def pack_mask_decoder_tc(md):
         nt1 = (H4 + LBN - 1) // LBN
         w1, b1, w2, b2, bn2 = [], [], [], [], []
         # bias of Conv1d(N,4N) as weight column N against the operand's constant-one column (bsrnn_norm_cast_kb8_ones): the
-        # GEMM then runs bias-free on the bulk-store tanh kernel (gemm_tc.cu, EPI_TANH_KB8 / BNC = 208)
-        one_col = N if (MASKDEC_ONES and N % 4 == 0 and kc1 * 8 > N) else -1
+        # GEMM then runs bias-free on the bulk-store tanh kernel (gemm_tc.cu, EPI_TANH_KB8 / BNC = 208).  Widths without a
+        # padding column for it (N % 16 == 0, or N % 4 != 0) keep the bias vector and one normalised operand per family.
+        one_col = N if (N % 4 == 0 and kc1 * 8 > N) else -1
         for k, m in enumerate(mlps):
             wk = m[1].weight[:, :, 0].float()
             if one_col >= 0:
-                bk = m[1].bias.float()
-                if MASKDEC_SHARED_NORM:
-                    # W (z * gamma + beta) + b = (W diag(gamma)) z + (W beta + b): with the per-channel affine of this family's
-                    # GroupNorm folded in, BOTH families read one operand z = (x - mean) * rstd (one norm_cast, not two)
-                    bk = bk + wk @ m[0].bias.float()
-                    wk = wk * m[0].weight.float()[None, :]
-                wk = torch.cat([wk, bk[:, None]], 1)
+                # W (z * gamma + beta) + b = (W diag(gamma)) z + (W beta + b): with the per-channel affine of this family's
+                # GroupNorm folded in, BOTH families read one operand z = (x - mean) * rstd (one norm_cast, not two)
+                bk = m[1].bias.float() + wk @ m[0].bias.float()
+                wk = torch.cat([wk * m[0].weight.float()[None, :], bk[:, None]], 1)
             w1.append(to_kb8(wk, LBN, kc1))
             bb = torch.zeros(nt1 * LBN, device=m[1].bias.device); bb[:H4] = m[1].bias
             b1.append(bb)
@@ -457,7 +443,7 @@ def pack_mask_decoder_tc(md):
         out[name] = dict(gamma=torch.stack([m[0].weight for m in mlps]).float().contiguous(),
                          beta=torch.stack([m[0].bias for m in mlps]).float().contiguous(),
                          w1=w1, b1=b1, w2=w2, b2=b2, bn2=bn2, kc1=kc1, kc2=kc2, nt1=nt1, N=N, one_col=one_col,
-                         shared_norm=bool(MASKDEC_SHARED_NORM and one_col >= 0),
+                         shared_norm=one_col >= 0,
                          eps=float(mlps[0][0].eps))
     return out
 
@@ -504,9 +490,6 @@ def mask_decoder_tc(skip, plan, md_pack, band_stats=None):
                    p["kc1"], K * tiles, tiles, B * T, 1, K, 0, 1, T * K, K, p["one_col"], st)
         fork.record(main)
         side.wait_event(fork)
-        # each family's GEMMs on MASKDEC_SMS persistent CTAs (0 = all): with half of the SMs per launch the two streams' kernels
-        # really run side by side (a 148-CTA launch holds every SM: 200 KB of shared memory and all of TMEM per CTA)
-        prev_limit = L.lib().bsrnn_gemm_tc_limit_ctas(MASKDEC_SMS)
         for name, stream in (("mlp_residual", side), ("mlp_mask", main)):
             p = md_pack[name]
             scale, shift = tabs[name][0], tabs[name][1]
@@ -529,7 +512,6 @@ def mask_decoder_tc(skip, plan, md_pack, band_stats=None):
                 for t in (xhat, hidden, o, skip, scale, shift):
                     t.record_stream(side)
             outs[name] = o
-        L.lib().bsrnn_gemm_tc_limit_ctas(prev_limit)
         main.wait_stream(side)
     return outs["mlp_mask"], outs["mlp_residual"]
 

@@ -20,19 +20,10 @@ from . import _lib as L
 from .runtime_tc import to_kb8, FC_EPI, lstm_ws, pack_fused, pack_steps, tile_width
 
 
-def _bn_for(cols, kcores=None):
-    """N-tile width of the step GEMM (widest that divides the gate columns).  BSRNN_STEP_RESIDENT=1 instead picks the widest
-    tile whose W_hh slice stays RESIDENT in shared memory beside a 4-stage A ring (H = 768 -> BN = 96, 147 KB) with the h
-    tiles multicast across clusters of N-tile CTAs -- measured slower (52 vs 34 us per step, profiles/r02 call13): the
-    narrow tiles pay the per-K-stage pipeline handshake 2.7x more often; kept as an A/B switch."""
-    import os
-    forced = int(os.environ.get("BSRNN_STEP_BN", "0"))
-    if forced:
-        return forced
-    if kcores is not None and os.environ.get("BSRNN_STEP_RESIDENT", "0") == "1":      # A/B switch, off: see launch_tc
-        for bn in range(256, 63, -32):
-            if cols % bn == 0 and kcores * bn * 16 + 65536 + 1024 <= 225 * 1024:
-                return bn
+def _bn_for(cols):
+    """N-tile width of the step GEMM: the widest that divides the gate columns.  (Narrow tiles whose W_hh slice stays resident
+    in shared memory, H = 768 -> BN = 96, measured slower: 52 vs 34 us per step, profiles/r02 call13 -- they pay the
+    per-K-stage pipeline handshake 2.7x more often.)"""
     return tile_width(cols, 32)
 
 
@@ -44,7 +35,7 @@ def pack_lstm_steps_tc(rnn):
     if H % 16:
         raise NotImplementedError(f"step-wise tensor-core LSTM needs H % 16 == 0, got {H}")
     kc_in = (N + 15) // 16 * 2
-    BN = _bn_for(4 * H, H // 8)
+    BN = _bn_for(4 * H)
     out = dict(pack_steps(ws, kc_in, BN), BN=BN, H=H, N=N, kc_in=kc_in, n_tiles=4 * H // BN)
     if H == 768 and N == 384:
         out.update(pack_lstm_fused768(rnn))

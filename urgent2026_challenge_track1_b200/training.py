@@ -17,7 +17,6 @@ What runs where (round-1 state, see DESIGN.md §7):
 from __future__ import annotations
 
 import math
-import os
 
 import torch
 import torch.nn.functional as F
@@ -239,10 +238,6 @@ def grad_decoder_batched(gd, skip, plan, F_bins):
     return outs[0], outs[1]
 
 
-# 0: the per-band loops (band_split_diff, mask_decoder_diff, grad_decoder_diff)
-BATCHED_BANDS = os.environ.get("BSRNN_TRAIN_BATCHED_BANDS", "1") == "1"
-
-
 def block_f32(x, rnn, fc, axis):
     """(BLSTM -> Linear) block, f32: CUDA-core recurrence kernels + library GEMMs (parity ~1e-6)."""
     return F.linear(blstm(x, rnn, axis), fc.weight, fc.bias)
@@ -345,9 +340,9 @@ def bsrnn_se_train_forward(model, wav, lens, fs, blstm_fn=None):
     lens_dev = R.device_lengths(lens, wav.device)
     with torch.no_grad():
         spec = R.stft(wav.contiguous().float(), lens_dev, n_fft, hop)           # (B,T,F,2), frames >= olens are zeros
-    skip = (band_split_batched if BATCHED_BANDS else band_split_diff)(core.band_split, spec, plan)      # (B,T,K',N)
+    skip = band_split_batched(core.band_split, spec, plan)                      # (B,T,K',N)
     skip = dual_path_diff(core, skip, blstm_fn=blstm_fn)
-    m_c, r_c = (mask_decoder_batched if BATCHED_BANDS else mask_decoder_diff)(core.mask_decoder, skip, plan, F_bins)
+    m_c, r_c = mask_decoder_batched(core.mask_decoder, skip, plan, F_bins)
     est = m_c * torch.view_as_complex(spec) + r_c                               # (B,T,F)
     if torch.cuda.is_current_stream_capturing():
         # reading device lengths would be a sync inside the capture: the output is the padded width, which is
@@ -365,9 +360,8 @@ def flow_bsrnn_train_forward(dnn, x_btf, y_btf, t, blstm_fn=None):
     import math
     F_bins = x_btf.shape[2]
     plan = R.BandPlan.make(dnn.band_split_x.subbands, F_bins)
-    bsf = band_split_batched if BATCHED_BANDS else band_split_diff
-    xx = bsf(dnn.band_split_x, x_btf, plan)
-    yy = bsf(dnn.band_split_y, y_btf, plan)
+    xx = band_split_batched(dnn.band_split_x, x_btf, plan)
+    yy = band_split_batched(dnn.band_split_y, y_btf, plan)
     skip = F.linear(torch.cat([xx, yy], dim=-1), dnn.condition_fc.weight, dnn.condition_fc.bias)    # :284-285
     t = t.to(device=x_btf.device, dtype=torch.float32)
     t_emb = []
@@ -375,7 +369,7 @@ def flow_bsrnn_train_forward(dnn, x_btf, y_btf, t, blstm_fn=None):
         proj = t[:, None] * dnn.t_cond[i].W[None, :] * 2 * math.pi
         t_emb.append(torch.cat([torch.sin(proj), torch.cos(proj)], dim=-1))
     skip = dual_path_diff(dnn, skip, t_emb=t_emb, blstm_fn=blstm_fn)
-    m_c, r_c = (grad_decoder_batched if BATCHED_BANDS else grad_decoder_diff)(dnn.grad_decoder, skip, plan, F_bins)
+    m_c, r_c = grad_decoder_batched(dnn.grad_decoder, skip, plan, F_bins)
     return m_c * torch.view_as_complex(x_btf.contiguous()) + r_c
 
 

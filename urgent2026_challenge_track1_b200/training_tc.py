@@ -37,9 +37,6 @@ def _bn_cover(rows, mult=16):
     return bn, nt
 
 
-NARROW_BN = int(os.environ.get("BSRNN_BWD_BN", "0"))      # 0 = automatic (see pack_block)
-
-
 @torch.no_grad()
 def pack_block(w_ih, w_hh, b_ih, b_hh, w_ih_r, w_hh_r, b_ih_r, b_hh_r, fc_w, narrow_bwd=False, fwd_steps=True):
     """All tensor-core operands of one block, from the f32 master weights (nn.LSTM / nn.Linear layouts).
@@ -59,8 +56,8 @@ def pack_block(w_ih, w_hh, b_ih, b_hh, w_ih_r, w_hh_r, b_ih_r, b_hh_r, fc_w, nar
     if narrow_bwd and H > 64:
         # one BPTT step is a single wave of tiles x ceil(H / bn) x 2 CTAs that each stream the whole 4H-wide dG tile: the narrowest
         # tile that still fits one wave of 148 SMs (config 5: 63.3 ms per step with 32, 68.0 with 64, 75.0 with 128; call74)
-        bn_h = NARROW_BN if NARROW_BN > 0 else (32 if isinstance(narrow_bwd, int) and not isinstance(narrow_bwd, bool)
-                                                 and 2 * narrow_bwd * ((H + 31) // 32) <= 148 else 64)
+        bn_h = (32 if isinstance(narrow_bwd, int) and not isinstance(narrow_bwd, bool)
+                and 2 * narrow_bwd * ((H + 31) // 32) <= 148 else 64)
         nt_h = (H + bn_h - 1) // bn_h
     bn_n, nt_n = _bn_cover(n_in, 16)
     p = dict(H=H, N=N, kc_in=kc_in, kc_h=kc_h, BN=BN, n_tiles=4 * H // BN, bn_h=bn_h, nt_h=nt_h, bn_n=bn_n, nt_n=nt_n)
