@@ -8,7 +8,7 @@ mkdir -p $OUT
 NVCC=${NVCC:-/usr/local/cuda/bin/nvcc}
 # no --use_fast_math: the f32-mode kernels call expf/tanhf for parity; approximations are explicit PTX where wanted
 FF="-gencode arch=compute_100a,code=sm_100a -O3 -lineinfo -std=c++17 -Xcompiler -fPIC -Xptxas -v $BSRNN_NVCC_FLAGS"
-SRCS="api fft norm gemm_f32 lstm_f32 flow pack gemm_tc lstm_tc lstm_fused optim loss bandsplit mix $EXTRA"
+SRCS="api fft norm gemm_f32 lstm_f32 flow pack gemm_tc lstm_tc lstm_fused optim loss bandsplit mix metrics $EXTRA"
 pids=""
 for f in $SRCS; do
   # rebuild only what changed (sources are independent translation units); compile in parallel

@@ -450,6 +450,43 @@ int bsrnn_mix_quantiles(const float* x, const int32_t* len, const double* q, flo
 int bsrnn_mix_finish(float* noisy, float* clean, const int32_t* len, const float* thr, const uint8_t* lost, int npk, int pkt,
                      uint32_t* peak, int B, int T, void* stream);
 
+/* ---------------------------------------------------------------------------------------------- intrusive metrics
+ * ESTOI and SDR of (reference, estimate) pairs [replaces pystoi.stoi(extended=True) and fast_bss_eval's SDR in the
+ * reference's evaluation_metrics/calculate_intrusive_se_metrics.py:37-48, :90-109].  Signals are (B, T) f32 rows valid on
+ * [0, len[b]), one sample rate per batch; no padded sample is read.  No floating-point atomics: a score is bitwise the same
+ * whether its utterance is scored alone or inside any batch.  ESTOI runs as four calls (metrics.py chains them):
+ * bsrnn_resample_poly: y[b, m] = scipy.signal.resample_poly(x[b, :len[b]], up, down, window=h)[m] for m < y_len[b] =
+ *   ceil(len[b] up / down), zeros on [y_len[b], T_out), T_out >= ceil(T up / down).  h has n_taps (odd) taps, already
+ *   normalised and scaled by up as resample_poly applies them; taps (up, ceil(n_taps / up)) f64 holds them by phase,
+ *   taps[ph, j] = h[ph + j up] (zero past n_taps).  f64 accumulation, f32 output.
+ * bsrnn_estoi_compact: silent-frame removal (256-sample frames of np.hanning(258)[1:-1], hop 128, over range(0, n - 256,
+ *   128)): the frames of x whose energy 20 log10(||frame|| + eps) is within 40 dB of x's loudest are kept, and xc / yc
+ *   (B, T) are the overlap-adds of the kept frames of x / y; c_len[b] = (kept - 1) 128 + 256 (0 without frames), zeros
+ *   beyond.  scratch: bsrnn_estoi_compact_scratch_bytes(B, T) bytes.
+ * bsrnn_estoi_bands: tob (B, 2, 15, NF) f64, [b, 0 | 1, k, t] = sqrt(sum_{band_lo[k] <= f < band_hi[k]} |X_t(f)|^2) of the
+ *   xc | yc STFT (Hann 256, hop 128, 512-point FFT in f32, frames of range(0, c_len - 256, 128)); NF >= the frame count
+ *   of T.  twiddle from bsrnn_fft_twiddle(512); band_lo / band_hi: 15 int32 each (device).
+ * bsrnn_estoi_score: for each 30-frame segment of both envelopes, rows then columns centred and scaled to unit norm (a
+ *   zero-norm row or column becomes zeros), d = sum(xn yn) / 30; out (B) f64 = the mean of d over the segments, 1e-5 with
+ *   fewer than 30 frames.  seg: B * NF doubles of scratch.
+ * bsrnn_sdr: BSS-eval v3 SDR with a 512-tap distortion filter, f64 throughout: the autocorrelation of the unit-norm
+ *   reference and its cross-correlation with the unit-norm estimate at lags 0..511 (direct sums), the symmetric Toeplitz
+ *   system solved by Levinson recursion (one CTA per utterance), coh = xcorr . sol clamped to [1e-5, 1e5] / (1 + .), out =
+ *   10 log10(coh / (1 - coh)) in [-50, 50].  A zero reference gives NaN; a non-positive Levinson pivot ends the recursion
+ *   at the last positive-definite order.  scratch: bsrnn_sdr_scratch_bytes(B, T) bytes.
+ */
+int bsrnn_resample_poly(const float* x, const int32_t* len, int B, int T, const double* taps, int n_taps, int up, int down,
+                        float* y, int32_t* y_len, int T_out, void* stream);
+long bsrnn_estoi_compact_scratch_bytes(int B, int T);
+int bsrnn_estoi_compact(const float* x, const float* y, const int32_t* len, int B, int T, float* xc, float* yc,
+                        int32_t* c_len, void* scratch, void* stream);
+int bsrnn_estoi_bands(const float* xc, const float* yc, const int32_t* c_len, int B, int T, const float* twiddle,
+                      const int32_t* band_lo, const int32_t* band_hi, double* tob, int NF, void* stream);
+int bsrnn_estoi_score(const double* tob, const int32_t* c_len, int B, int NF, double* seg, double* out, void* stream);
+long bsrnn_sdr_scratch_bytes(int B, int T);
+int bsrnn_sdr(const float* ref, const float* inf, const int32_t* len, int B, int T, double* out, double* scratch,
+              void* stream);
+
 #ifdef __cplusplus
 }
 #endif

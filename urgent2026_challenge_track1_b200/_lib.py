@@ -108,6 +108,14 @@ PROTOTYPES = {
     "bsrnn_mix_snr": [c_void_p] * 7 + [c_int, c_int, c_void_p],
     "bsrnn_mix_quantiles": [c_void_p] * 4 + [c_int, c_int, c_void_p],
     "bsrnn_mix_finish": [c_void_p] * 5 + [c_int, c_int, c_void_p, c_int, c_int, c_void_p],
+    "bsrnn_resample_poly": [c_void_p, c_void_p, c_int, c_int, c_void_p, c_int, c_int, c_int, c_void_p, c_void_p, c_int,
+                            c_void_p],
+    "bsrnn_estoi_compact_scratch_bytes": [c_int, c_int],
+    "bsrnn_estoi_compact": [c_void_p] * 3 + [c_int, c_int] + [c_void_p] * 5,
+    "bsrnn_estoi_bands": [c_void_p] * 3 + [c_int, c_int] + [c_void_p] * 4 + [c_int, c_void_p],
+    "bsrnn_estoi_score": [c_void_p, c_void_p, c_int, c_int, c_void_p, c_void_p, c_void_p],
+    "bsrnn_sdr_scratch_bytes": [c_int, c_int],
+    "bsrnn_sdr": [c_void_p] * 3 + [c_int, c_int] + [c_void_p] * 3,
 }
 
 # mirrors `bsrnn_gemm_desc` (include/bsrnn_b200.h); 144 bytes
@@ -151,6 +159,8 @@ def lib():
         handle.bsrnn_blstm_fused768_train_scratch_bytes.restype = C.c_long
         handle.bsrnn_mix_conv_scratch_bytes.restype = C.c_long
         handle.bsrnn_mix_snr_scratch_bytes.restype = C.c_long
+        handle.bsrnn_estoi_compact_scratch_bytes.restype = C.c_long
+        handle.bsrnn_sdr_scratch_bytes.restype = C.c_long
         handle.bsrnn_last_error.restype = C.c_char_p
         handle.bsrnn_last_error.argtypes = []
         _lib = handle
